@@ -15,6 +15,11 @@ One JSON line is printed by rank 0.
 
 `--impl reference` runs the UNMODIFIED reference (baseline/_ref: `pip install --target` of /root/reference, see DESIGN.md)
 on the host cores, one single-threaded process per core (the layout of `mpirun -n <cores> run-hydra-pspec.py`).
+
+`--dump-outputs DIR` (configs 1-4) writes what the last timed step computed as float64 DIR/<name>.npy, so that two builds
+can be compared output for output (the inputs and the Philox draws are seeded): signal_ps and ln_post of every chain on
+rank 0, and signal_cr, fg_amps and chisq (complex arrays with a trailing (real, imag) axis) of a fixed, seeded sample of
+its chains, as many as fit in 64 MB in all.
 """
 import argparse
 import json
@@ -48,7 +53,7 @@ CONFIGS = {
 }
 
 
-def parse_args():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=None)
@@ -61,7 +66,13 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None)
+    a = ap.parse_args(argv)
+    if a.steps is not None and a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.config == 0):
+        ap.error("--dump-outputs needs --impl b200 and --config 1..4")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------
@@ -95,6 +106,29 @@ def dense_ninv(nf):
     rng = np.random.default_rng(99)
     Xn = (rng.standard_normal((nf, 2 * nf)) + 1j * rng.standard_normal((nf, 2 * nf))) / np.sqrt(2)
     return np.linalg.inv(0.25 * (Xn @ Xn.conj().T / (2 * nf) + 0.2 * np.eye(nf)))
+
+
+DUMP_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(eng, out_dir, it):
+    """--dump-outputs: iteration `it` of every output the engine keeps, as float64 .npy files under `out_dir` (module
+    docstring).  Returns the indices of the chains whose signal_cr / fg_amps / chisq were written."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    B, T, n, m = eng.nchains, eng.ntimes, eng.nfreqs, eng.nmodes
+    out = {"signal_ps": np.stack([eng.signal_ps(c, it, 1)[0] for c in range(B)]),
+           "ln_post": np.concatenate([eng.ln_post(c, it, 1) for c in range(B)])}
+    per_chain = 8 * T * (2 * n + 2 * m + n)   # signal_cr + fg_amps + chisq of one chain
+    room = DUMP_BYTES - sum(a.nbytes for a in out.values())
+    chains = np.sort(np.random.default_rng(0).choice(B, min(B, room // per_chain), replace=False))
+    for name in ("signal_cr", "fg_amps", "chisq"):
+        out[name] = np.stack([getattr(eng, name)(int(c), it, 1)[0] for c in chains])
+    for name, a in out.items():
+        if np.iscomplexobj(a):
+            a = np.ascontiguousarray(a).view(np.float64).reshape(a.shape + (2,))
+        np.save(out_dir / f"{name}.npy", a)
+    return chains
 
 
 class ClockSampler:
@@ -480,6 +514,7 @@ def run_b200(args):
     barrier()
     ms = ev0.elapsed_time(ev1)
     launches = eng.launch_count - l0
+    dumped = dump_outputs(eng, args.dump_outputs, W + K - 1) if (args.dump_outputs and rank == 0) else None
     # per-kernel durations: same engine, sub-batches off so that the kernels do not overlap
     eng.set_substreams(1)
     eng.set_profile(True)
@@ -689,6 +724,8 @@ def run_b200(args):
             "roofline": roofline, "cpu_baseline": cpu, "e2e": e2e, "gpu_launches": int(launches), "parity_check": parity,
             "gather": gather, "clocks": clk.summary(), "chol_failures": bad, "finite": finite,
         }
+        if dumped is not None:
+            line["dump_outputs"] = {"dir": args.dump_outputs, "iteration": W + K - 1, "sampled_chains": dumped.tolist()}
         os.write(json_fd, (json.dumps(line) + "\n").encode())
     if world > 1:
         dist.destroy_process_group()

@@ -38,3 +38,56 @@ def test_cpu_arm_runs_on_the_smallest_config():
     assert dt > 0 and kind.split(" ")[0] in ("reference", "port")
     if (bench.ROOT / "baseline" / "_ref" / "hydra_pspec" / "pspec.py").is_file():
         assert kind.startswith("reference")
+
+
+class _FakeEngine:
+    """The read side of GibbsEngine at the configs[3] shape; every value encodes (chain, iteration)."""
+
+    def __init__(self, B=128, T=1024, n=384, m=32):
+        self.nchains, self.ntimes, self.nfreqs, self.nmodes = B, T, n, m
+
+    def _fill(self, c, it, shape, dtype=np.float64):
+        a = np.full(shape, 1000.0 * c + it, dtype=dtype)
+        if np.iscomplexobj(a):
+            a += 0.5j
+        return a
+
+    def signal_ps(self, c, it, k):
+        return self._fill(c, it, (k, self.nfreqs))
+
+    def ln_post(self, c, it, k):
+        return self._fill(c, it, (k,))
+
+    def signal_cr(self, c, it, k):
+        return self._fill(c, it, (k, self.ntimes, self.nfreqs), np.complex128)
+
+    def fg_amps(self, c, it, k):
+        return self._fill(c, it, (k, self.ntimes, self.nmodes), np.complex128)
+
+    def chisq(self, c, it, k):
+        return self._fill(c, it, (k, self.ntimes, self.nfreqs))
+
+
+def test_dump_outputs_writes_a_seeded_float64_sample_within_64_MB(tmp_path):
+    eng = _FakeEngine()
+    chains = bench.dump_outputs(eng, tmp_path / "a", 22)
+    assert np.array_equal(chains, bench.dump_outputs(eng, tmp_path / "b", 22))
+    assert 1 <= len(chains) < eng.nchains and np.all(np.diff(chains) > 0)
+    files = {p.name: p for p in (tmp_path / "a").iterdir()}
+    assert sorted(files) == sorted(f"{k}.npy" for k in ("signal_ps", "ln_post", "signal_cr", "fg_amps", "chisq"))
+    assert sum(p.stat().st_size for p in files.values()) <= 64 * 2 ** 20
+    out = {k[:-4]: np.load(p) for k, p in files.items()}
+    assert all(a.dtype == np.float64 for a in out.values())
+    assert np.array_equal(out["signal_ps"][:, 0], 1000.0 * np.arange(eng.nchains) + 22)
+    assert np.array_equal(out["ln_post"], 1000.0 * np.arange(eng.nchains) + 22)
+    assert out["signal_cr"].shape == (len(chains), 1024, 384, 2) and out["fg_amps"].shape == (len(chains), 1024, 32, 2)
+    assert out["chisq"].shape == (len(chains), 1024, 384)
+    assert np.array_equal(out["signal_cr"][:, 0, 0], np.stack([1000.0 * chains + 22, np.full(len(chains), 0.5)], axis=1))
+    assert np.array_equal(out["chisq"][:, 5, 7], 1000.0 * chains + 22)
+
+
+def test_steps_and_dump_arguments():
+    assert bench.parse_args(["--steps", "7"]).steps == 7
+    for bad in (["--steps", "0"], ["--config", "0", "--dump-outputs", "x"], ["--impl", "reference", "--dump-outputs", "x"]):
+        with pytest.raises(SystemExit):
+            bench.parse_args(bad)
