@@ -2,7 +2,7 @@
 //
 // The block lives in shared memory (planar re / im, row stride kLdBlk).  History: (1) all 512 threads,
 // two __syncthreads per column (128 block-wide barriers per block); (2) a two-warp pipeline, one named
-// barrier per column, ~20 us per block (measured by removing it: 30 % of k_pt_cholsolve, 17 % of k_chol).
+// barrier per column, ~20 us per block (measured by removing it: 30 % of k_pt_cholsolve, 17 % of the round-1 Cholesky kernel).
 // This version is a right-looking factorisation over the 4 x 4 grid of 8x8 sub-blocks:
 //
 //   for kk = 0..3:  one warp factors the 8x8 diagonal sub-block in registers (lane = row, shuffles for

@@ -266,10 +266,10 @@ struct hp_engine {
     std::vector<uint8_t> pt_loaded;   // per chain: loaded with per-time flags
     int gd_slots = 1;
     std::vector<uint8_t> pending;         // chains whose G / Rfix products are still to be built (flush_pending)
-    bool big_solve = false;               // N too large for k_solve's resident tile: dense k_zgemm products with W
+    bool big_solve = false;               // N too large for k_solve's resident tile: dense k_zgemm2 products with W
     bool solve2 = false;                  // k_solve2 (persistent, register-blocked, shared W ring) takes the solve
     bool solve3 = false;                  // k_solve3 (independent warps, W fragments streamed into registers) takes the solve
-    double *Wf1 = nullptr, *Wf2 = nullptr;   // fragment-major W for k_solve3 (k_trinv writes them)
+    double *Wf1 = nullptr, *Wf2 = nullptr;   // fragment-major W for k_solve3 (k_chol_w writes them)
     hp::Solve3Sched sched3{};
     int pp_tiles = 0;                     // partial |ytilde|^2 sums per chain in Ppart: ntiles (k_solve), 2 ntiles (k_solve2)
     double* Wp1 = nullptr;                // W diag(lam): pass-1 operand of k_solve2 when Rt holds the unscaled Rfix (Philox mode)
@@ -952,7 +952,7 @@ static void enqueue_dense_lnp1(hp_engine* e, const Sub& sb) {
     hp::ZgemmArgs y{};
     y.A = OFFS(e->Rm, 2 * Tp * n); y.sAi = e->n; y.sAk = 1; y.bsA = (long long)e->Tp * e->n;
     // r^H Ni r = 2 Re(r^H NiL r) with NiL the lower half of the Hermitian part of Ni (k_lower_half): Y = R conj(NiL) is a
-    // triangular product (B[k][j] = conj(NiL[k][j]) = 0 for k < j: k_zgemm skips that K range), half the flops of R Ni^T
+    // triangular product (B[k][j] = conj(NiL[k][j]) = 0 for k < j: k_zgemm2 skips that K range), half the flops of R Ni^T
     y.B = OFFS(e->NiL, 2 * n * n); y.sBk = e->n; y.sBj = 1; y.conjB = 1; y.bsB = (long long)e->n * e->n;
     y.C = OFFS(e->Yd, 2 * Tp * n); y.sCi = e->n; y.sCj = 1; y.bsC = (long long)e->Tp * e->n;
     y.M = e->T; y.N = e->n; y.K = e->n; y.alpha = 1.0; y.batch = sb.nc;
@@ -1006,14 +1006,11 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
     ca.Gp = OFFS(b.Gp, tri * hp::kBlkDoubles); ca.lam = OFFS(e->lam, Np); ca.Lp = OFFS(e->Lp, tri * hp::kLBlkDoubles);
     ca.Linvp = OFFS(e->Linvp, (size_t)e->nblk * hp::kLBlkDoubles); ca.info = e->info + sb.c0;
     ca.nblk = e->nblk; ca.n = e->n; ca.N = e->N; ca.nsys = sb.nc;
-    int nchol;
-    {
-        // Philox mode: the stored right-hand-side tiles are the unscaled Rfix, so pass 1 multiplies by W diag(lam)
-        hp::TrinvExtra ex{OFFS(e->Wp1, tri * hp::kLBlkDoubles), OFFS(e->Wf1, hp::solve3_frag_doubles(e->nblk)),
-                          OFFS(e->Wf2, hp::solve3_frag_doubles(e->nblk)), philox ? OFFS(e->lam, Np) : nullptr};
-        nchol = hp::launch_chol_trinv(ca, OFFS(e->Wp, tri * hp::kLBlkDoubles), ex, sb.st) - 1;
-    }
-    e->prof_end(CLS_CHOL, nchol + 1, sb.st);
+    // Philox mode: the stored right-hand-side tiles are the unscaled Rfix, so pass 1 multiplies by W diag(lam)
+    const hp::TrinvExtra ex{OFFS(e->Wp1, tri * hp::kLBlkDoubles), OFFS(e->Wf1, hp::solve3_frag_doubles(e->nblk)),
+                            OFFS(e->Wf2, hp::solve3_frag_doubles(e->nblk)), philox ? OFFS(e->lam, Np) : nullptr};
+    const int nchol = hp::launch_chol_trinv(ca, OFFS(e->Wp, tri * hp::kLBlkDoubles), ex, sb.st);
+    e->prof_end(CLS_CHOL, nchol, sb.st);
 
     if (e->big_solve) {
         // x = W^H (W r + xi) as two dense products (W unpacked to a dense lower-triangular matrix): the path for
@@ -1122,7 +1119,7 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
         e->prof_end(CLS_SOLVE, nl, sb.st);
     } else if (e->solve2) {
         // k_solve2: right-hand sides in tile layout.  Philox mode: the unscaled Rfix tiles built at load time and
-        // W1 = W diag(lam) from k_trinv; injected draws: r = lam * Rfix + wa rebuilt per solve, W1 = W.
+        // W1 = W diag(lam) from k_chol_w; injected draws: r = lam * Rfix + wa rebuilt per solve, W1 = W.
         e->prof_begin(CLS_SOLVE, sb.st);
         int nl = 1;
         const double* wa_sb = (!philox && any_omega) ? OFFS(b.wa, 2 * Tp * Np) : nullptr;

@@ -7,14 +7,15 @@
 //
 //      M = J + D G D,   G = [Q|F]^H N^-1 [Q|F],   D = diag(lam, 1),   J = diag(1_n, 0_m)
 //
-// so that one iteration needs a Hermitian positive definite factorisation M = L L^H (k_chol)
-// and a two-sided triangular solve for all Ntimes right-hand sides (k_solve); every O(N^3) /
-// O(N^2 T) contraction runs on the FP64 tensor pipe (hp_mma.cuh).
+// so that one iteration needs a Hermitian positive definite factorisation M = L L^H with the explicit
+// inverse W = L^-1 (k_chol_w, here) and two triangular products x = W^H (W r + xi) for all Ntimes
+// right-hand sides (k_solve3, hp_solve3.cu); every O(N^3) / O(N^2 T) contraction runs on the FP64
+// tensor pipe (hp_mma.cuh).  Also here: the set-up kernels k_fourier_operator and k_pack_lower, the
+// residual / chi^2 / ln-posterior terms (k_post, k_colsumsq) and the power-spectrum draw (k_sample).
 #include "hp_kernels.cuh"
 #include "hp_math.h"
 #include "hp_mma.cuh"
 #include "hp_diag.cuh"
-#include <cstdlib>
 
 namespace hp {
 
@@ -27,119 +28,6 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src)
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-
-// global L block (padded layout: re plane [32][36], im plane [32][36]) -> the same layout in shared
-// memory (s: 2304 contiguous doubles), async
-__device__ __forceinline__ void load_block_async(double* s, const double* g) {
-    for (int c = threadIdx.x; c < kLBlkDoubles / 2; c += 256) cp_async16(s + 2 * c, g + 2 * c);
-}
-
-// ==========================================================================================
-// generic zgemm (set-up contractions and v1 basis transforms)
-constexpr int ZG_BM = 64, ZG_BN = 64, ZG_BK = 16;
-constexpr int ZG_LDA = 20;  // 16 + 4
-constexpr int ZG_LDB = 68;  // 64 + 4
-
-__global__ void __launch_bounds__(256, 2) k_zgemm(ZgemmArgs a) {
-    __shared__ double Asr[ZG_BM * ZG_LDA], Asi[ZG_BM * ZG_LDA];
-    __shared__ double Bsr[ZG_BK * ZG_LDB], Bsi[ZG_BK * ZG_LDB];
-    const int b = blockIdx.z;
-    const double* A = a.A + 2 * a.bsA * b;
-    const double* B = a.B + 2 * a.bsB * b;
-    double* C = a.C + 2 * a.bsC * b;
-    const double* dk = a.dk ? a.dk + a.bsD * b : nullptr;
-    const int i0 = blockIdx.y * ZG_BM, j0 = blockIdx.x * ZG_BN;
-    if (a.lower_out && j0 > i0 + ZG_BM - 1) return;   // Hermitian result: only tiles that touch the lower triangle
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int wr = warp >> 2, wc = warp & 3;  // warp tile 32 x 16
-    // (3M accumulation was tried here: 48 accumulators + the register double buffer exceed the 128 registers of two CTAs per
-    //  SM, and the spills cost more than the saved DMMAs: configs[4] solve 14.0 -> 15.3 ms)
-    double cr[4][2][2], ci[4][2][2];
-    warp_zero<4, 2>(cr, ci);
-    const bool a_kfast = a.sAk <= a.sAi;
-    const bool b_jfast = a.sBj <= a.sBk;
-    const double sgnA = a.conjA ? -1.0 : 1.0, sgnB = a.conjB ? -1.0 : 1.0;
-    // triangular B: skip the K range where this column tile of B is structurally zero
-    //   tri = 1: B[k][j] = 0 for k > j  (k < j0 + BN suffices);   tri = 2: B[k][j] = 0 for k < j  (start at k = j0)
-    const int kbeg = a.tri == 2 ? (j0 / ZG_BK) * ZG_BK : 0;
-    const int kend = a.tri == 1 ? (a.K < j0 + ZG_BN ? a.K : j0 + ZG_BN) : a.K;
-    // register double buffer: the global loads of k-tile t + 1 are in flight while tile t is multiplied
-    double2 ra[4], rb[4];
-    auto load_tile = [&](int k0) {
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const int e = tid + 256 * r;
-            int i, k;
-            if (a_kfast) { i = e >> 4; k = e & 15; } else { i = e & 63; k = e >> 6; }
-            double2 x = make_double2(0.0, 0.0);
-            if (i0 + i < a.M && k0 + k < kend) {
-                x = *reinterpret_cast<const double2*>(A + 2 * ((long long)(i0 + i) * a.sAi + (long long)(k0 + k) * a.sAk));
-                x.y *= sgnA;
-                if (dk) { const double d = dk[k0 + k]; x.x *= d; x.y *= d; }
-            }
-            ra[r] = x;
-        }
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const int e = tid + 256 * r;
-            int k, j;
-            if (b_jfast) { k = e >> 6; j = e & 63; } else { k = e & 15; j = e >> 4; }
-            double2 x = make_double2(0.0, 0.0);
-            if (k0 + k < kend && j0 + j < a.N) {
-                x = *reinterpret_cast<const double2*>(B + 2 * ((long long)(k0 + k) * a.sBk + (long long)(j0 + j) * a.sBj));
-                x.y *= sgnB;
-            }
-            rb[r] = x;
-        }
-    };
-    auto store_tile = [&]() {
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const int e = tid + 256 * r;
-            int i, k;
-            if (a_kfast) { i = e >> 4; k = e & 15; } else { i = e & 63; k = e >> 6; }
-            Asr[i * ZG_LDA + k] = ra[r].x; Asi[i * ZG_LDA + k] = ra[r].y;
-        }
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const int e = tid + 256 * r;
-            int k, j;
-            if (b_jfast) { k = e >> 6; j = e & 63; } else { k = e & 15; j = e >> 4; }
-            Bsr[k * ZG_LDB + j] = rb[r].x; Bsi[k * ZG_LDB + j] = rb[r].y;
-        }
-    };
-    if (kbeg < kend) load_tile(kbeg);
-    for (int k0 = kbeg; k0 < kend; k0 += ZG_BK) {
-        store_tile();
-        __syncthreads();
-        if (k0 + ZG_BK < kend) load_tile(k0 + ZG_BK);
-        warp_zgemm<4, 2, false, false, false, false>(cr, ci, Asr + 32 * wr * ZG_LDA, Asi + 32 * wr * ZG_LDA, ZG_LDA,
-                                                     Bsr + 16 * wc, Bsi + 16 * wc, ZG_LDB, ZG_BK);
-        __syncthreads();
-    }
-    const int g = lane >> 2, q = lane & 3;
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 2; ++j)
-#pragma unroll
-            for (int e = 0; e < 2; ++e) {
-                int row = i0 + 32 * wr + 8 * i + g, col = j0 + 16 * wc + 8 * j + 2 * q + e;
-                if (row < a.M && col < a.N) {
-                    double* p = C + 2 * ((long long)row * a.sCi + (long long)col * a.sCj);
-                    double vr = a.alpha * cr[i][j][e], vi = a.alpha * ci[i][j][e];
-                    if (a.accumulate) { vr += p[0]; vi += p[1]; }
-                    p[0] = vr; p[1] = vi;
-                }
-            }
-}
-
-// round-1 kernel, kept for A/B runs (HP_ZGEMM_V1=1); launch_zgemm is in hp_zgemm.cu
-void launch_zgemm_v1(const ZgemmArgs& a, cudaStream_t st) {
-    dim3 grid((a.N + ZG_BN - 1) / ZG_BN, (a.M + ZG_BM - 1) / ZG_BM, a.batch);
-    k_zgemm<<<grid, 256, 0, st>>>(a);
-}
 
 // ==========================================================================================
 __global__ void k_fourier_operator(double* out, int n, double scale) {
@@ -177,286 +65,19 @@ void launch_pack_lower(const double* dense, long long ld, long long bs, double* 
     k_pack_lower<<<dim3(nblk, nblk, batch), 256, 0, st>>>(dense, ld, bs, packed, N, nblk);
 }
 
-__global__ void k_scale_rows(double* A, const double* d, int rows, int cols, long long ld) {
-    long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (e >= (long long)rows * cols) return;
-    int r = (int)(e / cols), c = (int)(e % cols);
-    A[2 * (r * ld + c)] *= d[r];
-    A[2 * (r * ld + c) + 1] *= d[r];
-}
-void launch_scale_rows(double* A, const double* d, int rows, int cols, long long ld, cudaStream_t st) {
-    long long tot = (long long)rows * cols;
-    k_scale_rows<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(A, d, rows, cols, ld);
-}
-__global__ void k_fill(double* p, double v, size_t count) {
-    size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
-    if (e < count) p[e] = v;
-}
-void launch_fill(double* p, double v, size_t count, cudaStream_t st) {
-    if (count) k_fill<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(p, v, count);
-}
-
 // ==========================================================================================
-// k_chol: one CTA per system.  Left-looking blocked Cholesky of M = J + D G D with 32x32
-// blocks; M is never materialised (G blocks are scaled by lam on the fly).  Off-diagonal work
-// is DMMA; the 32x32 diagonal factorisation and its triangular inverse are done by all 256
-// threads in shared memory.
-constexpr int kCT = 512;  // threads of k_chol / k_trinv: 16 warps, one 8x8 tile of a 32x32 block each
+constexpr int kCT = 512;  // threads of k_chol_w: 16 warps, one 8x8 tile of a 32x32 block each
 
 // global L block -> shared memory, async, by all kCT threads
 __device__ __forceinline__ void load_block_async_ct(double* s, const double* g) {
     for (int c = threadIdx.x; c < kLBlkDoubles / 2; c += kCT) cp_async16(s + 2 * c, g + 2 * c);
 }
 
-struct CholSmem {
-    double A[2][2 * kLBlkDoubles];   // L_ij, L_i,j+1 (double buffered, two K blocks per stage); A[0] also holds the block being finished
-    double B[2][2 * kLBlkDoubles];   // L_kj, L_k,j+1 (double buffered)
-    double V[kLBlkDoubles];          // inverse of the current diagonal block
-};
-
-__global__ void __launch_bounds__(kCT) k_chol(CholArgs a) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    CholSmem& s = *reinterpret_cast<CholSmem*>(smem_raw);
-    const int sys = blockIdx.x;
-    const int nblk = a.nblk, Np = nblk * 32;
-    const double* Gp = a.Gp + (size_t)sys * tri_blocks(nblk) * kBlkDoubles;
-    double* Lp = a.Lp + (size_t)sys * tri_blocks(nblk) * kLBlkDoubles;
-    double* Linvp = a.Linvp + (size_t)sys * nblk * kLBlkDoubles;
-    const double* lam = a.lam + (size_t)sys * Np;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int g = lane >> 2, q = lane & 3;
-    const int ti = warp >> 2, tj = warp & 3;  // warp tile: rows 8 ti .. +8, cols 8 tj .. +8
-    double* Ar = s.A[0];
-    double* Ai = s.A[0] + kLPlane;
-    double* Vr = s.V;
-    double* Vi = s.V + kLPlane;
-    int bad = 0;
-
-    for (int k = 0; k < nblk; ++k) {
-        for (int i = k; i < nblk; ++i) {
-            double cr[1][1][2], ci[1][1][2];
-            warp_zero<1, 1>(cr, ci);
-            double P3m[3][1][1][2];
-            warp_zero3m<1, 1>(P3m);
-            // acc = sum_{j<k} L_ij . L_kj^H.  A stage holds two consecutive K blocks of both operands (blocks j, j + 1
-            // of a block row are contiguous in the packed layout): 64 DMMAs per warp between barriers.
-            auto issue = [&](int stg, int j0) {
-                const int cnt = (k - j0 < 2 ? k - j0 : 2) * (kLBlkDoubles / 2);
-                const double* ga = Lp + blk_index(i, j0) * kLBlkDoubles;
-                const double* gb = Lp + blk_index(k, j0) * kLBlkDoubles;
-                for (int c = tid; c < cnt; c += kCT) {
-                    cp_async16(s.A[stg] + 2 * c, ga + 2 * c);
-                    if (i != k) cp_async16(s.B[stg] + 2 * c, gb + 2 * c);
-                }
-                cp_async_commit();
-            };
-            __syncthreads();  // buffers free (previous block finished: its TRSM / write-out still read A[0] and V)
-            if (k > 0) issue(0, 0);
-            for (int j = 0, it = 0; j < k; j += 2, ++it) {
-                const int st = it & 1;
-                if (j + 2 < k) {
-                    issue(st ^ 1, j + 2);
-                    cp_async_wait<1>();
-                } else {
-                    cp_async_wait<0>();
-                }
-                __syncthreads();
-                const int nb = k - j < 2 ? k - j : 2;
-                for (int h = 0; h < nb; ++h) {
-                    const double* ar = s.A[st] + h * kLBlkDoubles;
-                    const double* br = (i != k) ? s.B[st] + h * kLBlkDoubles : ar;
-                    warp_zgemm3m<1, 1, false, false, true, true>(P3m, ar + 8 * ti * kLdBlk, ar + kLPlane + 8 * ti * kLdBlk, kLdBlk,
-                                                               br + 8 * tj * kLdBlk, br + kLPlane + 8 * tj * kLdBlk, kLdBlk, 32);
-                }
-                __syncthreads();  // stage st may be overwritten by the load issued in the next iteration
-            }
-            warp_zgemm3m_finish<1, 1, false, true>(P3m, cr, ci);
-            // C = M_ik - acc, M_ik = J + lam_i G_ik lam_k
-            const double* Gb = Gp + blk_index(i, k) * kBlkDoubles;
-#pragma unroll
-            for (int e = 0; e < 2; ++e) {
-                int r = 8 * ti + g, c = 8 * tj + 2 * q + e;
-                int gi = 32 * i + r, gj = 32 * k + c;
-                double sc = lam[gi] * lam[gj];
-                double vr = sc * Gb[r * 32 + c], vi = sc * Gb[1024 + r * 32 + c];
-                if (gi == gj && (gi < a.n || gi >= a.N)) vr += 1.0;
-                Ar[r * kLdBlk + c] = vr - cr[0][0][e];
-                Ai[r * kLdBlk + c] = vi - ci[0][0][e];
-            }
-            __syncthreads();
-            if (i == k) {
-                // ---- Cholesky of the 32x32 diagonal block and its inverse, blocked 8x8 (hp_diag.cuh)
-                if (diag_chol_inverse_block(Ar, Ai, Vr, Vi, tid, kCT)) bad = k + 1;
-                __syncthreads();
-                // write L_kk and V to global
-                double* Lb = Lp + blk_index(k, k) * kLBlkDoubles;
-                double* Vb = Linvp + (size_t)k * kLBlkDoubles;
-                for (int e = tid; e < kLBlkDoubles; e += kCT) {
-                    Lb[e] = s.A[0][e];
-                    Vb[e] = s.V[e];
-                }
-            } else {
-                // L_ik = C . V^H
-                double dr[1][1][2], di[1][1][2];
-                warp_zero<1, 1>(dr, di);
-            double Q3m[3][1][1][2];
-            warp_zero3m<1, 1>(Q3m);
-                warp_zgemm3m<1, 1, false, false, true, true>(Q3m, Ar + 8 * ti * kLdBlk, Ai + 8 * ti * kLdBlk, kLdBlk,
-                                                           Vr + 8 * tj * kLdBlk, Vi + 8 * tj * kLdBlk, kLdBlk, 32);
-                warp_zgemm3m_finish<1, 1, false, true>(Q3m, dr, di);
-                double* Lb = Lp + blk_index(i, k) * kLBlkDoubles;
-                int r = 8 * ti + g, c = 8 * tj + 2 * q;
-                *reinterpret_cast<double2*>(Lb + r * kLdBlk + c) = make_double2(dr[0][0][0], dr[0][0][1]);
-                *reinterpret_cast<double2*>(Lb + kLPlane + r * kLdBlk + c) = make_double2(di[0][0][0], di[0][0][1]);
-            }
-        }
-    }
-    __syncthreads();
-    if (tid == 0 && a.info) a.info[sys] = bad;
-}
-
-// ------------------------------------------------------------------------------------------
-// k_chol_col: the same factorisation, one block column per launch and one CTA per block.
-//   diag = 1: grid (1, nsys)            block (k, k): update, factorisation + inverse, writes L_kk and V_kk
-//   diag = 0: grid (nblk - k - 1, nsys) block (i, k), i = k + 1 + blockIdx.x: update, L_ik = C V_kk^H
-// Two launches per block column instead of one CTA walking the whole matrix: the blocks of a column are
-// independent, so a column's work spreads over (nblk - k) x nsys CTAs, two per SM.  With few systems resident
-// (32 per GPU at BASELINE.json configs[4], 33 block columns) k_chol leaves 116 of 148 SMs idle for the whole
-// factorisation; the critical path of the column version is one block per column.
-struct CholColSmem {
+struct CholWSmem {
     double A[2][kLBlkDoubles];   // L_ij (double buffered); A[0] also holds the block being finished
     double B[2][kLBlkDoubles];   // L_kj (double buffered)
     double V[kLBlkDoubles];      // V_kk
 };
-
-__global__ void __launch_bounds__(kCT, 2) k_chol_col(CholArgs a, int k, int diag) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    CholColSmem& s = *reinterpret_cast<CholColSmem*>(smem_raw);
-    const int sys = blockIdx.y;
-    const int i = diag ? k : k + 1 + (int)blockIdx.x;
-    const int nblk = a.nblk, Np = nblk * 32;
-    const double* Gp = a.Gp + (size_t)sys * tri_blocks(nblk) * kBlkDoubles;
-    double* Lp = a.Lp + (size_t)sys * tri_blocks(nblk) * kLBlkDoubles;
-    double* Linvp = a.Linvp + (size_t)sys * nblk * kLBlkDoubles;
-    const double* lam = a.lam + (size_t)sys * Np;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int g = lane >> 2, q = lane & 3;
-    const int ti = warp >> 2, tj = warp & 3;
-    double* Ar = s.A[0];
-    double* Ai = s.A[0] + kLPlane;
-    double* Vr = s.V;
-    double* Vi = s.V + kLPlane;
-
-    double cr[1][1][2], ci[1][1][2], P3m[3][1][1][2];
-    warp_zero<1, 1>(cr, ci);
-    warp_zero3m<1, 1>(P3m);
-    // this thread's two elements of M_ik = J + lam_i G_ik lam_k do not depend on the update: fetch them now, so that
-    // their global-load latency runs under the operand stream instead of after it
-    double mr_[2], mi_[2];
-    {
-        const double* Gb = Gp + blk_index(i, k) * kBlkDoubles;
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-            const int r = 8 * ti + g, c = 8 * tj + 2 * q + e;
-            const int gi = 32 * i + r, gj = 32 * k + c;
-            const double sc = lam[gi] * lam[gj];
-            mr_[e] = sc * Gb[r * 32 + c];
-            mi_[e] = sc * Gb[1024 + r * 32 + c];
-            if (gi == gj && (gi < a.n || gi >= a.N)) mr_[e] += 1.0;
-        }
-    }
-    if (!diag) load_block_async_ct(s.V, Linvp + (size_t)k * kLBlkDoubles);   // rides with the first operand stage
-    if (k > 0) {
-        load_block_async_ct(s.A[0], Lp + blk_index(i, 0) * kLBlkDoubles);
-        if (!diag) load_block_async_ct(s.B[0], Lp + blk_index(k, 0) * kLBlkDoubles);
-    }
-    cp_async_commit();
-    for (int j = 0; j < k; ++j) {
-        const int st = j & 1;
-        if (j + 1 < k) {
-            load_block_async_ct(s.A[st ^ 1], Lp + blk_index(i, j + 1) * kLBlkDoubles);
-            if (!diag) load_block_async_ct(s.B[st ^ 1], Lp + blk_index(k, j + 1) * kLBlkDoubles);
-            cp_async_commit();
-            cp_async_wait<1>();
-        } else {
-            cp_async_wait<0>();
-        }
-        __syncthreads();
-        const double* ar = s.A[st];
-        const double* br = diag ? s.A[st] : s.B[st];
-        warp_zgemm3m<1, 1, false, false, true, true>(P3m, ar + 8 * ti * kLdBlk, ar + kLPlane + 8 * ti * kLdBlk, kLdBlk,
-                                                     br + 8 * tj * kLdBlk, br + kLPlane + 8 * tj * kLdBlk, kLdBlk, 32);
-        __syncthreads();
-    }
-    cp_async_wait<0>();
-    __syncthreads();   // V_kk landed (k = 0: nothing else waited for it); A[0] is free
-    warp_zgemm3m_finish<1, 1, false, true>(P3m, cr, ci);
-#pragma unroll
-    for (int e = 0; e < 2; ++e) {
-        int r = 8 * ti + g, c = 8 * tj + 2 * q + e;
-        Ar[r * kLdBlk + c] = mr_[e] - cr[0][0][e];
-        Ai[r * kLdBlk + c] = mi_[e] - ci[0][0][e];
-    }
-    __syncthreads();
-    if (diag) {
-        const bool bad = diag_chol_inverse_block(Ar, Ai, Vr, Vi, tid, kCT);
-        __syncthreads();
-        double* Lb = Lp + blk_index(k, k) * kLBlkDoubles;
-        double* Vb = Linvp + (size_t)k * kLBlkDoubles;
-        for (int e = tid; e < kLBlkDoubles; e += kCT) {
-            Lb[e] = s.A[0][e];
-            Vb[e] = s.V[e];
-        }
-        if (bad && tid == 0 && a.info) atomicMax(a.info + sys, k + 1);
-    } else {
-        double dr[1][1][2], di[1][1][2], Q3m[3][1][1][2];
-        warp_zero3m<1, 1>(Q3m);
-        warp_zgemm3m<1, 1, false, false, true, true>(Q3m, Ar + 8 * ti * kLdBlk, Ai + 8 * ti * kLdBlk, kLdBlk, Vr + 8 * tj * kLdBlk,
-                                                     Vi + 8 * tj * kLdBlk, kLdBlk, 32);
-        warp_zgemm3m_finish<1, 1, false, true>(Q3m, dr, di);
-        double* Lb = Lp + blk_index(i, k) * kLBlkDoubles;
-        int r = 8 * ti + g, c = 8 * tj + 2 * q;
-        *reinterpret_cast<double2*>(Lb + r * kLdBlk + c) = make_double2(dr[0][0][0], dr[0][0][1]);
-        *reinterpret_cast<double2*>(Lb + kLPlane + r * kLdBlk + c) = make_double2(di[0][0][0], di[0][0][1]);
-    }
-}
-
-int launch_chol(const CholArgs& a, cudaStream_t st) {
-    static bool attr_dev[kMaxDev] = {false};
-    bool& attr_set = attr_dev[current_device_slot()];
-    static int mode = -1;   // HP_CHOL_COLUMNS = 0 (one CTA per system), 1 (one launch pair per block column), unset: auto
-    if (!attr_set) {
-        cudaFuncSetAttribute(k_chol, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CholSmem));
-        cudaFuncSetAttribute(k_chol_col, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CholColSmem));
-        const char* ev = getenv("HP_CHOL_COLUMNS");
-        mode = ev ? atoi(ev) : -1;
-        attr_set = true;
-    }
-    const bool columns = mode >= 0 ? mode == 1 : true;
-    if (!columns) {
-        k_chol<<<a.nsys, kCT, sizeof(CholSmem), st>>>(a);
-        return 1;
-    }
-    if (a.info) cudaMemsetAsync(a.info, 0, sizeof(int) * a.nsys, st);
-    for (int k = 0; k < a.nblk; ++k) {
-        k_chol_col<<<dim3(1, a.nsys), kCT, sizeof(CholColSmem), st>>>(a, k, 1);
-        if (k + 1 < a.nblk) k_chol_col<<<dim3(a.nblk - k - 1, a.nsys), kCT, sizeof(CholColSmem), st>>>(a, k, 0);
-    }
-    return 2 * a.nblk - 1;
-}
-
-// ==========================================================================================
-// k_trinv: W = L^-1 (block lower triangular), one CTA per (block column, system).
-//   W_jj = V_jj (inverse of the diagonal block, from k_chol)
-//   W_ij = -V_ii sum_{k=j}^{i-1} L_ik W_kj            (i > j)
-// With W explicit, both triangular solves of k_solve become plain block products without any
-// dependency between block rows.
-struct TrinvSmem {
-    double A[2][kLBlkDoubles];   // L_ik (double buffered); A[0] later holds the accumulated sum (as B operand)
-    double B[2][kLBlkDoubles];   // W_kj (double buffered)
-    double V[kLBlkDoubles];      // V_ii
-};
-
 // Fragment-major copies of W for k_solve3 (hp_solve3.cu).  One k-step (4 values of k) of one 16-row strip is 2 row groups x
 // 32 lanes x [re, im] = 128 doubles: lane 4 g + q holds A[8 wi + g][4 t + q] at [wi][lane][re, im], so that each of the two
 // 16-byte loads of a warp covers 512 contiguous, fully used bytes.
@@ -473,143 +94,31 @@ __device__ __forceinline__ void store_frag2(double* Wf2, int nblk, int R, int C,
     *reinterpret_cast<double2*>(d) = make_double2(re, im);
 }
 
-__global__ void __launch_bounds__(kCT) k_trinv(const double* __restrict__ Lp_all, const double* __restrict__ Linvp_all,
-                                               double* Wp_all, TrinvExtra ex, int nblk) {
-    double* Wp1_all = ex.Wp1;
-    const double* lam_all = ex.lam;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    TrinvSmem& s = *reinterpret_cast<TrinvSmem*>(smem_raw);
-    const int j = blockIdx.x, sys = blockIdx.y;
-    const double* Lp = Lp_all + (size_t)sys * tri_blocks(nblk) * kLBlkDoubles;
-    const double* Vp = Linvp_all + (size_t)sys * nblk * kLBlkDoubles;
-    double* Wp = Wp_all + (size_t)sys * tri_blocks(nblk) * kLBlkDoubles;
-    // W1 = W diag(lam): columns of block column j scaled by lam[32 j ..]
-    double* Wp1 = (Wp1_all && lam_all) ? Wp1_all + (size_t)sys * tri_blocks(nblk) * kLBlkDoubles : nullptr;
-    const double* lamj = lam_all ? lam_all + (size_t)sys * nblk * 32 + 32 * j : nullptr;
-    const size_t wf = (size_t)4 * nblk * (2 * nblk + 1) * 128;
-    double* Wf1 = ex.Wf1 ? ex.Wf1 + (size_t)sys * wf : nullptr;
-    double* Wf2 = ex.Wf2 ? ex.Wf2 + (size_t)sys * wf : nullptr;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int g = lane >> 2, q = lane & 3;
-    const int ti = warp >> 2, tj = warp & 3;
-    // W_jj = V_jj
-    for (int e = tid; e < kLBlkDoubles; e += kCT) {
-        const double v = Vp[(size_t)j * kLBlkDoubles + e];
-        Wp[blk_index(j, j) * kLBlkDoubles + e] = v;
-        if (Wp1) {
-            const int c = (e % kLPlane) % kLdBlk;
-            Wp1[blk_index(j, j) * kLBlkDoubles + e] = c < 32 ? v * lamj[c] : 0.0;
-        }
-    }
-    if (Wf1 || Wf2) {
-        // diagonal block (lower triangular, zeros above the diagonal are part of the 16-row strips' k range)
-        const double* Vb = Vp + (size_t)j * kLBlkDoubles;
-        for (int e = tid; e < 1024; e += kCT) {
-            const int r = e >> 5, c = e & 31;
-            const double re = Vb[r * kLdBlk + c], im = Vb[kLPlane + r * kLdBlk + c];
-            if (Wf1 && c < 16 * ((r >> 4) + 1)) {
-                const double l = lamj ? lamj[c] : 1.0;
-                store_frag1(Wf1, 32 * j + r, 32 * j + c, l * re, l * im);
-            }
-            if (Wf2 && r >= 16 * (c >> 4)) store_frag2(Wf2, nblk, 32 * j + r, 32 * j + c, re, im);
-        }
-    }
-    for (int i = j + 1; i < nblk; ++i) {
-        double cr[1][1][2], ci[1][1][2];
-        warp_zero<1, 1>(cr, ci);
-            double P3m[3][1][1][2];
-            warp_zero3m<1, 1>(P3m);
-        __syncthreads();  // buffers free; W blocks written by this CTA so far are visible
-        load_block_async_ct(s.V, Vp + (size_t)i * kLBlkDoubles);
-        load_block_async_ct(s.A[0], Lp + blk_index(i, j) * kLBlkDoubles);
-        load_block_async_ct(s.B[0], Wp + blk_index(j, j) * kLBlkDoubles);
-        cp_async_commit();
-        for (int k = j; k < i; ++k) {
-            const int st = (k - j) & 1;
-            // W_{k+1, j} was written at the end of the previous i iteration (k + 1 <= i - 1) -- visible
-            if (k + 1 < i) {
-                load_block_async_ct(s.A[st ^ 1], Lp + blk_index(i, k + 1) * kLBlkDoubles);
-                load_block_async_ct(s.B[st ^ 1], Wp + blk_index(k + 1, j) * kLBlkDoubles);
-                cp_async_commit();
-                cp_async_wait<1>();
-            } else {
-                cp_async_wait<0>();
-            }
-            __syncthreads();
-            warp_zgemm3m<1, 1, false, false, false, false>(P3m, s.A[st] + 8 * ti * kLdBlk, s.A[st] + kLPlane + 8 * ti * kLdBlk,
-                                                         kLdBlk, s.B[st] + 8 * tj, s.B[st] + kLPlane + 8 * tj, kLdBlk, 32);
-            __syncthreads();
-        }
-        warp_zgemm3m_finish<1, 1, false, false>(P3m, cr, ci);
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-            int r = 8 * ti + g, c = 8 * tj + 2 * q + e;
-            s.A[0][r * kLdBlk + c] = -cr[0][0][e];
-            s.A[0][kLPlane + r * kLdBlk + c] = -ci[0][0][e];
-        }
-        __syncthreads();
-        double dr[1][1][2], di[1][1][2];
-        warp_zero<1, 1>(dr, di);
-            double Q3m[3][1][1][2];
-            warp_zero3m<1, 1>(Q3m);
-        // V_ii is lower triangular: rows 8 ti.. only need k < 8 (ti + 1)
-        warp_zgemm3m<1, 1, false, false, false, false>(Q3m, s.V + 8 * ti * kLdBlk, s.V + kLPlane + 8 * ti * kLdBlk, kLdBlk,
-                                                     s.A[0] + 8 * tj, s.A[0] + kLPlane + 8 * tj, kLdBlk, 8 * (ti + 1));
-        warp_zgemm3m_finish<1, 1, false, false>(Q3m, dr, di);
-        double* Wb = Wp + blk_index(i, j) * kLBlkDoubles;
-        int r = 8 * ti + g, c = 8 * tj + 2 * q;
-        *reinterpret_cast<double2*>(Wb + r * kLdBlk + c) = make_double2(dr[0][0][0], dr[0][0][1]);
-        *reinterpret_cast<double2*>(Wb + kLPlane + r * kLdBlk + c) = make_double2(di[0][0][0], di[0][0][1]);
-        if (Wp1) {
-            double* Wb1 = Wp1 + blk_index(i, j) * kLBlkDoubles;
-            const double l0 = lamj[c], l1 = lamj[c + 1];
-            *reinterpret_cast<double2*>(Wb1 + r * kLdBlk + c) = make_double2(l0 * dr[0][0][0], l1 * dr[0][0][1]);
-            *reinterpret_cast<double2*>(Wb1 + kLPlane + r * kLdBlk + c) = make_double2(l0 * di[0][0][0], l1 * di[0][0][1]);
-        }
-        if (Wf1 || Wf2) {
-#pragma unroll
-            for (int e = 0; e < 2; ++e) {
-                const int R = 32 * i + r, C = 32 * j + c + e;
-                if (Wf1) {
-                    const double l = lamj ? lamj[c + e] : 1.0;
-                    store_frag1(Wf1, R, C, l * dr[0][0][e], l * di[0][0][e]);
-                }
-                if (Wf2) store_frag2(Wf2, nblk, R, C, dr[0][0][e], di[0][0][e]);
-            }
-        }
-    }
-}
-
-void launch_trinv(const double* Lp, const double* Linvp, double* Wp, const TrinvExtra& ex, int nblk, int nsys, cudaStream_t st) {
-    static bool attr_dev[kMaxDev] = {false};
-    bool& attr_set = attr_dev[current_device_slot()];
-    if (!attr_set) {
-        cudaFuncSetAttribute(k_trinv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TrinvSmem));
-        attr_set = true;
-    }
-    k_trinv<<<dim3(nblk, nsys), kCT, sizeof(TrinvSmem), st>>>(Lp, Linvp, Wp, ex, nblk);
-}
-
 // ------------------------------------------------------------------------------------------
-// k_chol_w: the block-column Cholesky of k_chol_col with the inverse W = L^-1 built on the way, row by row:
+// k_chol_w: left-looking blocked Cholesky of M = J + D G D with 32x32 blocks (M is never materialised: G blocks are
+// scaled by lam on the fly), with the inverse W = L^-1 built on the way, row by row:
 //      W_kk = V_kk,     W_kj' = -V_kk sum_{j = j'}^{k-1} L_kj W_jj'      (j' < k)
+// where V_kk = L_kk^-1 comes with the factorisation of the diagonal block (hp_diag.cuh).  Off-diagonal work is DMMA.
+// One launch per block column and one CTA per block: the blocks of a column are independent, so a column's work spreads
+// over (nblk - k) x nsys CTAs, where one CTA per system would leave 116 of 148 SMs idle with 32 systems resident
+// (BASELINE.json configs[4]).
 // Row k of W needs row k of L (finished by the panel launches of the columns < k), the rows < k of W and V_kk, i.e.
 // exactly what the panel launch of column k waits for: its grid takes the nblk - k - 1 panel blocks (i, k) AND the k
 // blocks (k, j') of W.  The number of CTAs per launch is nblk - 1 for every column, so the late columns, whose panels
-// leave most SMs idle (one or two blocks per system), carry most of the inverse: the separate k_trinv launch (0.65 ms at
-// the headline shape) disappears into launches that were under-filled.
+// leave most SMs idle (one or two blocks per system), carry most of the inverse: a separate launch for W (0.65 ms at the
+// headline shape) disappears into launches that were under-filled.
 // The diagonal block of the NEXT column rides along as well (look-ahead): block (k + 1, k + 1) needs row k + 1 of L up to
 // column k, and its last piece L_{k+1,k} is the first panel block of this launch -- the CTA that computes it goes on to
 // update, factor and invert block (k + 1, k + 1) while the other CTAs of the launch work through the rest of the column.
-// One launch per block column (plus one for block (0, 0)) instead of two: the 17 - 30 us of the latency-bound diagonal
-// kernels (128 CTAs with one 32 x 32 factorisation each) no longer sit between the launches.
-//   first = 1: grid (nsys, 1):        block (0, 0)
+// So the diagonal blocks need no launches of their own, which would be latency bound (128 CTAs with one 32 x 32
+// factorisation each, 17 - 30 us) and sit between the panel launches.
+//   first = 1: grid (nsys, 1):        block (0, 0) (for nblk = 1 the whole factorisation)
 //   first = 0: grid (nsys, nblk - 1): blockIdx.y = 0: panel block (k + 1, k), then diagonal block (k + 1, k + 1);
 //              0 < blockIdx.y < nblk - k - 1: panel block (k + 1 + blockIdx.y, k);  else W block (k, j')
 //              (systems along x: the look-ahead CTAs of all systems start in the first wave)
 __global__ void __launch_bounds__(kCT, 2) k_chol_w(CholArgs a, TrinvExtra ex, double* Wp_all, int k, int first) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    CholColSmem& s = *reinterpret_cast<CholColSmem*>(smem_raw);
+    CholWSmem& s = *reinterpret_cast<CholWSmem*>(smem_raw);
     const int sys = blockIdx.x;
     const int nblk = a.nblk, Np = nblk * 32;
     const int npanel = nblk - k - 1;
@@ -694,7 +203,7 @@ __global__ void __launch_bounds__(kCT, 2) k_chol_w(CholArgs a, TrinvExtra ex, do
         return;
     }
 
-    // ---- Cholesky block (i, kc): the update, then the factorisation + inverse (diag) or L_i,kc = C V_kc^H; as k_chol_col
+    // ---- Cholesky block (i, kc): the update, then the factorisation + inverse (diag) or L_i,kc = C V_kc^H
     auto chol_block = [&](int i, int kc, bool diag) {
         double cr[1][1][2], ci[1][1][2], P3m[3][1][1][2];
         warp_zero<1, 1>(cr, ci);
@@ -793,25 +302,18 @@ __global__ void __launch_bounds__(kCT, 2) k_chol_w(CholArgs a, TrinvExtra ex, do
     }
 }
 
-// Cholesky + explicit inverse of the factor in one sequence of block-column launches (nblk + 1 of them)
+// Cholesky + explicit inverse of the factor in one sequence of block-column launches
 int launch_chol_trinv(const CholArgs& a, double* Wp, const TrinvExtra& ex, cudaStream_t st) {
     static bool attr_dev[kMaxDev] = {false};
     bool& attr_set = attr_dev[current_device_slot()];
-    static int fused = -1;   // HP_CHOL_FUSED=0: k_chol_col + k_trinv (A/B runs)
     if (!attr_set) {
-        cudaFuncSetAttribute(k_chol_w, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CholColSmem));
-        const char* ev = getenv("HP_CHOL_FUSED");
-        fused = (ev && ev[0] == '0') ? 0 : 1;
+        cudaFuncSetAttribute(k_chol_w, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CholWSmem));
         attr_set = true;
     }
-    if (!fused || a.nblk < 2) {
-        const int n = launch_chol(a, st);
-        launch_trinv(a.Lp, a.Linvp, Wp, ex, a.nblk, a.nsys, st);
-        return n + 1;
-    }
     if (a.info) cudaMemsetAsync(a.info, 0, sizeof(int) * a.nsys, st);
-    k_chol_w<<<dim3(a.nsys, 1), kCT, sizeof(CholColSmem), st>>>(a, ex, Wp, 0, 1);
-    for (int k = 0; k < a.nblk; ++k) k_chol_w<<<dim3(a.nsys, a.nblk - 1), kCT, sizeof(CholColSmem), st>>>(a, ex, Wp, k, 0);
+    k_chol_w<<<dim3(a.nsys, 1), kCT, sizeof(CholWSmem), st>>>(a, ex, Wp, 0, 1);
+    if (a.nblk == 1) return 1;   // block (0, 0) is the whole matrix; the column launches would have no CTAs
+    for (int k = 0; k < a.nblk; ++k) k_chol_w<<<dim3(a.nsys, a.nblk - 1), kCT, sizeof(CholWSmem), st>>>(a, ex, Wp, k, 0);
     return a.nblk + 1;
 }
 

@@ -64,19 +64,19 @@ struct CholArgs {
     int* info;             // [nsys]  0 ok, k+1 = non-positive pivot in block column k
     int nblk, n, N, nsys;
 };
-int launch_chol(const CholArgs& a, cudaStream_t st);   // returns the number of kernel launches (1, or 2 nblk - 1 in column mode)
-// W = L^-1 in the same padded block layout as L ([nsys][tri_blocks][2304]); Wp1 (optional) receives W diag(lam), the
-// pass-1 operand of k_solve2 when the stored right-hand sides are unscaled (lam: [nsys][Np])
-//   ex.Wp1: W diag(lam) in block layout (k_solve2 pass 1);  ex.Wf1 / ex.Wf2: fragment-major copies for k_solve3
-//   (hp_solve3.cu: Wf1 = pass-1 operand, scaled by lam when ex.lam is given; Wf2 = W in pass-2 (transposed) fragment order)
+// Further copies of W = L^-1 that launch_chol_trinv writes besides Wp, each optional (null: not written):
+//   ex.Wp1: W diag(lam) in block layout, the pass-1 operand of k_solve2 when the stored right-hand sides are unscaled
+//           (written only when ex.lam is given; lam: [nsys][Np]);
+//   ex.Wf1 / ex.Wf2: fragment-major copies for k_solve3 (hp_solve3.cu: Wf1 = pass-1 operand, scaled by lam when ex.lam is
+//           given; Wf2 = W in pass-2 (transposed) fragment order), [nsys][solve3_frag_doubles]
 struct TrinvExtra { double* Wp1; double* Wf1; double* Wf2; const double* lam; };
-void launch_trinv(const double* Lp, const double* Linvp, double* Wp, const TrinvExtra& ex, int nblk, int nsys, cudaStream_t st);
-// Both in one sequence of block-column launches: the panel launch of column k also carries row k of W (k_chol_w).  Returns
-// the number of launches.  HP_CHOL_FUSED=0 falls back to launch_chol + launch_trinv.
+// M = L L^H and W = L^-1 (Wp: the padded block layout of L, [nsys][tri_blocks][2304]) in one sequence of block-column
+// launches of k_chol_w: the panel launch of column k also carries row k of W.  Returns the number of launches (1 for
+// nblk = 1, otherwise nblk + 1).
 int launch_chol_trinv(const CholArgs& a, double* Wp, const TrinvExtra& ex, cudaStream_t st);
 
 struct SolveArgs {
-    const double* Wp;      // [nsys][tri_blocks][2304]  W = L^-1 (k_trinv)
+    const double* Wp;      // [nsys][tri_blocks][2304]  W = L^-1 (launch_chol_trinv)
     const double* lam;     // [nsys][Np]
     const double* Rfix;    // [nsys][Tp][Np] complex: B^H N^-1 (w d)   (+ frozen noise term in numpy mode)
     const double* wa;      // [nsys][Tp][Np] complex or null: Q^H omega_a (rows < n)
@@ -260,7 +260,7 @@ struct PostFftArgs {
     long long w_bs, w_ts;  // w[sys * w_bs + t * w_ts + x]: (n, 0) time-invariant flags, (Tp n, n) per-time flags
     double* fg_out; double* chisq_out; long long fg_bs, chisq_bs;
     double* lnp1;          // [nsys][Tp]
-    double* Rm;            // [nsys][Tp][n] complex or null: w * resid (dense noise: ln_post term via k_zgemm)
+    double* Rm;            // [nsys][Tp][n] complex or null: w * resid (dense noise: ln_post term via k_zgemm2)
     double* Empart;        // [nsys][tiles][n] or null
     double* Eupart;        // [nsys][tiles][n] or null
     int m, Np, T, Tp, nsys, do_inverse;
@@ -272,10 +272,5 @@ bool make_fft2_plan(int n, FftPlan* fwd, FftPlan* rev);   // false: Nfreqs not c
 size_t postfft2_smem_bytes(int n, int m);
 bool launch_post_fft2(const PostFftArgs& a, const FftPlan& fwd, const FftPlan& rev, cudaStream_t st);
 bool launch_fft2_tables(double* tw2, const double* tw, int n, cudaStream_t st);   // tw2: 4 n doubles; false: Nfreqs not covered
-
-
-// small elementwise helpers used by the set-up
-void launch_scale_rows(double* A, const double* d, int rows, int cols, long long ld, cudaStream_t st);  // A[r][:] *= d[r]
-void launch_fill(double* p, double v, size_t count, cudaStream_t st);
 
 }  // namespace hp

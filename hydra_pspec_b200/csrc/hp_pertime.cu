@@ -13,10 +13,10 @@
 // M_t is never stored.  In the delay eigenbasis Q = U^H the signal block of G_t is circulant,
 // G_t[k][k'] = chat_t[(k - k') mod n] with chat_t the (shifted) DFT of w_t N^-1 / n, so a system is
 // described by n + (n + m) m numbers: chat_t and the foreground columns [Q|F]^H (w_t N^-1) F
-// (`H`, built once per baseline by k_zgemm when the chain is loaded).
+// (`H`, built once per baseline by k_zgemm2 when the chain is loaded).
 //
 // The factor L lives in a per-CTA global scratch slot (L2 / HBM), streamed through shared memory by
-// cp.async exactly as in k_chol.  The forward substitution y = L^-1 r is folded into the
+// cp.async, double buffered as in k_chol_w.  The forward substitution y = L^-1 r is folded into the
 // factorisation (the blocks L_kj pass through shared memory anyway when the diagonal block k is
 // updated), the Philox fluctuation xi ~ CN(0, I) is added to y, and the backward substitution
 // x = L^-H (y + xi) re-reads L once from the scratch slot.

@@ -1,7 +1,7 @@
 // hp_solve.cu -- k_solve: the GCR solve for all times of a baseline as two triangular block products.
 //
 // Replaces the per-time preconditioned CG of the reference (gcr_fgmodes_1d, pspec.py:151-235).
-// With M = L L^H (k_chol) and W = L^-1 formed explicitly (k_trinv), the solution for every time
+// With M = L L^H and W = L^-1 formed explicitly (k_chol_w), the solution for every time
 // sample is  x = W^H (W r [+ xi]):  two block-triangular products without any dependency between
 // block rows, instead of a substitution that serialises on every diagonal block.
 //

@@ -11,7 +11,7 @@
 //   * a warp owns whole 16-row strips of the output (16 x 16 complex register tile, 3M DMMA products, full K range): no K
 //     split, no partial-sum exchange, no ring.  Strips are dealt to the warps by a longest-first schedule computed on the
 //     host so that every scheduler (warp pair) gets the same number of k-steps;
-//   * the A operand never touches shared memory: k_trinv writes W in fragment-major order (per strip and k-step 2 row groups
+//   * the A operand never touches shared memory: k_chol_w writes W in fragment-major order (per strip and k-step 2 row groups
 //     x 32 lanes x [re, im] = 1 KiB contiguous), and every warp streams its own fragments from L2 into registers one
 //     k-step ahead, across strip, pass and tile boundaries (the schedule is static); four warps per scheduler hide the L2
 //     latency (a deeper register queue does not: ptxas gives all prefetch sites one scoreboard);

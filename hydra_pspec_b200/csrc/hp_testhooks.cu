@@ -52,8 +52,7 @@ int hp_test_chol_solve(int n, int m, int T, const double* G, const double* lam, 
     hp::launch_pack_lower(dG, N, 0, dGp, N, nblk, 1, 0);
     hp::CholArgs ca{};
     ca.Gp = dGp; ca.lam = dlam; ca.Lp = dLp; ca.Linvp = dLinv; ca.info = dinfo; ca.nblk = nblk; ca.n = n; ca.N = N; ca.nsys = 1;
-    hp::launch_chol(ca, 0);
-    hp::launch_trinv(dLp, dLinv, dWp, hp::TrinvExtra{nullptr, nullptr, nullptr, nullptr}, nblk, 1, 0);
+    hp::launch_chol_trinv(ca, dWp, hp::TrinvExtra{nullptr, nullptr, nullptr, nullptr}, 0);
     hp::SolveArgs sa{};
     sa.Wp = dWp; sa.lam = dlam; sa.Rfix = dR; sa.wa = dW; sa.X = dX; sa.Ssc = dS; sa.Ppart = dP;
     sa.nblk = nblk; sa.n = n; sa.N = N; sa.Tp = Tp; sa.ntiles = ntiles; sa.nsys = 1; sa.T = T; sa.cg_compat = cg_compat;
@@ -118,13 +117,12 @@ int hp_test_solve2(int n, int m, int T, int nsys, const double* G, const double*
     hp::launch_pack_lower(dG, N, 0, dGp, N, nblk, 1, 0);
     hp::CholArgs ca{};
     ca.Gp = dGp; ca.lam = dlam; ca.Lp = dLp; ca.Linvp = dLinv; ca.info = dinfo; ca.nblk = nblk; ca.n = n; ca.N = N; ca.nsys = 1;
-    hp::launch_chol(ca, 0);
     if (variant == 3) {
         cudaMalloc(&dWf1, 8 * wf * nsys); cudaMalloc(&dWf2, 8 * wf * nsys);
         cudaMemset(dWf1, 0xff, 8 * wf * nsys); cudaMemset(dWf2, 0xff, 8 * wf * nsys);   // NaN: every fragment must be written
     }
     // wa given: r = lam * Rfix + wa is built by k_rhs_tile and pass 1 uses the unscaled W
-    hp::launch_trinv(dLp, dLinv, dWp, hp::TrinvExtra{dWp1, dWf1, dWf2, wa ? nullptr : dlam}, nblk, 1, 0);
+    hp::launch_chol_trinv(ca, dWp, hp::TrinvExtra{dWp1, dWf1, dWf2, wa ? nullptr : dlam}, 0);
     if (variant != 3 && wa) cudaMemcpy(dWp1, dWp, 8 * tri, cudaMemcpyDeviceToDevice);
     for (int s = 0; s < nsys; ++s) {
         // lam is shared by the systems while k_rhs_tile indexes lam by system: build the tiles one system at a time

@@ -5,10 +5,9 @@
 // dense-noise ln-posterior term (pspec.py:474-478) per iteration (BASELINE.json configs[4]), and P = A^H R of the
 // per-time low-rank form (hp_ptlow.cu, configs[2]).
 //
-// The round-1 kernel (k_zgemm in hp_kernels.cu, kept as HP_ZGEMM_V1=1) stages 64 x 64 x 16 tiles through registers into
-// planar shared memory, 8 warps with 32 x 16 tiles and four real DMMAs per complex MAC: 0.60 of the DMMA peak at
-// configs[4].  This one follows what k_solve3 showed to work (profiles/r2_dmma_mix.txt: 12 DMMA + 4 DADD + 8 LDS per
-// k-step sustain 95 % of the pipe with four warps per scheduler):
+// The round-1 kernel staged 64 x 64 x 16 tiles through registers into planar shared memory, 8 warps with 32 x 16 tiles and
+// four real DMMAs per complex MAC: 0.60 of the DMMA peak at configs[4].  This one follows what k_solve3 showed to work
+// (profiles/r2_dmma_mix.txt: 12 DMMA + 4 DADD + 8 LDS per k-step sustain 95 % of the pipe with four warps per scheduler):
 //   * 16 warps, each a 16 x 16 complex tile with the 3M scheme (three real products per complex MAC, 48 accumulators);
 //   * operands go global -> shared with cp.async (16 bytes = one complex element, any stride, zero-filled outside the
 //     matrix or the triangular K range), three stages of 64 x 32 (A) and 32 x 64 (B), one barrier per 32-deep k-tile;
@@ -19,11 +18,8 @@
 // class 12.2 -> 12.5 ms, ln-posterior term 5.0 -> 5.2 ms even with a grid size coprime to the number of column tiles).
 #include "hp_kernels.cuh"
 #include "hp_mma.cuh"
-#include <cstdlib>
 
 namespace hp {
-void launch_zgemm_v1(const ZgemmArgs& a, cudaStream_t st);   // hp_kernels.cu
-
 namespace {
 
 constexpr int Z2_BM = 64, Z2_BN = 64, Z2_BK = 32, Z2_THREADS = 512, Z2_STAGES = 3;
@@ -147,9 +143,6 @@ __global__ void __launch_bounds__(Z2_THREADS, 1) k_zgemm2(ZgemmArgs a) {
 }  // namespace
 
 void launch_zgemm(const ZgemmArgs& a, cudaStream_t st) {
-    static int v1 = -1;
-    if (v1 < 0) { const char* ev = getenv("HP_ZGEMM_V1"); v1 = (ev && ev[0] == '1') ? 1 : 0; }
-    if (v1) { launch_zgemm_v1(a, st); return; }
     static bool attr_dev[kMaxDev] = {false};
     bool& done = attr_dev[current_device_slot()];
     if (!done) {

@@ -75,14 +75,15 @@ def test_chol_solve(n, m, T):
 
 def test_chol_reports_indefinite():
     L = _lib()
-    n, m, T = 40, 0, 4
-    G = -2.0 * np.eye(n, dtype=np.complex128)  # M = I - 2 I is negative definite
-    lam = np.ones(n)
-    Rfix = np.zeros((T, n), dtype=np.complex128)
-    X = np.empty((T, n), dtype=np.complex128)
-    info = np.zeros(1, dtype=np.int32)
-    L.check(L.lib().hp_test_chol_solve(n, m, T, L.ptr(G), L.ptr(lam), L.ptr(Rfix), None, 0, None, L.ptr(X), L.ptr(info)))
-    assert info[0] != 0
+    m, T = 0, 4
+    for n in (40, 20):   # two block columns; one block (the factorisation is k_chol_w's first launch only)
+        G = -2.0 * np.eye(n, dtype=np.complex128)  # M = I - 2 I is negative definite
+        lam = np.ones(n)
+        Rfix = np.zeros((T, n), dtype=np.complex128)
+        X = np.empty((T, n), dtype=np.complex128)
+        info = np.zeros(1, dtype=np.int32)
+        L.check(L.lib().hp_test_chol_solve(n, m, T, L.ptr(G), L.ptr(lam), L.ptr(Rfix), None, 0, None, L.ptr(X), L.ptr(info)))
+        assert info[0] != 0, n
 
 
 def test_arena_cache_and_deferred_setup_survive_engine_churn():
