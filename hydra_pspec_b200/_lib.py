@@ -13,6 +13,7 @@ HP_KEEP_CR, HP_KEEP_FG, HP_KEEP_CHISQ = 1, 2, 4
 (HP_BUF_PS, HP_BUF_LNPOST, HP_BUF_CR, HP_BUF_FG, HP_BUF_CHISQ, HP_BUF_LAST_CR, HP_BUF_LAST_FG,
  HP_BUF_PS_CUR) = range(8)
 HP_NUM_KERNEL_CLASSES = 6
+HP_SUMMARY_CR, HP_SUMMARY_FG = 1, 2
 
 
 class HPConfig(C.Structure):
@@ -59,6 +60,9 @@ _SIGNATURES = {
     "hp_engine_set_chain_ids": (C.c_int, [C.c_void_p, C.c_void_p]),
     "hp_engine_set_profile": (C.c_int, [C.c_void_p, C.c_int]),
     "hp_engine_launch_count": (C.c_longlong, [C.c_void_p]),
+    "hp_engine_set_summary": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
+    "hp_engine_read_summary": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t,
+                                         C.POINTER(C.c_int)]),
     "hp_engine_pt_form": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "hp_kernel_class_name": (C.c_char_p, [C.c_int]),
     "hp_sample_S": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -273,4 +273,15 @@ size_t postfft2_smem_bytes(int n, int m);
 bool launch_post_fft2(const PostFftArgs& a, const FftPlan& fwd, const FftPlan& rev, cudaStream_t st);
 bool launch_fft2_tables(double* tw2, const double* tw, int n, cudaStream_t st);   // tw2: 4 n doubles; false: Nfreqs not covered
 
+// k_moments (hp_moments.cu): Welford update of per-chain posterior moments from one iteration's samples.
+// Element i < L of chain c is src[c * src_cs + (i / w) * rs + i % w] (complex); its accumulators are mean[c * ld + i]
+// (complex) and m2[c * ld + i] (real), ld even.  src = NULL or L = 0: nothing to update.
+struct MomentsArr {
+    const double* src; long long src_cs; int w, rs;
+    int L, nsys; long long ld;
+    double* mean; double* m2;
+};
+// one launch for both arrays (returns the number of launches, 0 or 1); invk = 1 / (accumulated iterations including this one)
+int launch_moments(const MomentsArr& cr, const MomentsArr& fg, double invk, cudaStream_t st);
+
 }  // namespace hp

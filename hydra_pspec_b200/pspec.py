@@ -268,6 +268,7 @@ class GibbsEngine:
         self.keep = tuple(keep)
         self.general_basis0 = bool(general_basis0)
         self.time_flags = bool(time_flags)
+        self.summary_what = ()
 
     def close(self):
         if self._h is not None:
@@ -446,12 +447,87 @@ class GibbsEngine:
         _lib.check(_lib.lib().hp_engine_read_signal_S(self._h, int(chain), _lib.ptr(out)))
         return out
 
+    # -- posterior summary (hp_engine_set_summary)
+    _SUMMARY = {"cr": (_lib.HP_SUMMARY_CR, "signal_cr"), "fg": (_lib.HP_SUMMARY_FG, "fg_amps")}
+
+    def set_summary(self, what=("cr", "fg"), burn_in=0, thin=1):
+        """(Re)start the on-device posterior moments of ``signal_cr`` ("cr") and / or ``fg_amps`` ("fg"): of the iterations
+        computed from now on the first ``burn_in`` are skipped, then every ``thin``-th is accumulated.  ``what=()`` stops."""
+        what = tuple(what)
+        bad = [w for w in what if w not in self._SUMMARY]
+        if bad:
+            raise ValueError(f"set_summary: unknown quantities {bad} (expected 'cr' and / or 'fg')")
+        mask = 0
+        for w in what:
+            mask |= self._SUMMARY[w][0]
+        _lib.check(_lib.lib().hp_engine_set_summary(self._h, mask, int(burn_in), int(thin)))
+        self.summary_what = what
+
+    def summary(self, chain):
+        """``{"count", "signal_cr_mean", "signal_cr_var", "fg_amps_mean", "fg_amps_var"}`` of one chain, with only the
+        quantities being accumulated: means (Ntimes, Nfreqs | Nmodes) complex128, variances E|x - mean|^2 (ddof = 0, as
+        ``numpy.var`` of the complex samples), count = accumulated iterations."""
+        if not self.summary_what:
+            raise ValueError("summary: no posterior summary is being accumulated (set_summary)")
+        out = {}
+        count = _lib.C.c_int(0)
+        for w in self.summary_what:
+            bit, name = self._SUMMARY[w]
+            width = self.nfreqs if w == "cr" else self.nmodes
+            mean = np.empty((self.ntimes, width), dtype=np.complex128)
+            var = np.empty((self.ntimes, width), dtype=np.float64)
+            _lib.check(_lib.lib().hp_engine_read_summary(self._h, int(chain), bit, _lib.ptr(mean), _lib.ptr(var), mean.nbytes,
+                                                         _lib.C.byref(count)))
+            out[f"{name}_mean"], out[f"{name}_var"] = mean, var
+        out["count"] = int(count.value)
+        return out
+
 
 
 # Device slots of the big per-iteration outputs when they are streamed to the host (cfg.ring_iters): the device footprint
 # of a chain does not grow with Niter (the reference keeps one baseline's samples in host RAM, pspec.py:590-596).
 _RING_ITERS = 3
 _STAGING_BYTES = int(float(os.environ.get("HP_STAGING_GB", "2")) * 2 ** 30)   # page-locked staging area
+
+
+def _device_bytes_per_chain(ntimes, nfreqs, nmodes, Niter, rng, big_per_iter, general, dense, per_time, summary):
+    """Estimated device memory of one chain of an engine (how many chains share an engine in gibbs_sample_batch).
+    ``big_per_iter``: host bytes of one chain's kept outputs per iteration (``_big_bytes_per_iter`` / nchains)."""
+    Np = 32 * ((nfreqs + nmodes + 31) // 32)
+    Tp = 16 * ((ntimes + 15) // 16)
+    per_chain = 16 * Tp * Np * (4 if rng == "numpy" else 3) + 16 * Tp * nfreqs * 3 + 16 * nfreqs * Np * (2 if general else 1) \
+        + 8 * 3 * (Np * Np // 2 + 18 * Np) * 2 + _RING_ITERS * big_per_iter + 8 * Niter * nfreqs * (2 if rng == "numpy" else 1)
+    if dense:
+        per_chain += 16 * nfreqs * nfreqs * 3 + 16 * Tp * nfreqs * 2
+    if per_time:
+        # low-rank form (csrc/hp_ptlow.cu): Nfreqs more right-hand sides ride through the solve, plus P and the flag lists
+        Tx = Tp + 16 * ((nfreqs + 15) // 16)
+        per_chain = per_chain * Tx // Tp + 16 * Tx * (1 + nmodes) * Np + 8 * Tx * nfreqs + 16 * nfreqs * nfreqs + 132 * ntimes
+    if summary:
+        per_chain += 24 * ntimes * (nfreqs + nmodes)   # posterior moments: complex mean + real M2 per element
+    return per_chain
+
+
+def _check_summary(summary):
+    """Validate the ``summary=`` argument of the sampling functions: None, or a dict with the optional keys ``burn_in``
+    (integer >= 0, default 0) and ``thin`` (integer >= 1, default 1).  Returns None or ``{"burn_in", "thin"}``."""
+    if summary is None:
+        return None
+    if not isinstance(summary, dict):
+        raise TypeError("summary must be None or a dict(burn_in=..., thin=...)")
+    unknown = set(summary) - {"burn_in", "thin"}
+    if unknown:
+        raise ValueError(f"summary: unknown keys {sorted(unknown)} (expected burn_in, thin)")
+    out = {"burn_in": summary.get("burn_in", 0), "thin": summary.get("thin", 1)}
+    for k, v in out.items():
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)):
+            raise TypeError(f"summary: {k} must be an integer")
+        out[k] = int(v)
+    if out["burn_in"] < 0:
+        raise ValueError("summary: burn_in must be >= 0")
+    if out["thin"] < 1:
+        raise ValueError("summary: thin must be >= 1")
+    return out
 
 
 def _big_bytes_per_iter(nchains, ntimes, nfreqs, nmodes, keep):
@@ -671,14 +747,18 @@ def gibbs_step_fgmodes(vis, flags, signal_S, fgmodes, Ninv, ps_prior=None, f0=No
 
 def gibbs_sample_with_fg(vis, flags, S_initial, fgmodes, Ninv, ps_prior, Niter=100, seed=None, verbose=True,
                          nproc=1, write_Niter=100, out_dir=None, map_estimate=False, rng="numpy", solver=None,
-                         device=0):
+                         device=0, summary=None):
     """Gibbs chain for one baseline (pspec.py:493-658); same arguments and return tuple:
     ``signal_cr, signal_S, signal_ps, fg_amps, chisq, ln_post, write_time``.
 
     Extra keyword arguments: ``rng`` / ``solver`` (see the module docstring) and ``device``.
     ``nproc`` is accepted and ignored (all times are solved in one batched launch).
+    ``summary=dict(burn_in=..., thin=...)``: the posterior moments of signal_cr and fg_amps are accumulated on the device
+    (:meth:`GibbsEngine.set_summary`) and returned as an 8th element, the dict of :meth:`GibbsEngine.summary`; with
+    ``out_dir`` they are also written (``utils.write_summary_files``) at every ``write_Niter`` boundary and at the end.
     """
     t_start = time.perf_counter()
+    summary = _check_summary(summary)
     if map_estimate:
         Niter = 1
         write_Niter = 1
@@ -702,7 +782,10 @@ def gibbs_sample_with_fg(vis, flags, S_initial, fgmodes, Ninv, ps_prior, Niter=1
     eng = _single_chain_engine(vis, flags, S_initial, fgmodes, Ninv, pr, Niter, rng, solver, map_estimate,
                                ("cr", "fg", "chisq"), seed, device, s_uniforms=u, ring_iters=_RING_ITERS)
     write_time = [0.0]
+    moments = None
     try:
+        if summary is not None:
+            eng.set_summary(("cr", "fg"), **summary)
         # the reference's return arrays (pspec.py:590-596), filled chunk by chunk from a bounded page-locked staging area
         signal_cr = np.empty((1, Niter, ntimes, nfreqs), dtype=np.complex128)
         signal_ps = np.empty((1, Niter, nfreqs))
@@ -715,6 +798,8 @@ def gibbs_sample_with_fg(vis, flags, S_initial, fgmodes, Ninv, ps_prior, Niter=1
             t0 = time.perf_counter()
             utils.write_numpy_files(out_dir, signal_cr[0, :done], eng.signal_S(0), signal_ps[0, :done], fg_amps[0, :done],
                                     chisq[0, :done], ln_post[0, :done])
+            if summary is not None:
+                utils.write_summary_files(out_dir, eng.summary(0), **summary)
             write_time[0] += time.perf_counter() - t0
 
         _staged_run(eng, Niter, dest, write_Niter=write_Niter if out_dir is not None else None,
@@ -724,6 +809,8 @@ def gibbs_sample_with_fg(vis, flags, S_initial, fgmodes, Ninv, ps_prior, Niter=1
             raise np.linalg.LinAlgError("GCR system not positive definite (Cholesky failed in block column "
                                         f"{int(bad[0]) - 1})")
         signal_S = eng.signal_S(0)
+        if summary is not None:
+            moments = eng.summary(0)
         signal_cr, signal_ps, fg_amps, chisq, ln_post = signal_cr[0], signal_ps[0], fg_amps[0], chisq[0], ln_post[0]
     finally:
         eng.close()
@@ -743,11 +830,13 @@ def gibbs_sample_with_fg(vis, flags, S_initial, fgmodes, Ninv, ps_prior, Niter=1
             res = "exact" if eff != "reference-cg" else "(cg)"
             print(f"{i + 1:<9d}{per_it:<12.4f}{0.0:<8.1f}{res:<12s}{cs}{lp:<12.1f}")
         print()
+    if summary is not None:
+        return signal_cr, signal_S, signal_ps, fg_amps, chisq, ln_post, write_time, moments
     return signal_cr, signal_S, signal_ps, fg_amps, chisq, ln_post, write_time
 
 
 def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=None, keep=("cr", "fg", "chisq"),
-                       write_Niter=100, map_estimate=False, device=0, verbose=False, substreams=1, chain_ids=None):
+                       write_Niter=100, map_estimate=False, device=0, verbose=False, substreams=1, chain_ids=None, summary=None):
     """Advance the Gibbs chains of several baselines of identical shape together on one GPU.
 
     This is the batched form of the reference's per-rank loop over baselines
@@ -757,7 +846,13 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
     them.  Returns one ``gibbs_sample_with_fg``-style tuple per baseline (arrays that were not kept
     are ``None``).  With ``rng="numpy"`` each chain gets the reference's draws for ``seed`` (every
     baseline the same streams, as in the reference, where each chain reseeds numpy).
+
+    ``summary=dict(burn_in=..., thin=...)``: the posterior moments of signal_cr and fg_amps are accumulated on the device
+    and each tuple gains an 8th element, the dict of :meth:`GibbsEngine.summary`.  Baselines with an ``out_dir`` also get
+    them written (``utils.write_summary_files``) at every ``write_Niter`` boundary and at the end.  With ``keep=()`` only
+    signal_ps / ln_post leave the device per iteration, and no ``out_dir`` is needed however long the chain.
     """
+    summary = _check_summary(summary)
     if not baselines:
         return []
     if map_estimate:
@@ -837,20 +932,13 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
 
     # ---- how many chains share an engine: all of them unless the device arena would not fit (then groups run one after
     # the other; the Philox chain ids keep the samples independent of the grouping)
-    Np = 32 * ((nfreqs + nmodes + 31) // 32)
-    Tp = 16 * ((ntimes + 15) // 16)
-    per_chain = 16 * Tp * Np * (4 if rng == "numpy" else 3) + 16 * Tp * nfreqs * 3 + 16 * nfreqs * Np * (2 if general else 1) \
-        + 8 * 3 * (Np * Np // 2 + 18 * Np) * 2 + _RING_ITERS * per_iter // nb + 8 * Niter * nfreqs * (2 if rng == "numpy" else 1)
-    if dense:
-        per_chain += 16 * nfreqs * nfreqs * 3 + 16 * Tp * nfreqs * 2
-    if per_time:
-        # low-rank form (csrc/hp_ptlow.cu): Nfreqs more right-hand sides ride through the solve, plus P and the flag lists
-        Tx = Tp + 16 * ((nfreqs + 15) // 16)
-        per_chain = per_chain * Tx // Tp + 16 * Tx * (1 + nmodes) * Np + 8 * Tx * nfreqs + 16 * nfreqs * nfreqs + 132 * ntimes
+    per_chain = _device_bytes_per_chain(ntimes, nfreqs, nmodes, Niter, rng, per_iter // nb, general, dense, per_time,
+                                        summary is not None)
     dev_budget = float(os.environ.get("HP_DEVICE_BUDGET_GB", "150")) * 2 ** 30
     group = max(1, min(nb, int(dev_budget // per_chain)))
     write_times = [0.0] * nb
     signal_S = [None] * nb
+    moments = [None] * nb
     any_out = any(b.get("out_dir") is not None for b in baselines)
 
     for g0 in range(0, nb, group):
@@ -875,6 +963,8 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
                                ninv_dense=nD, nih_dense=nH)
                 if rng == "numpy":
                     eng.set_draws(lc, oma, omb, _s_draws_from_uniforms(u, p["prior"], ntimes))
+            if summary is not None:
+                eng.set_summary(("cr", "fg"), **summary)
 
             class _Dest:
                 """[chain][iteration] view over the per-baseline destination arrays of this group."""
@@ -898,7 +988,19 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
                         continue
                     t0 = time.perf_counter()
                     r = results[c]
-                    if in_ram:
+                    if summary is not None:
+                        # the sample files of the kept arrays only, and the moments
+                        for k, (_, _, _, fname) in shapes.items():
+                            if r[k] is not None:
+                                if in_ram:
+                                    np.save(os.path.join(str(b["out_dir"]), fname), r[k][:done])
+                                else:
+                                    r[k].flush()
+                        np.save(os.path.join(str(b["out_dir"]), "cov-eor.npy"), eng.signal_S(lc))
+                        np.save(os.path.join(str(b["out_dir"]), "dps-eor.npy"), r["signal_ps"][:done])
+                        np.save(os.path.join(str(b["out_dir"]), "ln-post.npy"), r["ln_post"][:done])
+                        utils.write_summary_files(b["out_dir"], eng.summary(lc), **summary)
+                    elif in_ram:
                         z = lambda k: r[k][:done] if r[k] is not None else np.zeros(0)  # noqa: E731
                         utils.write_numpy_files(b["out_dir"], z("signal_cr"), eng.signal_S(lc), r["signal_ps"][:done],
                                                 z("fg_amps"), z("chisq"), r["ln_post"][:done])
@@ -919,10 +1021,12 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
                                             f"(Cholesky failed in block column {int(bad[lc]) - 1})")
             for lc, c in enumerate(cs):
                 signal_S[c] = eng.signal_S(lc)
+                if summary is not None:
+                    moments[c] = eng.summary(lc)
         finally:
             eng.close()
     out = [(results[c]["signal_cr"], signal_S[c], results[c]["signal_ps"], results[c]["fg_amps"], results[c]["chisq"],
-            results[c]["ln_post"], write_times[c]) for c in range(nb)]
+            results[c]["ln_post"], write_times[c]) + ((moments[c],) if summary is not None else ()) for c in range(nb)]
     if verbose:
         for c in range(nb):
             print(f"baseline {c}: ln_post[-1] = {out[c][5][-1]:.1f}")

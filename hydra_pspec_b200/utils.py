@@ -31,6 +31,19 @@ def write_numpy_files(fp, signal_cr, signal_S, signal_ps, fg_amps, chisq, ln_pos
     np.save(fp / "ln-post.npy", ln_post)
 
 
+def write_summary_files(fp, moments, burn_in, thin):
+    """Posterior moments of a chain (``GibbsEngine.summary``): ``gcr-eor-mean.npy`` / ``gcr-eor-var.npy`` (signal_cr),
+    ``fg-amps-mean.npy`` / ``fg-amps-var.npy`` (fg_amps) and ``summary.json`` (count, burn_in, thin)."""
+    import json
+    fp = Path(fp)
+    for key, stem in (("signal_cr", "gcr-eor"), ("fg_amps", "fg-amps")):
+        if f"{key}_mean" in moments:
+            np.save(fp / f"{stem}-mean.npy", moments[f"{key}_mean"])
+            np.save(fp / f"{stem}-var.npy", moments[f"{key}_var"])
+    with open(fp / "summary.json", "w") as f:
+        json.dump({"count": int(moments["count"]), "burn_in": int(burn_in), "thin": int(thin)}, f, indent=2)
+
+
 def filter_freqs(freq_str, freqs_in):
     """Subset of ``freqs_in`` (MHz) selected by ``freq_str`` (hydra_pspec/utils.py:137-196): a single
     frequency, a comma list (closest channels are kept) or ``'lo-hi'``.  Plain floats in MHz stand in

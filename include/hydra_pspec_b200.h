@@ -159,6 +159,26 @@ int hp_engine_rewind(hp_engine* e);
 
 /* Copy results to the host.  iter0/niter select iterations for the per-iteration buffers. */
 int hp_engine_read(hp_engine* e, int chain, int buffer, int iter0, int niter, void* dst, size_t dst_bytes);
+
+/* Posterior moments accumulated on the device (csrc/hp_moments.cu).  Instead of streaming every sample of signal_cr /
+ * fg_amps to the host and reducing it there, the engine keeps a running mean and variance per (chain, time, channel) and
+ * (chain, time, mode), updated in FP64 in iteration order (Welford): the moments of a chain are bit-identical however its
+ * iterations were split over hp_engine_run / hp_engine_run_to_host calls, sub-streams or read-ahead.  The accumulators
+ * (24 bytes per complex element and chain) are allocated when first asked for, outside the creation-time arena.  Enabling
+ * the summary changes no draw and no output of the chain; it needs no HP_KEEP_* bit.  hp_engine_gcr does not accumulate;
+ * hp_engine_rewind keeps the accumulators.  Replaces the host-side reduction of the reference's sample arrays
+ * (pspec.py:590-596). */
+enum hp_summary_what { HP_SUMMARY_CR = 1, HP_SUMMARY_FG = 2 };
+/* (Re)start on-device posterior moments: accumulators zeroed; of the iterations computed from now on the first
+ * burn_in are skipped, then every thin-th is accumulated (burn_in >= 0, thin >= 1).  what = 0 stops accumulating.
+ * Refused while read-ahead iterations are pending. */
+int hp_engine_set_summary(hp_engine* e, int what, int burn_in, int thin);
+/* mean [T][n|m] complex128 and var [T][n|m] double (E|x - mean|^2 over the accumulated iterations, ddof = 0, i.e.
+ * numpy.var of the complex samples); either may be NULL.  *count = accumulated iterations.  what = one HP_SUMMARY_* bit.
+ * bytes_each: capacity of each destination (mean needs 16 T n|m bytes, var 8 T n|m).  With count = 0 both read as zeros.
+ * Refused (HP_ERR_ARG) for a quantity that is not being accumulated and while read-ahead iterations are pending. */
+int hp_engine_read_summary(hp_engine* e, int chain, int what, double* mean, double* var, size_t bytes_each, int* count);
+
 /* signal_S of the reference's return value: F^H diag(ps / Nfreqs^2) F for the current spectrum
  * (covariance_from_pspec, pspec.py:313-322).  dst [Nfreqs][Nfreqs] complex128. */
 int hp_engine_read_signal_S(hp_engine* e, int chain, double* dst);

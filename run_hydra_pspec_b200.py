@@ -18,6 +18,10 @@ Same command line, config file keys, input files and output files as the referen
 * uvh5 input goes through pyuvdata when it is importable, else through the built-in reader
   (``hydra_pspec_b200.uvh5``).
 * ``--Nproc`` is accepted and ignored (all times of all resident baselines are solved in one launch).
+* ``--samples summary`` (or ``both``) writes the posterior mean and variance of the in-painted signal and of the foreground
+  amplitudes after ``--burn_in`` iterations, thinned by ``--thin``, accumulated on the GPU: ``gcr-eor-mean.npy``,
+  ``gcr-eor-var.npy``, ``fg-amps-mean.npy``, ``fg-amps-var.npy`` and ``summary.json``.  With ``summary`` the per-sample files
+  ``gcr-eor.npy`` / ``fg-amps.npy`` / ``chisq.npy`` are not written, and those samples never leave the GPU.
 """
 import argparse
 import json
@@ -73,6 +77,12 @@ def build_parser():
     p.add_argument("--time_flags", choices=("any", "per-time"), default="any",
                    help="any: a channel flagged at any time is flagged at all times (the reference, "
                         "run-hydra-pspec.py:520-526); per-time: keep the (Ntimes, Nfreqs) flags (in-painting)")
+    p.add_argument("--samples", choices=("all", "summary", "both"), default="all",
+                   help="all: every sample of signal_cr / fg_amps / chisq (gcr-eor.npy, fg-amps.npy, chisq.npy); summary: only "
+                        "their posterior mean and variance, accumulated on the GPU (gcr-eor-mean.npy, gcr-eor-var.npy, "
+                        "fg-amps-mean.npy, fg-amps-var.npy, summary.json); both: the two")
+    p.add_argument("--burn_in", type=int, default=0, help="--samples summary / both: iterations skipped before accumulating")
+    p.add_argument("--thin", type=int, default=1, help="--samples summary / both: accumulate every thin-th iteration")
     return p
 
 
@@ -230,6 +240,9 @@ def time_invariant_flags(w):
 
 def main(argv=None):
     parser, args = parse_args(argv)
+    if args.burn_in < 0 or args.thin < 1:
+        parser.error("--burn_in must be >= 0 and --thin >= 1")
+    summary = None if args.samples == "all" else dict(burn_in=args.burn_in, thin=args.thin)
     rank = int(os.environ.get("RANK", "0"))
     size = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -302,23 +315,31 @@ def main(argv=None):
         for job in jobs:  # one chain after the other, the reference's streams
             if verbose:
                 print(f"Printing status messages for:\nRank:     {rank}\nBaseline: {job['antpair']}", end="\n\n")
-            res = pspec.gibbs_sample_with_fg(job["vis"], job["flags"], job["S_initial"], job["fgmodes"], job["Ninv"],
-                                             job["ps_prior"], Niter=args.Niter, seed=args.seed,
-                                             map_estimate=args.map_estimate, verbose=verbose, nproc=args.Nproc,
-                                             write_Niter=args.write_Niter, out_dir=job["out_dir"], rng="numpy",
-                                             solver=args.solver, device=local_rank)
+            if args.samples == "summary":
+                # the same chain through the batched form, which can leave the samples on the device (keep=())
+                res = pspec.gibbs_sample_batch([job], Niter=args.Niter, seed=args.seed, rng="numpy", solver=args.solver,
+                                               keep=(), write_Niter=args.write_Niter, map_estimate=args.map_estimate,
+                                               device=local_rank, verbose=verbose, summary=summary)[0]
+            else:
+                res = pspec.gibbs_sample_with_fg(job["vis"], job["flags"], job["S_initial"], job["fgmodes"], job["Ninv"],
+                                                 job["ps_prior"], Niter=args.Niter, seed=args.seed,
+                                                 map_estimate=args.map_estimate, verbose=verbose, nproc=args.Nproc,
+                                                 write_Niter=args.write_Niter, out_dir=job["out_dir"], rng="numpy",
+                                                 solver=args.solver, device=local_rank, summary=summary)
             ant_pairs.append(f"{job['antpair'][0]}_{job['antpair'][1]}")
-            write_times.append(res[-1])
+            write_times.append(res[6])
     else:
         # one Philox key for the whole job, chain id = global baseline index: the samples of a baseline do not
         # depend on the number of ranks / GPUs
         seed = 0 if args.seed is None else args.seed
+        keep = () if args.samples == "summary" else ("cr", "fg", "chisq")
         res = pspec.gibbs_sample_batch(jobs, Niter=args.Niter, seed=int(seed) & 0xFFFFFFFFFFFFFFFF, rng="philox",
-                                       solver=args.solver, write_Niter=args.write_Niter, map_estimate=args.map_estimate,
-                                       device=local_rank, verbose=verbose, chain_ids=global_ids)
+                                       solver=args.solver, keep=keep, write_Niter=args.write_Niter,
+                                       map_estimate=args.map_estimate, device=local_rank, verbose=verbose,
+                                       chain_ids=global_ids, summary=summary)
         for job, r in zip(jobs, res):
             ant_pairs.append(f"{job['antpair'][0]}_{job['antpair'][1]}")
-            write_times.append(r[-1])
+            write_times.append(r[6])
     write_timings = {"rank": rank, "ant_pairs": ant_pairs, "write_times": write_times}
     if dist is not None:
         gathered = [None] * size
