@@ -63,6 +63,9 @@ _SIGNATURES = {
     "hp_engine_set_summary": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
     "hp_engine_read_summary": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t,
                                          C.POINTER(C.c_int)]),
+    "hp_engine_set_summary_batched": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "hp_engine_read_summary_mcse": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t,
+                                              C.POINTER(C.c_int)]),
     "hp_engine_pt_form": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "hp_kernel_class_name": (C.c_char_p, [C.c_int]),
     "hp_sample_S": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -307,12 +307,15 @@ struct hp_engine {
     long long launches = 0;
     // posterior moments (hp_engine_set_summary): own allocations, made when first asked for, so that an engine without the
     // summary pays nothing for it.  Accumulators [C][ld] with ld = T * n (T * m) rounded up to even (k_moments' pairs).
+    // Batch means (batch > 0, hp_engine_set_summary_batched): snap (complex) and M2_bm (real) in the same layout, allocated
+    // the first time batch means are asked for.
     struct Summary {
-        int what = 0, burn_in = 0, thin = 1;
+        int what = 0, burn_in = 0, thin = 1, batch = 0;
         long long seen = 0;   // iterations computed since the summary was (re)started
         int count = 0;        // iterations accumulated
         long long ld_cr = 0, ld_fg = 0;
         double *cr_mean = nullptr, *cr_m2 = nullptr, *fg_mean = nullptr, *fg_m2 = nullptr;
+        double *cr_snap = nullptr, *cr_m2bm = nullptr, *fg_snap = nullptr, *fg_m2bm = nullptr;
     } sum;
     // profiling
     std::vector<cudaEvent_t> ev;
@@ -434,7 +437,8 @@ int hp_engine_destroy(hp_engine* e) {
     if (e->st) cudaStreamSynchronize(e->st);
     for (auto& x : e->ev) cudaEventDestroy(x);
     arena_release(e->arena, e->arena_bytes, e->cfg.device);
-    for (double* p : {e->sum.cr_mean, e->sum.cr_m2, e->sum.fg_mean, e->sum.fg_m2}) if (p) cudaFree(p);
+    for (double* p : {e->sum.cr_mean, e->sum.cr_m2, e->sum.fg_mean, e->sum.fg_m2, e->sum.cr_snap, e->sum.cr_m2bm, e->sum.fg_snap,
+                      e->sum.fg_m2bm}) if (p) cudaFree(p);
     if (e->copy_st) cudaStreamDestroy(e->copy_st);
     for (auto x : e->sub_st) cudaStreamDestroy(x);
     if (e->fork_ev) cudaEventDestroy(e->fork_ev);
@@ -1295,20 +1299,30 @@ int hp_engine_gcr(hp_engine* e) {
 
 // Whether the next computed iteration is accumulated into the posterior moments: after hp_engine_set_summary the first
 // burn_in iterations are skipped, then every thin-th one is taken.  Decided on the host once per iteration, for all
-// sub-batches alike.  Returns 1 / (accumulated iterations including this one), or 0 when it is not accumulated.
-static double summary_step(hp_engine* e) {
+// sub-batches alike, and so is whether it closes a batch of the batch means (the count reaches j * batch).
+struct SumStep {
+    double invk = 0.0;   // 1 / (accumulated iterations including this one); 0: not accumulated
+    double jj1 = -1.0;   // j (j - 1) when the iteration closes batch j; < 0: it closes none
+};
+static SumStep summary_step(hp_engine* e) {
     auto& s = e->sum;
-    if (!s.what) return 0.0;
+    SumStep r;
+    if (!s.what) return r;
     const long long k = s.seen++ - s.burn_in;
-    if (k < 0 || k % s.thin != 0) return 0.0;
-    return 1.0 / (double)(++s.count);
+    if (k < 0 || k % s.thin != 0) return r;
+    r.invk = 1.0 / (double)(++s.count);
+    if (s.batch > 0 && s.count % s.batch == 0) {
+        const double j = (double)(s.count / s.batch);
+        r.jj1 = j * (j - 1.0);
+    }
+    return r;
 }
 
 // one Gibbs iteration of all chains (gibbs_step_fgmodes, pspec.py:377-490), enqueued on e->st
 // one Gibbs iteration (gibbs_step_fgmodes, pspec.py:377-490) of the chains of one sub-batch
-// sum_invk > 0: accumulate the iteration into the posterior moments, sum_invk = 1 / (accumulated iterations including it)
+// sum.invk > 0: accumulate the iteration into the posterior moments (SumStep)
 static void enqueue_iteration_sub(hp_engine* e, const Sub& sb, int it, uint32_t iter, uint32_t draw_iter, bool general,
-                                  double sum_invk) {
+                                  const SumStep& sum) {
     const size_t n = e->n, m = e->m, T = e->T, Tp = e->Tp, I = e->cfg.max_iters, Np = e->Np;
     const bool philox = e->cfg.rng_mode == HP_RNG_PHILOX;
     Basis& b = general ? e->b0 : e->bF;
@@ -1322,22 +1336,27 @@ static void enqueue_iteration_sub(hp_engine* e, const Sub& sb, int it, uint32_t 
     o.chisq = e->chisq_out ? e->chisq_out + slot * Cn * T * n : nullptr; o.chisq_bs = (long long)(T * n);
     enqueue_gcr(e, b, o, sb, draw_iter);
 
-    if (sum_invk > 0.0) {
+    if (sum.invk > 0.0) {
         // signal_cr from the slot the iteration wrote; fg_amps straight from the solution X (rows t < T, columns n .. n + m),
         // where HP_BUF_LAST_FG reads it too, so that it needs no HP_KEEP_FG
         const auto& s = e->sum;
         hp::MomentsArr cr{}, fg{};
+        hp::MomentsBatch crb{}, fgb{};
         if (s.what & HP_SUMMARY_CR) {
             cr.src = o.sf + 2 * (size_t)sb.c0 * (size_t)o.sf_bs; cr.src_cs = o.sf_bs; cr.w = e->n; cr.rs = e->n;
             cr.L = (int)(T * n); cr.nsys = sb.nc; cr.ld = s.ld_cr;
             cr.mean = s.cr_mean + 2 * (size_t)sb.c0 * s.ld_cr; cr.m2 = s.cr_m2 + (size_t)sb.c0 * s.ld_cr;
+            if (s.batch > 0) { crb.snap = s.cr_snap + 2 * (size_t)sb.c0 * s.ld_cr; crb.m2 = s.cr_m2bm + (size_t)sb.c0 * s.ld_cr; }
         }
         if ((s.what & HP_SUMMARY_FG) && m > 0) {
             fg.src = OFFS(e->X, 2 * Tp * Np) + 2 * n; fg.src_cs = (long long)(Tp * Np); fg.w = e->m; fg.rs = e->Np;
             fg.L = (int)(T * m); fg.nsys = sb.nc; fg.ld = s.ld_fg;
             fg.mean = s.fg_mean + 2 * (size_t)sb.c0 * s.ld_fg; fg.m2 = s.fg_m2 + (size_t)sb.c0 * s.ld_fg;
+            if (s.batch > 0) { fgb.snap = s.fg_snap + 2 * (size_t)sb.c0 * s.ld_fg; fgb.m2 = s.fg_m2bm + (size_t)sb.c0 * s.ld_fg; }
         }
-        e->launches += hp::launch_moments(cr, fg, sum_invk, sb.st);
+        // only the iterations that close a batch run the longer k_moments_batch; the launch count is the same
+        e->launches += sum.jj1 >= 0.0 ? hp::launch_moments_batch(cr, fg, crb, fgb, sum.invk, sum.jj1, sb.st)
+                                      : hp::launch_moments(cr, fg, sum.invk, sb.st);
     }
 
     e->prof_begin(CLS_SAMPLE, sb.st);
@@ -1373,8 +1392,8 @@ static void enqueue_iterations(hp_engine* e, int niter, F&& after_iter) {
     for (int k = 0; k < niter; ++k) {
         const bool general = e->cfg.general_basis0 && e->iter == 0;
         const uint32_t draw_iter = (philox && !e->cfg.refresh_omega) ? 0u : e->draw_counter++;
-        const double sum_invk = summary_step(e);
-        for (auto& sb : subs) enqueue_iteration_sub(e, sb, e->out_pos, (uint32_t)e->iter, draw_iter, general, sum_invk);
+        const SumStep sum = summary_step(e);
+        for (auto& sb : subs) enqueue_iteration_sub(e, sb, e->out_pos, (uint32_t)e->iter, draw_iter, general, sum);
         e->iter++;
         e->out_pos++;
         if (after_iter(k)) { join_subs(e, subs); after_iter(-1 - k); if (k + 1 < niter) fork_subs(e, subs); }
@@ -1435,11 +1454,11 @@ int hp_engine_run_to_host(hp_engine* e, int niter, const hp_host_sink* sink) {
         const size_t slot = it % R;
         const bool general = e->cfg.general_basis0 && e->iter == 0;
         const uint32_t draw_iter = (philox && !e->cfg.refresh_omega) ? 0u : e->draw_counter++;
-        const double sum_invk = summary_step(e);
+        const SumStep sum = summary_step(e);
         for (size_t i = 0; i < nsub; ++i) {
             // the slot was last used by iteration it - R: wait for its copies unless they completed in an earlier call
             if (big && it >= R + (size_t)first) cudaStreamWaitEvent(subs[i].st, e->copy_done[slot], 0);
-            enqueue_iteration_sub(e, subs[i], (int)it, (uint32_t)e->iter, draw_iter, general, sum_invk);
+            enqueue_iteration_sub(e, subs[i], (int)it, (uint32_t)e->iter, draw_iter, general, sum);
             if (big) cudaEventRecord(e->it_done[slot * nsub + i], subs[i].st);
         }
         e->iter++;
@@ -1607,9 +1626,14 @@ int hp_engine_read(hp_engine* e, int c, int buffer, int iter0, int niter, void* 
 }
 
 int hp_engine_set_summary(hp_engine* e, int what, int burn_in, int thin) {
+    return hp_engine_set_summary_batched(e, what, burn_in, thin, 0);
+}
+
+int hp_engine_set_summary_batched(hp_engine* e, int what, int burn_in, int thin, int batch) {
     if (!e) return fail(HP_ERR_ARG, "null engine");
     if (what < 0 || (what & ~(HP_SUMMARY_CR | HP_SUMMARY_FG))) return fail(HP_ERR_ARG, "hp_engine_set_summary: unknown quantity");
     if (burn_in < 0 || thin < 1) return fail(HP_ERR_ARG, "hp_engine_set_summary: needs burn_in >= 0 and thin >= 1");
+    if (batch < 0) return fail(HP_ERR_ARG, "hp_engine_set_summary_batched: needs batch >= 0 (0: no batch means)");
     if (e->ahead > 0) return fail(HP_ERR_ARG, kAheadMsg);   // read-ahead iterations were computed under the old settings
     CU_TRY(cudaSetDevice(e->cfg.device));
     CU_TRY(cudaStreamSynchronize(e->st));   // no accumulation in flight
@@ -1626,6 +1650,14 @@ int hp_engine_set_summary(hp_engine* e, int what, int burn_in, int thin) {
         CU_TRY(dalloc(&s.fg_mean, 2 * C * s.ld_fg)); CU_TRY(dalloc(&s.fg_m2, C * s.ld_fg));
         grown = true;
     }
+    if (batch > 0 && (what & HP_SUMMARY_CR) && !s.cr_snap) {
+        CU_TRY(dalloc(&s.cr_snap, 2 * C * s.ld_cr)); CU_TRY(dalloc(&s.cr_m2bm, C * s.ld_cr));
+        grown = true;
+    }
+    if (batch > 0 && (what & HP_SUMMARY_FG) && !s.fg_snap && e->m > 0) {
+        CU_TRY(dalloc(&s.fg_snap, 2 * C * s.ld_fg)); CU_TRY(dalloc(&s.fg_m2bm, C * s.ld_fg));
+        grown = true;
+    }
     if (grown) CU_TRY(cudaStreamSynchronize(0));   // dalloc zeroes on the legacy stream, which the engine's streams do not wait for
     if (s.cr_mean) {
         CU_TRY(cudaMemsetAsync(s.cr_mean, 0, 2 * C * s.ld_cr * sizeof(double), e->st));
@@ -1635,16 +1667,32 @@ int hp_engine_set_summary(hp_engine* e, int what, int burn_in, int thin) {
         CU_TRY(cudaMemsetAsync(s.fg_mean, 0, 2 * C * s.ld_fg * sizeof(double), e->st));
         CU_TRY(cudaMemsetAsync(s.fg_m2, 0, C * s.ld_fg * sizeof(double), e->st));
     }
-    s.what = what; s.burn_in = burn_in; s.thin = thin; s.seen = 0; s.count = 0;
+    if (s.cr_snap) {
+        CU_TRY(cudaMemsetAsync(s.cr_snap, 0, 2 * C * s.ld_cr * sizeof(double), e->st));
+        CU_TRY(cudaMemsetAsync(s.cr_m2bm, 0, C * s.ld_cr * sizeof(double), e->st));
+    }
+    if (s.fg_snap) {
+        CU_TRY(cudaMemsetAsync(s.fg_snap, 0, 2 * C * s.ld_fg * sizeof(double), e->st));
+        CU_TRY(cudaMemsetAsync(s.fg_m2bm, 0, C * s.ld_fg * sizeof(double), e->st));
+    }
+    s.what = what; s.burn_in = burn_in; s.thin = thin; s.batch = batch; s.seen = 0; s.count = 0;
+    return HP_OK;
+}
+
+// the refusals shared by hp_engine_read_summary and hp_engine_read_summary_mcse (fn: the caller's name for the messages)
+static int check_summary_read(hp_engine* e, int c, int what, const char* fn) {
+    if (!e) return fail(HP_ERR_ARG, "null engine");
+    if (c < 0 || c >= e->C) return fail(HP_ERR_ARG, "chain index out of range");
+    if (what != HP_SUMMARY_CR && what != HP_SUMMARY_FG)
+        return fail(HP_ERR_ARG, std::string(fn) + ": what must be one HP_SUMMARY_* bit");
+    if (!(e->sum.what & what))
+        return fail(HP_ERR_ARG, std::string(fn) + ": this quantity is not being accumulated (hp_engine_set_summary)");
+    if (e->ahead > 0) return fail(HP_ERR_ARG, kAheadMsg);   // the moments include iterations not delivered yet
     return HP_OK;
 }
 
 int hp_engine_read_summary(hp_engine* e, int c, int what, double* mean, double* var, size_t bytes_each, int* count) {
-    if (!e) return fail(HP_ERR_ARG, "null engine");
-    if (c < 0 || c >= e->C) return fail(HP_ERR_ARG, "chain index out of range");
-    if (what != HP_SUMMARY_CR && what != HP_SUMMARY_FG) return fail(HP_ERR_ARG, "hp_engine_read_summary: what must be one HP_SUMMARY_* bit");
-    if (!(e->sum.what & what)) return fail(HP_ERR_ARG, "hp_engine_read_summary: this quantity is not being accumulated (hp_engine_set_summary)");
-    if (e->ahead > 0) return fail(HP_ERR_ARG, kAheadMsg);   // the moments include iterations not delivered yet
+    if (int rc = check_summary_read(e, c, what, "hp_engine_read_summary")) return rc;
     const auto& s = e->sum;
     const size_t L = (size_t)e->T * (what == HP_SUMMARY_CR ? e->n : e->m);
     if ((mean && bytes_each < L * 16) || (var && bytes_each < L * 8)) return fail(HP_ERR_ARG, "destination too small");
@@ -1661,6 +1709,40 @@ int hp_engine_read_summary(hp_engine* e, int c, int what, double* mean, double* 
         if (s.count == 0) { std::memset(var, 0, L * 8); return HP_OK; }
         CU_TRY(cudaMemcpy(var, dm2 + (size_t)c * ld, L * 8, cudaMemcpyDeviceToHost));
         for (size_t i = 0; i < L; ++i) var[i] /= (double)s.count;
+    }
+    return HP_OK;
+}
+
+int hp_engine_read_summary_mcse(hp_engine* e, int c, int what, double* mcse, double* ess, size_t bytes_each, int* nbatch) {
+    if (int rc = check_summary_read(e, c, what, "hp_engine_read_summary_mcse")) return rc;
+    const auto& s = e->sum;
+    if (s.batch <= 0) return fail(HP_ERR_ARG, "hp_engine_read_summary_mcse: batch means are off (hp_engine_set_summary_batched)");
+    const size_t L = (size_t)e->T * (what == HP_SUMMARY_CR ? e->n : e->m);
+    if ((mcse || ess) && bytes_each < L * 8) return fail(HP_ERR_ARG, "destination too small");
+    CU_TRY(cudaSetDevice(e->cfg.device));
+    CU_TRY(cudaStreamSynchronize(e->st));
+    const int nb = s.count / s.batch;   // complete batches; a trailing partial batch counts in k and var only
+    if (nbatch) *nbatch = nb;
+    if (L == 0 || (!mcse && !ess)) return HP_OK;
+    if (nb < 2) {
+        const double nan = std::nan("");
+        for (size_t i = 0; i < L; ++i) {
+            if (mcse) mcse[i] = nan;
+            if (ess) ess[i] = nan;
+        }
+        return HP_OK;
+    }
+    const size_t ld = what == HP_SUMMARY_CR ? s.ld_cr : s.ld_fg;
+    std::vector<double> m2(L), m2bm(L);
+    CU_TRY(cudaMemcpy(m2.data(), (what == HP_SUMMARY_CR ? s.cr_m2 : s.fg_m2) + (size_t)c * ld, L * 8, cudaMemcpyDeviceToHost));
+    CU_TRY(cudaMemcpy(m2bm.data(), (what == HP_SUMMARY_CR ? s.cr_m2bm : s.fg_m2bm) + (size_t)c * ld, L * 8,
+                      cudaMemcpyDeviceToHost));
+    // s2_bm = M2_bm / (nb - 1);  mcse^2 = b s2_bm / k;  ess = var / mcse^2 with var = M2 / k as hp_engine_read_summary
+    const double k = (double)s.count, b = (double)s.batch;
+    for (size_t i = 0; i < L; ++i) {
+        const double mcse2 = b * (m2bm[i] / (double)(nb - 1)) / k;
+        if (mcse) mcse[i] = std::sqrt(mcse2);
+        if (ess) ess[i] = (m2[i] / k) / mcse2;
     }
     return HP_OK;
 }

@@ -283,5 +283,13 @@ struct MomentsArr {
 };
 // one launch for both arrays (returns the number of launches, 0 or 1); invk = 1 / (accumulated iterations including this one)
 int launch_moments(const MomentsArr& cr, const MomentsArr& fg, double invk, cudaStream_t st);
+// k_moments_batch: the same update, then the close of batch j of the batch means.  snap[c * ld + i] (complex) is the mean at
+// the previous batch boundary, m2[c * ld + i] (real) the batch means' sum of squared deviations; same layout as MomentsArr.
+struct MomentsBatch {
+    double* snap; double* m2;
+};
+// jj1 = j (j - 1); launches as launch_moments (0 or 1)
+int launch_moments_batch(const MomentsArr& cr, const MomentsArr& fg, const MomentsBatch& crb, const MomentsBatch& fgb,
+                         double invk, double jj1, cudaStream_t st);
 
 }  // namespace hp

@@ -269,6 +269,7 @@ class GibbsEngine:
         self.general_basis0 = bool(general_basis0)
         self.time_flags = bool(time_flags)
         self.summary_what = ()
+        self.summary_batch = 0
 
     def close(self):
         if self._h is not None:
@@ -450,9 +451,11 @@ class GibbsEngine:
     # -- posterior summary (hp_engine_set_summary)
     _SUMMARY = {"cr": (_lib.HP_SUMMARY_CR, "signal_cr"), "fg": (_lib.HP_SUMMARY_FG, "fg_amps")}
 
-    def set_summary(self, what=("cr", "fg"), burn_in=0, thin=1):
+    def set_summary(self, what=("cr", "fg"), burn_in=0, thin=1, batch=0):
         """(Re)start the on-device posterior moments of ``signal_cr`` ("cr") and / or ``fg_amps`` ("fg"): of the iterations
-        computed from now on the first ``burn_in`` are skipped, then every ``thin``-th is accumulated.  ``what=()`` stops."""
+        computed from now on the first ``burn_in`` are skipped, then every ``thin``-th is accumulated.  ``what=()`` stops.
+        ``batch > 0`` also keeps batch means over ``batch`` accumulated samples, for the Monte-Carlo standard error and
+        effective sample size of each mean (:meth:`summary`)."""
         what = tuple(what)
         bad = [w for w in what if w not in self._SUMMARY]
         if bad:
@@ -460,17 +463,23 @@ class GibbsEngine:
         mask = 0
         for w in what:
             mask |= self._SUMMARY[w][0]
-        _lib.check(_lib.lib().hp_engine_set_summary(self._h, mask, int(burn_in), int(thin)))
+        _lib.check(_lib.lib().hp_engine_set_summary_batched(self._h, mask, int(burn_in), int(thin), int(batch)))
         self.summary_what = what
+        self.summary_batch = int(batch)
 
     def summary(self, chain):
         """``{"count", "signal_cr_mean", "signal_cr_var", "fg_amps_mean", "fg_amps_var"}`` of one chain, with only the
         quantities being accumulated: means (Ntimes, Nfreqs | Nmodes) complex128, variances E|x - mean|^2 (ddof = 0, as
-        ``numpy.var`` of the complex samples), count = accumulated iterations."""
+        ``numpy.var`` of the complex samples), count = accumulated iterations.
+
+        With batch means on (``set_summary(batch=b)``) the dict also has ``"<name>_mcse"`` and ``"<name>_ess"`` (float64,
+        same shape), ``"batch"`` and ``"nbatch"``: with k = count, nb = k // b complete batches of means Ybar_j and their
+        mean Ybar, ``s2_bm = sum_j |Ybar_j - Ybar|^2 / (nb - 1)``, ``mcse = sqrt(b s2_bm / k)`` (the standard error of the
+        mean) and ``ess = var / mcse**2``; NaN while nb < 2."""
         if not self.summary_what:
             raise ValueError("summary: no posterior summary is being accumulated (set_summary)")
         out = {}
-        count = _lib.C.c_int(0)
+        count, nbatch = _lib.C.c_int(0), _lib.C.c_int(0)
         for w in self.summary_what:
             bit, name = self._SUMMARY[w]
             width = self.nfreqs if w == "cr" else self.nmodes
@@ -479,7 +488,15 @@ class GibbsEngine:
             _lib.check(_lib.lib().hp_engine_read_summary(self._h, int(chain), bit, _lib.ptr(mean), _lib.ptr(var), mean.nbytes,
                                                          _lib.C.byref(count)))
             out[f"{name}_mean"], out[f"{name}_var"] = mean, var
+            if self.summary_batch > 0:
+                mcse = np.empty((self.ntimes, width), dtype=np.float64)
+                ess = np.empty((self.ntimes, width), dtype=np.float64)
+                _lib.check(_lib.lib().hp_engine_read_summary_mcse(self._h, int(chain), bit, _lib.ptr(mcse), _lib.ptr(ess),
+                                                                  mcse.nbytes, _lib.C.byref(nbatch)))
+                out[f"{name}_mcse"], out[f"{name}_ess"] = mcse, ess
         out["count"] = int(count.value)
+        if self.summary_batch > 0:
+            out["batch"], out["nbatch"] = self.summary_batch, int(nbatch.value)
         return out
 
 
@@ -490,9 +507,11 @@ _RING_ITERS = 3
 _STAGING_BYTES = int(float(os.environ.get("HP_STAGING_GB", "2")) * 2 ** 30)   # page-locked staging area
 
 
-def _device_bytes_per_chain(ntimes, nfreqs, nmodes, Niter, rng, big_per_iter, general, dense, per_time, summary):
+def _device_bytes_per_chain(ntimes, nfreqs, nmodes, Niter, rng, big_per_iter, general, dense, per_time, summary,
+                            batch=False):
     """Estimated device memory of one chain of an engine (how many chains share an engine in gibbs_sample_batch).
-    ``big_per_iter``: host bytes of one chain's kept outputs per iteration (``_big_bytes_per_iter`` / nchains)."""
+    ``big_per_iter``: host bytes of one chain's kept outputs per iteration (``_big_bytes_per_iter`` / nchains).
+    ``summary`` / ``batch``: the posterior moments / their batch means are accumulated."""
     Np = 32 * ((nfreqs + nmodes + 31) // 32)
     Tp = 16 * ((ntimes + 15) // 16)
     per_chain = 16 * Tp * Np * (4 if rng == "numpy" else 3) + 16 * Tp * nfreqs * 3 + 16 * nfreqs * Np * (2 if general else 1) \
@@ -505,20 +524,25 @@ def _device_bytes_per_chain(ntimes, nfreqs, nmodes, Niter, rng, big_per_iter, ge
         per_chain = per_chain * Tx // Tp + 16 * Tx * (1 + nmodes) * Np + 8 * Tx * nfreqs + 16 * nfreqs * nfreqs + 132 * ntimes
     if summary:
         per_chain += 24 * ntimes * (nfreqs + nmodes)   # posterior moments: complex mean + real M2 per element
+    if batch:
+        per_chain += 24 * ntimes * (nfreqs + nmodes)   # batch means: complex snapshot + real M2_bm per element
     return per_chain
 
 
 def _check_summary(summary):
     """Validate the ``summary=`` argument of the sampling functions: None, or a dict with the optional keys ``burn_in``
-    (integer >= 0, default 0) and ``thin`` (integer >= 1, default 1).  Returns None or ``{"burn_in", "thin"}``."""
+    (integer >= 0, default 0), ``thin`` (integer >= 1, default 1) and ``batch`` (integer >= 0, batch means over that many
+    accumulated samples, 0: off).  Returns None or ``{"burn_in", "thin"}``, plus ``"batch"`` when it was given."""
     if summary is None:
         return None
     if not isinstance(summary, dict):
-        raise TypeError("summary must be None or a dict(burn_in=..., thin=...)")
-    unknown = set(summary) - {"burn_in", "thin"}
+        raise TypeError("summary must be None or a dict(burn_in=..., thin=..., batch=...)")
+    unknown = set(summary) - {"burn_in", "thin", "batch"}
     if unknown:
-        raise ValueError(f"summary: unknown keys {sorted(unknown)} (expected burn_in, thin)")
+        raise ValueError(f"summary: unknown keys {sorted(unknown)} (expected burn_in, thin, batch)")
     out = {"burn_in": summary.get("burn_in", 0), "thin": summary.get("thin", 1)}
+    if "batch" in summary:
+        out["batch"] = summary["batch"]
     for k, v in out.items():
         if isinstance(v, bool) or not isinstance(v, (int, np.integer)):
             raise TypeError(f"summary: {k} must be an integer")
@@ -527,6 +551,8 @@ def _check_summary(summary):
         raise ValueError("summary: burn_in must be >= 0")
     if out["thin"] < 1:
         raise ValueError("summary: thin must be >= 1")
+    if out.get("batch", 0) < 0:
+        raise ValueError("summary: batch must be >= 0")
     return out
 
 
@@ -756,6 +782,7 @@ def gibbs_sample_with_fg(vis, flags, S_initial, fgmodes, Ninv, ps_prior, Niter=1
     ``summary=dict(burn_in=..., thin=...)``: the posterior moments of signal_cr and fg_amps are accumulated on the device
     (:meth:`GibbsEngine.set_summary`) and returned as an 8th element, the dict of :meth:`GibbsEngine.summary`; with
     ``out_dir`` they are also written (``utils.write_summary_files``) at every ``write_Niter`` boundary and at the end.
+    ``summary=dict(..., batch=b)`` adds the batch-means Monte-Carlo standard error and effective sample size of each mean.
     """
     t_start = time.perf_counter()
     summary = _check_summary(summary)
@@ -851,6 +878,7 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
     and each tuple gains an 8th element, the dict of :meth:`GibbsEngine.summary`.  Baselines with an ``out_dir`` also get
     them written (``utils.write_summary_files``) at every ``write_Niter`` boundary and at the end.  With ``keep=()`` only
     signal_ps / ln_post leave the device per iteration, and no ``out_dir`` is needed however long the chain.
+    ``summary=dict(..., batch=b)`` adds the batch-means Monte-Carlo standard error and effective sample size of each mean.
     """
     summary = _check_summary(summary)
     if not baselines:
@@ -933,7 +961,7 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
     # ---- how many chains share an engine: all of them unless the device arena would not fit (then groups run one after
     # the other; the Philox chain ids keep the samples independent of the grouping)
     per_chain = _device_bytes_per_chain(ntimes, nfreqs, nmodes, Niter, rng, per_iter // nb, general, dense, per_time,
-                                        summary is not None)
+                                        summary is not None, batch=summary is not None and summary.get("batch", 0) > 0)
     dev_budget = float(os.environ.get("HP_DEVICE_BUDGET_GB", "150")) * 2 ** 30
     group = max(1, min(nb, int(dev_budget // per_chain)))
     write_times = [0.0] * nb

@@ -31,17 +31,25 @@ def write_numpy_files(fp, signal_cr, signal_S, signal_ps, fg_amps, chisq, ln_pos
     np.save(fp / "ln-post.npy", ln_post)
 
 
-def write_summary_files(fp, moments, burn_in, thin):
+def write_summary_files(fp, moments, burn_in, thin, batch=0):
     """Posterior moments of a chain (``GibbsEngine.summary``): ``gcr-eor-mean.npy`` / ``gcr-eor-var.npy`` (signal_cr),
-    ``fg-amps-mean.npy`` / ``fg-amps-var.npy`` (fg_amps) and ``summary.json`` (count, burn_in, thin)."""
+    ``fg-amps-mean.npy`` / ``fg-amps-var.npy`` (fg_amps) and ``summary.json`` (count, burn_in, thin).  With ``batch > 0``
+    also the batch-means standard errors and effective sample sizes, ``gcr-eor-mcse.npy`` / ``gcr-eor-ess.npy`` /
+    ``fg-amps-mcse.npy`` / ``fg-amps-ess.npy``, and ``batch`` / ``nbatch`` in ``summary.json``."""
     import json
     fp = Path(fp)
     for key, stem in (("signal_cr", "gcr-eor"), ("fg_amps", "fg-amps")):
         if f"{key}_mean" in moments:
             np.save(fp / f"{stem}-mean.npy", moments[f"{key}_mean"])
             np.save(fp / f"{stem}-var.npy", moments[f"{key}_var"])
+            if batch > 0:
+                np.save(fp / f"{stem}-mcse.npy", moments[f"{key}_mcse"])
+                np.save(fp / f"{stem}-ess.npy", moments[f"{key}_ess"])
+    meta = {"count": int(moments["count"]), "burn_in": int(burn_in), "thin": int(thin)}
+    if batch > 0:
+        meta.update(batch=int(batch), nbatch=int(moments["nbatch"]))
     with open(fp / "summary.json", "w") as f:
-        json.dump({"count": int(moments["count"]), "burn_in": int(burn_in), "thin": int(thin)}, f, indent=2)
+        json.dump(meta, f, indent=2)
 
 
 def filter_freqs(freq_str, freqs_in):

@@ -167,7 +167,8 @@ int hp_engine_read(hp_engine* e, int chain, int buffer, int iter0, int niter, vo
  * (24 bytes per complex element and chain) are allocated when first asked for, outside the creation-time arena.  Enabling
  * the summary changes no draw and no output of the chain; it needs no HP_KEEP_* bit.  hp_engine_gcr does not accumulate;
  * hp_engine_rewind keeps the accumulators.  Replaces the host-side reduction of the reference's sample arrays
- * (pspec.py:590-596). */
+ * (pspec.py:590-596).  Optional batch means add the Monte-Carlo standard error and effective sample size of each mean
+ * (hp_engine_set_summary_batched, hp_engine_read_summary_mcse). */
 enum hp_summary_what { HP_SUMMARY_CR = 1, HP_SUMMARY_FG = 2 };
 /* (Re)start on-device posterior moments: accumulators zeroed; of the iterations computed from now on the first
  * burn_in are skipped, then every thin-th is accumulated (burn_in >= 0, thin >= 1).  what = 0 stops accumulating.
@@ -178,6 +179,16 @@ int hp_engine_set_summary(hp_engine* e, int what, int burn_in, int thin);
  * bytes_each: capacity of each destination (mean needs 16 T n|m bytes, var 8 T n|m).  With count = 0 both read as zeros.
  * Refused (HP_ERR_ARG) for a quantity that is not being accumulated and while read-ahead iterations are pending. */
 int hp_engine_read_summary(hp_engine* e, int chain, int what, double* mean, double* var, size_t bytes_each, int* count);
+/* hp_engine_set_summary with batch means: batch > 0 also keeps, per element, the spread of the means of consecutive
+ * batches of `batch` accumulated (thinned) samples, for the Monte-Carlo standard error of the posterior mean
+ * (hp_engine_read_summary_mcse); 24 more bytes per complex element and chain, allocated when first asked for.  batch = 0:
+ * no batch means (hp_engine_set_summary); batch < 0 is refused.  Changes neither mean nor var. */
+int hp_engine_set_summary_batched(hp_engine* e, int what, int burn_in, int thin, int batch);
+/* Batch-means Monte-Carlo standard error of the mean and effective sample size, [T][n|m] doubles each (either may be NULL;
+ * bytes_each: capacity of each, 8 T n|m bytes).  With k accumulated samples, b = batch, nb = floor(k / b) complete batches
+ * (*nbatch) of means Ybar_j and their mean Ybar: s2_bm = sum_j |Ybar_j - Ybar|^2 / (nb - 1), mcse = sqrt(b s2_bm / k),
+ * ess = var / mcse^2.  NaN while nb < 2.  Refused as hp_engine_read_summary, and when batch means are off. */
+int hp_engine_read_summary_mcse(hp_engine* e, int chain, int what, double* mcse, double* ess, size_t bytes_each, int* nbatch);
 
 /* signal_S of the reference's return value: F^H diag(ps / Nfreqs^2) F for the current spectrum
  * (covariance_from_pspec, pspec.py:313-322).  dst [Nfreqs][Nfreqs] complex128. */

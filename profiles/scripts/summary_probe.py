@@ -12,8 +12,15 @@ Prints one JSON line with
      arrays (the bench's e2e call) against keep=() + summary through the engine, and through gibbs_sample_batch.
 The card's name and power limit are read with nvidia-smi in the same run.
 
-    python profiles/scripts/summary_probe.py [OUT_DIR]      (default: a new temporary directory)
+With --batch B (batch means, k_moments_batch) the JSON line also has
+  4. the step time with batch means over B accumulated samples, alternated with the two settings of 1 (thin = 1, so one
+     iteration in B closes a batch and runs k_moments_batch instead of k_moments);
+  5. k_moments_batch's time per launch from a profiler run of its own (batch = 1: every launch closes a batch), against
+     its 112 B / complex element model (the 64 B above, 32 B snapshot read + write, 16 B M2_bm read + write).
+
+    python profiles/scripts/summary_probe.py [--batch B] [OUT_DIR]      (default: a new temporary directory)
 """
+import argparse
 import json
 import subprocess
 import sys
@@ -30,6 +37,7 @@ B, NT, NF, NM = 128, 1024, 384, 32
 SUBSTREAMS = 4
 HBM_BYTES_PER_S = 7.7e12
 BYTES_PER_ELEMENT = 64
+BYTES_PER_ELEMENT_BATCH = 112
 
 
 def card():
@@ -44,9 +52,15 @@ def main():
     import bench
     from hydra_pspec_b200 import _lib, pspec
 
+    ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
+    ap.add_argument("out_dir", nargs="?", default=None)
+    ap.add_argument("--batch", type=int, default=0, help="also measure batch means over BATCH accumulated samples")
+    opts = ap.parse_args()
+    if opts.batch < 0:
+        ap.error("--batch must be >= 0")
     if not torch.cuda.is_available():
         raise SystemExit("summary_probe.py: no CUDA device")
-    out_dir = Path(sys.argv[1] if len(sys.argv) > 1 else tempfile.mkdtemp(prefix="summary_probe_"))
+    out_dir = Path(opts.out_dir if opts.out_dir is not None else tempfile.mkdtemp(prefix="summary_probe_"))
     out_dir.mkdir(parents=True, exist_ok=True)
     name, plim = card()
     torch.cuda.set_device(0)
@@ -62,9 +76,9 @@ def main():
     for ch, (v, fl, F, nd, l0) in enumerate(inputs):
         eng.load_chain(ch, v, fl, F, nd, l0)
 
-    def steps(on, k):
+    def steps(on, k, batch=0):
         eng.rewind()
-        eng.set_summary(("cr", "fg") if on else (), burn_in=0, thin=1)
+        eng.set_summary(("cr", "fg") if on else (), burn_in=0, thin=1, batch=batch)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         eng.run(k)
@@ -74,10 +88,14 @@ def main():
 
     steps(False, W)
     steps(True, W)
-    off_ms, on_ms = [], []
+    if opts.batch:
+        steps(True, W, batch=1)   # every iteration launches k_moments_batch (first-launch module load)
+    off_ms, on_ms, batch_ms = [], [], []
     for _ in range(3):
         off_ms.append(steps(False, K))
         on_ms.append(steps(True, K))
+        if opts.batch:
+            batch_ms.append(steps(True, K, batch=opts.batch))
     assert eng.summary(0)["count"] == K
 
     # ---- 2. k_moments per launch (profiler run of its own; sub-batches off so that kernels do not overlap)
@@ -89,12 +107,27 @@ def main():
         steps(True, KP)
     durs = [ev.time_range.elapsed_us() for ev in prof.events() if "k_moments" in ev.name and str(ev.device_type).endswith("CUDA")]
     (out_dir / "summary_probe_profile.txt").write_text(prof.key_averages().table(sort_by="cuda_time_total", row_limit=30))
+    if opts.batch:
+        # ---- 5. k_moments_batch per launch: batch = 1, so that every accumulated iteration closes a batch
+        steps(True, 2, batch=1)
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            steps(True, KP, batch=1)
+        bdurs = [ev.time_range.elapsed_us() for ev in prof.events()
+                 if "k_moments_batch" in ev.name and str(ev.device_type).endswith("CUDA")]
+        (out_dir / "summary_probe_batch_profile.txt").write_text(
+            prof.key_averages().table(sort_by="cuda_time_total", row_limit=30))
     eng.close()
     kmom_ms = float(np.mean(durs)) / 1e3 if durs else None
     bytes_per_launch = BYTES_PER_ELEMENT * B * NT * (NF + NM)   # one launch covers the whole batch here
     kmom = {"launches": len(durs), "ms_per_launch": kmom_ms, "bytes_per_launch": bytes_per_launch,
             "bytes_per_s": bytes_per_launch / (kmom_ms * 1e-3) if kmom_ms else None}
     kmom["fraction_of_7.7TBps"] = kmom["bytes_per_s"] / HBM_BYTES_PER_S if kmom_ms else None
+    if opts.batch:
+        kb_ms = float(np.mean(bdurs)) / 1e3 if bdurs else None
+        kb_bytes = BYTES_PER_ELEMENT_BATCH * B * NT * (NF + NM)
+        kbatch = {"launches": len(bdurs), "ms_per_launch": kb_ms, "bytes_per_launch": kb_bytes,
+                  "bytes_per_s": kb_bytes / (kb_ms * 1e-3) if kb_ms else None}
+        kbatch["fraction_of_7.7TBps"] = kbatch["bytes_per_s"] / HBM_BYTES_PER_S if kb_ms else None
 
     # ---- 3. end to end, 64 iterations from pinned inputs
     Ke, chunk = 64, 2
@@ -154,6 +187,11 @@ def main():
            "step_overhead_ms": float(np.median(on_ms) - np.median(off_ms)),
            "step_overhead_fraction": float(np.median(on_ms) / np.median(off_ms) - 1.0),
            "k_moments": kmom, "e2e": e2e}
+    if opts.batch:
+        res.update({"batch": opts.batch, "step_ms_batch": batch_ms, "step_ms_batch_median": float(np.median(batch_ms)),
+                    "batch_overhead_ms": float(np.median(batch_ms) - np.median(on_ms)),
+                    "batch_overhead_fraction": float(np.median(batch_ms) / np.median(on_ms) - 1.0),
+                    "k_moments_batch": kbatch})
     print(json.dumps(res))
 
 

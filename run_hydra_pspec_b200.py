@@ -21,7 +21,8 @@ Same command line, config file keys, input files and output files as the referen
 * ``--samples summary`` (or ``both``) writes the posterior mean and variance of the in-painted signal and of the foreground
   amplitudes after ``--burn_in`` iterations, thinned by ``--thin``, accumulated on the GPU: ``gcr-eor-mean.npy``,
   ``gcr-eor-var.npy``, ``fg-amps-mean.npy``, ``fg-amps-var.npy`` and ``summary.json``.  With ``summary`` the per-sample files
-  ``gcr-eor.npy`` / ``fg-amps.npy`` / ``chisq.npy`` are not written, and those samples never leave the GPU.
+  ``gcr-eor.npy`` / ``fg-amps.npy`` / ``chisq.npy`` are not written, and those samples never leave the GPU.  ``--batch B`` adds
+  the batch-means Monte-Carlo standard error and effective sample size of each mean (``*-mcse.npy``, ``*-ess.npy``).
 """
 import argparse
 import json
@@ -83,6 +84,11 @@ def build_parser():
                         "fg-amps-mean.npy, fg-amps-var.npy, summary.json); both: the two")
     p.add_argument("--burn_in", type=int, default=0, help="--samples summary / both: iterations skipped before accumulating")
     p.add_argument("--thin", type=int, default=1, help="--samples summary / both: accumulate every thin-th iteration")
+    p.add_argument("--batch", type=int, default=argparse.SUPPRESS,
+                   help="--samples summary / both: also write the batch-means Monte-Carlo standard error and effective "
+                        "sample size of each mean (gcr-eor-mcse.npy, gcr-eor-ess.npy, fg-amps-mcse.npy, fg-amps-ess.npy), "
+                        "from batches of BATCH accumulated (i.e. thinned) samples.  Choose BATCH well above the "
+                        "autocorrelation time, about sqrt of the accumulated samples; fewer than 2 complete batches give NaN")
     return p
 
 
@@ -242,7 +248,15 @@ def main(argv=None):
     parser, args = parse_args(argv)
     if args.burn_in < 0 or args.thin < 1:
         parser.error("--burn_in must be >= 0 and --thin >= 1")
+    batch = getattr(args, "batch", 0)   # absent from the namespace unless given
+    if hasattr(args, "batch"):
+        if args.samples == "all":
+            parser.error("--batch needs --samples summary or both")
+        if batch < 1:
+            parser.error("--batch must be >= 1")
     summary = None if args.samples == "all" else dict(burn_in=args.burn_in, thin=args.thin)
+    if batch:
+        summary["batch"] = batch
     rank = int(os.environ.get("RANK", "0"))
     size = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
