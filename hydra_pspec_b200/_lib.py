@@ -75,8 +75,8 @@ _SIGNATURES = {
                                 C.c_int, C.c_void_p, C.c_void_p]),
     "hp_test_chol_solve": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "hp_test_solve2": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                 C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "hp_test_solve3": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                 C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "hp_test_solve3_schedule": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "hp_fp64_peak_tflops": (C.c_double, [C.c_int, C.c_double]),
     "hp_release_cached_memory": (None, []),

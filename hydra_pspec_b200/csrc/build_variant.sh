@@ -7,7 +7,7 @@ tag=$1; shift
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 FLAGS="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC $*"
 mkdir -p build_$tag
-for f in hp_kernels hp_zgemm hp_solve hp_solve2 hp_solve3 hp_fft hp_fft2 hp_pertime hp_ptlow hp_eigh hp_engine hp_testhooks; do
+for f in hp_kernels hp_zgemm hp_solve hp_solve3 hp_fft hp_fft2 hp_pertime hp_ptlow hp_eigh hp_engine hp_testhooks; do
   $NVCC $FLAGS -c $f.cu -o build_$tag/$f.o &
 done
 wait

@@ -228,7 +228,7 @@ struct Basis {
     double* Gp = nullptr;    // [C][tri][2048]
     double* Rfix = nullptr;  // [C][Tp][Np]
     double* wa = nullptr;    // [C][Tp][Np]   injected mode: Q^H omega_a
-    double* Rt = nullptr;    // [C][ntiles][nblk][2][32][16]  right-hand sides in k_solve2's tile layout (k_rhs_tile)
+    double* Rt = nullptr;    // [C][ntiles][nblk][2][32][16]  right-hand sides in k_solve3's tile layout (k_rhs_tile)
 };
 
 enum { CLS_CHOL = 0, CLS_SOLVE = 1, CLS_TRANSFORM = 2, CLS_POST = 3, CLS_SAMPLE = 4, CLS_LOWRANK = 5 };
@@ -267,12 +267,9 @@ struct hp_engine {
     int gd_slots = 1;
     std::vector<uint8_t> pending;         // chains whose G / Rfix products are still to be built (flush_pending)
     bool big_solve = false;               // N too large for k_solve's resident tile: dense k_zgemm2 products with W
-    bool solve2 = false;                  // k_solve2 (persistent, register-blocked, shared W ring) takes the solve
     bool solve3 = false;                  // k_solve3 (independent warps, W fragments streamed into registers) takes the solve
     double *Wf1 = nullptr, *Wf2 = nullptr;   // fragment-major W for k_solve3 (k_chol_w writes them)
     hp::Solve3Sched sched3{};
-    int pp_tiles = 0;                     // partial |ytilde|^2 sums per chain in Ppart: ntiles (k_solve), 2 ntiles (k_solve2)
-    double* Wp1 = nullptr;                // W diag(lam): pass-1 operand of k_solve2 when Rt holds the unscaled Rfix (Philox mode)
     double *Wd = nullptr, *Yb = nullptr;
     double *NiL = nullptr;   // dense noise: lower half of the Hermitian part of NiD (ln_post term as a triangular product)
     double *NiD = nullptr, *NihD = nullptr, *Td = nullptr, *Rm = nullptr, *Yd = nullptr;  // dense (non-diagonal) noise
@@ -403,7 +400,7 @@ void want_basis(hp_engine* e, ArenaPlan& ap, Basis& b) {
     ap.want(&b.Gp, C * hp::tri_blocks(e->nblk) * hp::kBlkDoubles);
     ap.want(&b.Rfix, 2 * C * e->Tp * e->Np);
     if (e->cfg.rng_mode == HP_RNG_INJECTED) ap.want(&b.wa, 2 * C * e->Tp * e->Np);
-    if (e->solve2 || e->solve3) ap.want(&b.Rt, 2 * C * e->Tp * e->Np);
+    if (e->solve3) ap.want(&b.Rt, 2 * C * e->Tp * e->Np);
 }
 }  // namespace
 
@@ -472,11 +469,8 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device);
     e->big_solve = cfg->force_dense_solve || !hp::solve_resident_ok(e->nblk, (size_t)max_smem);
     {
-        // HP_SOLVE_KERNEL = 1 | 2 | 3 (experiments): round-1 k_solve, k_solve2, k_solve3; default: the newest that fits
-        const char* kv = getenv("HP_SOLVE_KERNEL");
-        const int want = kv ? atoi(kv) : 3;
-        const bool resident = !e->big_solve && !cfg->time_flags;
-        e->solve3 = resident && want >= 3 && hp::solve3_ok(e->nblk, (size_t)max_smem);
+        // k_solve3 where it fits (Np <= 448), else round-1 k_solve while W stays resident (Np <= 576), else the dense products
+        e->solve3 = !e->big_solve && !cfg->time_flags && hp::solve3_ok(e->nblk, (size_t)max_smem);
         // per-time flags: low-rank form on top of k_solve3 unless HP_PT_DIRECT=1 (A/B runs, tests of k_pt_cholsolve)
         const char* pd = getenv("HP_PT_DIRECT");
         if (cfg->time_flags && !(pd && pd[0] == '1') && !cfg->force_dense_solve && hp::solve3_ok(e->nblk, (size_t)max_smem) &&
@@ -487,7 +481,6 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
             e->Tp += hp::kTT * ((e->n + hp::kTT - 1) / hp::kTT);
             e->ntiles = e->Tp / hp::kTT;
         }
-        e->solve2 = resident && !e->solve3 && want >= 2 && hp::solve2_stages(e->nblk, (size_t)max_smem) >= 2;
         if (e->solve3) hp::solve3_make_schedule(e->nblk, &e->sched3, (e->N + 15) / 16);
     }
     // a general (non-delay-diagonal) S_initial is possible in the low-rank form only: k_pt_cholsolve relies on the circulant
@@ -510,12 +503,9 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     e->ktp = hp::postfft_ktp(e->n, e->m, (size_t)max_smem);
     e->fft_ok = hp::make_fft_plan(e->n, &e->plan) && e->ktp > 0 &&
                 !cfg->force_dense_transforms;
-    {
-        const char* v1 = getenv("HP_POST_FFT_V1");   // experiments: keep the round-1 kernel
-        e->fft2_ok = e->fft_ok && !(v1 && v1[0] == '1') && hp::make_fft2_plan(e->n, &e->plan2f, &e->plan2r) &&
-                     hp::postfft2_smem_bytes(e->n, e->m) <= (size_t)max_smem / (e->n >= 512 ? 1 : 2);   // one CTA per SM from 512 channels on
-        if (e->fft2_ok) e->ktp = 8;   // k_post_fft2 handles eight times per CTA
-    }
+    e->fft2_ok = e->fft_ok && hp::make_fft2_plan(e->n, &e->plan2f, &e->plan2r) &&
+                 hp::postfft2_smem_bytes(e->n, e->m) <= (size_t)max_smem / (e->n >= 512 ? 1 : 2);   // one CTA per SM from 512 channels on
+    if (e->fft2_ok) e->ktp = 8;   // k_post_fft2 handles eight times per CTA
     e->ntilesE = hp::postfft_tiles(e->T, e->ktp > 0 ? e->ktp : 8);
     const bool dense = !e->fft_ok;                       // dense-transform scratch
     const bool need_ssc = dense || cfg->general_basis0;  // lam * ytilde as input of the dense back-transform
@@ -530,14 +520,12 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     ap.want(&e->Lp, C * hp::tri_blocks(e->nblk) * hp::kLBlkDoubles);
     ap.want(&e->Linvp, C * e->nblk * hp::kLBlkDoubles);
     ap.want(&e->Wp, C * hp::tri_blocks(e->nblk) * hp::kLBlkDoubles);
-    if (e->solve2 && cfg->rng_mode == HP_RNG_PHILOX) ap.want(&e->Wp1, C * hp::tri_blocks(e->nblk) * hp::kLBlkDoubles);
     if (e->solve3) { ap.want(&e->Wf1, C * hp::solve3_frag_doubles(e->nblk)); ap.want(&e->Wf2, C * hp::solve3_frag_doubles(e->nblk)); }
     ap.want(&e->info, C);
     ap.want(&e->chain_ids, C);
     ap.want(&e->X, 2 * C * Tp * Np);
     if (need_ssc) ap.want(&e->Ssc, 2 * C * Tp * n);   // (dense transforms / general first basis)
-    e->pp_tiles = (e->solve2 ? 2 : 1) * e->ntiles;
-    ap.want(&e->Ppart, C * e->pp_tiles * n); ap.want(&e->Sf, 2 * C * Tp * n);
+    ap.want(&e->Ppart, C * e->ntiles * n); ap.want(&e->Sf, 2 * C * Tp * n);
     if (dense) { ap.want(&e->Wm, 2 * C * Tp * n); ap.want(&e->Tmp, 2 * C * Tp * n); ap.want(&e->Em, C * n); ap.want(&e->Eu, C * n); }
     ap.want(&e->lnp1, C * Tp);
     if (e->big_solve && !cfg->time_flags) { ap.want(&e->Wd, 2 * C * Np * Np); ap.want(&e->Yb, 2 * C * Tp * Np); }
@@ -1012,7 +1000,7 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
         pa.chain_ids = OFFS(e->chain_ids, 1); pa.chain0 = sb.c0;
         hp::launch_pt_cholsolve(pa, grid, sb.st);
         // beta partial sums: Ppart[sys][0][k] = sum_t |ytilde_k|^2
-        hp::launch_colsumsq(OFFS(e->X, 2 * Tp * Np), OFFS(e->Ppart, (size_t)e->pp_tiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
+        hp::launch_colsumsq(OFFS(e->X, 2 * Tp * Np), OFFS(e->Ppart, (size_t)e->ntiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
         e->prof_end(CLS_SOLVE, 2, sb.st);
     } else {
     e->prof_begin(CLS_CHOL, sb.st);
@@ -1021,8 +1009,8 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
     ca.Linvp = OFFS(e->Linvp, (size_t)e->nblk * hp::kLBlkDoubles); ca.info = e->info + sb.c0;
     ca.nblk = e->nblk; ca.n = e->n; ca.N = e->N; ca.nsys = sb.nc;
     // Philox mode: the stored right-hand-side tiles are the unscaled Rfix, so pass 1 multiplies by W diag(lam)
-    const hp::TrinvExtra ex{OFFS(e->Wp1, tri * hp::kLBlkDoubles), OFFS(e->Wf1, hp::solve3_frag_doubles(e->nblk)),
-                            OFFS(e->Wf2, hp::solve3_frag_doubles(e->nblk)), philox ? OFFS(e->lam, Np) : nullptr};
+    const hp::TrinvExtra ex{OFFS(e->Wf1, hp::solve3_frag_doubles(e->nblk)), OFFS(e->Wf2, hp::solve3_frag_doubles(e->nblk)),
+                            philox ? OFFS(e->lam, Np) : nullptr};
     const int nchol = hp::launch_chol_trinv(ca, OFFS(e->Wp, tri * hp::kLBlkDoubles), ex, sb.st);
     e->prof_end(CLS_CHOL, nchol, sb.st);
 
@@ -1064,7 +1052,7 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
                                 e->n, e->N, e->Np, e->T, e->Tp, sb.nc, sb.st);
             ++nl;
         }
-        hp::launch_colsumsq(X, OFFS(e->Ppart, (size_t)e->pp_tiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
+        hp::launch_colsumsq(X, OFFS(e->Ppart, (size_t)e->ntiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
         ++nl;
         if (!fused_inverse) {
             k_make_ssc<<<dim3(nblocks((long long)e->T * e->n), sb.nc), 256, 0, sb.st>>>(OFFS(e->Ssc, 2 * Tp * n), X, OFFS(e->lam, Np),
@@ -1087,7 +1075,7 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
         sa.Wf1 = OFFS(e->Wf1, hp::solve3_frag_doubles(e->nblk)); sa.Wf2 = OFFS(e->Wf2, hp::solve3_frag_doubles(e->nblk));
         sa.Rt = OFFS(b.Rt, 2 * Tp * Np);
         sa.X = OFFS(e->X, 2 * Tp * Np);
-        sa.Ppart = OFFS(e->Ppart, (size_t)e->pp_tiles * n);
+        sa.Ppart = OFFS(e->Ppart, (size_t)e->ntiles * n);
         sa.nblk = e->nblk; sa.n = e->n; sa.N = e->N; sa.Tp = e->Tp; sa.ntiles = e->ntiles; sa.nsys = sb.nc; sa.T = e->T;
         sa.philox = philox ? 1 : 0;
         sa.key0 = (uint32_t)e->cfg.seed; sa.key1 = (uint32_t)(e->cfg.seed >> 32); sa.iter = draw_iter;
@@ -1116,46 +1104,13 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
             la.key0 = (uint32_t)e->cfg.seed; la.key1 = (uint32_t)(e->cfg.seed >> 32); la.iter = draw_iter;
             la.chain_ids = OFFS(e->chain_ids, 1); la.chain0 = sb.c0;
             hp::launch_pt_lowrank(la, sb.st);
-            hp::launch_colsumsq(sa.X, OFFS(e->Ppart, (size_t)e->pp_tiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
+            hp::launch_colsumsq(sa.X, OFFS(e->Ppart, (size_t)e->ntiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
             e->prof_end(CLS_LOWRANK, 3, sb.st);
             e->prof_begin(CLS_SOLVE, sb.st);   // (empty for per-time flags: no reference-CG mode, fused inverse transform)
         }
         if (e->cfg.cg_compat) {
             hp::launch_cg_scale(sa.X, OFFS(b.Rfix, 2 * Tp * Np), wa_sb, OFFS(e->lam, Np), e->n, e->N, e->Np, e->T, e->Tp, sb.nc, sb.st);
-            hp::launch_colsumsq(sa.X, OFFS(e->Ppart, (size_t)e->pp_tiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
-            nl += 2;
-        }
-        if (!fused_inverse) {
-            k_make_ssc<<<dim3(nblocks((long long)e->T * e->n), sb.nc), 256, 0, sb.st>>>(OFFS(e->Ssc, 2 * Tp * n), sa.X, OFFS(e->lam, Np),
-                                                                                       e->n, e->Np, e->T, e->Tp);
-            ++nl;
-        }
-        e->prof_end(CLS_SOLVE, nl, sb.st);
-    } else if (e->solve2) {
-        // k_solve2: right-hand sides in tile layout.  Philox mode: the unscaled Rfix tiles built at load time and
-        // W1 = W diag(lam) from k_chol_w; injected draws: r = lam * Rfix + wa rebuilt per solve, W1 = W.
-        e->prof_begin(CLS_SOLVE, sb.st);
-        int nl = 1;
-        const double* wa_sb = (!philox && any_omega) ? OFFS(b.wa, 2 * Tp * Np) : nullptr;
-        if (!philox) {
-            hp::launch_rhs_tile(OFFS(b.Rt, 2 * Tp * Np), OFFS(b.Rfix, 2 * Tp * Np), wa_sb, OFFS(e->lam, Np), e->nblk, e->n, e->N, e->T,
-                                e->Tp, e->ntiles, sb.nc, sb.st);
-            ++nl;
-        }
-        hp::Solve2Args sa{};
-        sa.W1 = philox ? OFFS(e->Wp1, tri * hp::kLBlkDoubles) : OFFS(e->Wp, tri * hp::kLBlkDoubles);
-        sa.W2 = OFFS(e->Wp, tri * hp::kLBlkDoubles);
-        sa.Rt = OFFS(b.Rt, 2 * Tp * Np);
-        sa.X = OFFS(e->X, 2 * Tp * Np);
-        sa.Ppart = OFFS(e->Ppart, (size_t)e->pp_tiles * n);
-        sa.nblk = e->nblk; sa.n = e->n; sa.N = e->N; sa.Tp = e->Tp; sa.ntiles = e->ntiles; sa.nsys = sb.nc; sa.T = e->T;
-        sa.philox = philox ? 1 : 0;
-        sa.key0 = (uint32_t)e->cfg.seed; sa.key1 = (uint32_t)(e->cfg.seed >> 32); sa.iter = draw_iter;
-        sa.chain_ids = OFFS(e->chain_ids, 1); sa.chain0 = sb.c0;
-        hp::launch_solve2(sa, sb.st);
-        if (e->cfg.cg_compat) {
-            hp::launch_cg_scale(sa.X, OFFS(b.Rfix, 2 * Tp * Np), wa_sb, OFFS(e->lam, Np), e->n, e->N, e->Np, e->T, e->Tp, sb.nc, sb.st);
-            hp::launch_colsumsq(sa.X, OFFS(e->Ppart, (size_t)e->pp_tiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
+            hp::launch_colsumsq(sa.X, OFFS(e->Ppart, (size_t)e->ntiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
             nl += 2;
         }
         if (!fused_inverse) {
@@ -1171,7 +1126,7 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
     sa.Rfix = OFFS(b.Rfix, 2 * Tp * Np);
     sa.wa = (!philox && any_omega) ? OFFS(b.wa, 2 * Tp * Np) : nullptr;
     sa.X = OFFS(e->X, 2 * Tp * Np); sa.Ssc = fused_inverse ? nullptr : OFFS(e->Ssc, 2 * Tp * n);
-    sa.Ppart = OFFS(e->Ppart, (size_t)e->pp_tiles * n);
+    sa.Ppart = OFFS(e->Ppart, (size_t)e->ntiles * n);
     sa.nblk = e->nblk; sa.n = e->n; sa.N = e->N; sa.Tp = e->Tp; sa.ntiles = e->ntiles; sa.nsys = sb.nc; sa.T = e->T;
     sa.philox_wa = philox ? 1 : 0;
     sa.cg_compat = e->cfg.cg_compat;
@@ -1361,7 +1316,7 @@ static void enqueue_iteration_sub(hp_engine* e, const Sub& sb, int it, uint32_t 
 
     e->prof_begin(CLS_SAMPLE, sb.st);
     hp::SampleArgs sp{};
-    sp.Ppart = OFFS(e->Ppart, (size_t)e->pp_tiles * n);
+    sp.Ppart = OFFS(e->Ppart, (size_t)e->ntiles * n);
     sp.ntilesE = e->fft_ok ? e->ntilesE : 0;
     sp.Eu = e->fft_ok ? OFFS(e->Eupart, (size_t)e->ntilesE * n) : OFFS(e->Eu, n);
     sp.Em = e->any_flagged ? (e->fft_ok ? OFFS(e->Empart, (size_t)e->ntilesE * n) : OFFS(e->Em, n)) : nullptr;
@@ -1370,9 +1325,8 @@ static void enqueue_iteration_sub(hp_engine* e, const Sub& sb, int it, uint32_t 
     sp.ps = OFFS(e->ps, n); sp.lam = OFFS(e->lam, Np);
     sp.ps_out = OFFS(e->ps_out, I * n) + (size_t)it * n; sp.ps_bs = (long long)(I * n);
     sp.lnpost_out = OFFS(e->lnpost_out, I) + it; sp.lnpost_bs = (long long)I;
-    sp.n = e->n; sp.Np = e->Np; sp.T = e->T; sp.Tp = e->Tp; sp.ntiles = e->ntiles; sp.nsys = sb.nc;
-    sp.ntiles = e->pp_tiles;
-    if (e->cfg.time_flags || e->big_solve || ((e->solve2 || e->solve3) && e->cfg.cg_compat)) sp.ntiles = 1;  // one partial sum per chain (k_colsumsq)
+    sp.n = e->n; sp.Np = e->Np; sp.T = e->T; sp.Tp = e->Tp; sp.nsys = sb.nc;
+    sp.ntiles = (e->cfg.time_flags || e->big_solve || (e->solve3 && e->cfg.cg_compat)) ? 1 : e->ntiles;  // 1: one partial sum per chain (k_colsumsq)
     sp.beta_mode = general ? 1 : 0; sp.philox = philox ? 1 : 0;
     sp.key0 = (uint32_t)e->cfg.seed; sp.key1 = (uint32_t)(e->cfg.seed >> 32); sp.iter = iter;
     sp.chain_ids = OFFS(e->chain_ids, 1); sp.chain0 = sb.c0;

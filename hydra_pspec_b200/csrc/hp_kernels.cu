@@ -129,7 +129,6 @@ __global__ void __launch_bounds__(kCT, 2) k_chol_w(CholArgs a, TrinvExtra ex, do
     double* Linvp = a.Linvp + (size_t)sys * nblk * kLBlkDoubles;
     double* Wp = Wp_all + (size_t)sys * tri_blocks(nblk) * kLBlkDoubles;
     const double* lam = a.lam + (size_t)sys * Np;
-    double* Wp1 = (ex.Wp1 && ex.lam) ? ex.Wp1 + (size_t)sys * tri_blocks(nblk) * kLBlkDoubles : nullptr;
     const size_t wf = (size_t)4 * nblk * (2 * nblk + 1) * 128;
     double* Wf1 = ex.Wf1 ? ex.Wf1 + (size_t)sys * wf : nullptr;
     double* Wf2 = ex.Wf2 ? ex.Wf2 + (size_t)sys * wf : nullptr;
@@ -183,12 +182,6 @@ __global__ void __launch_bounds__(kCT, 2) k_chol_w(CholArgs a, TrinvExtra ex, do
         const int r = 8 * ti + g, c = 8 * tj + 2 * q;
         *reinterpret_cast<double2*>(Wb + r * kLdBlk + c) = make_double2(dr[0][0][0], dr[0][0][1]);
         *reinterpret_cast<double2*>(Wb + kLPlane + r * kLdBlk + c) = make_double2(di[0][0][0], di[0][0][1]);
-        if (Wp1) {
-            double* Wb1 = Wp1 + blk_index(k, jp) * kLBlkDoubles;
-            const double l0 = lamj[c], l1 = lamj[c + 1];
-            *reinterpret_cast<double2*>(Wb1 + r * kLdBlk + c) = make_double2(l0 * dr[0][0][0], l1 * dr[0][0][1]);
-            *reinterpret_cast<double2*>(Wb1 + kLPlane + r * kLdBlk + c) = make_double2(l0 * di[0][0][0], l1 * di[0][0][1]);
-        }
         if (Wf1 || Wf2) {
 #pragma unroll
             for (int e = 0; e < 2; ++e) {
@@ -263,10 +256,6 @@ __global__ void __launch_bounds__(kCT, 2) k_chol_w(CholArgs a, TrinvExtra ex, do
                 Lb[e] = s.A[0][e];
                 Vb[e] = v;
                 Wb[e] = v;                                   // W_kk = V_kk
-                if (Wp1) {
-                    const int c = (e % kLPlane) % kLdBlk;
-                    Wp1[blk_index(kc, kc) * kLBlkDoubles + e] = c < 32 ? v * lamk[c] : 0.0;
-                }
             }
             if (Wf1 || Wf2) {
                 // diagonal block (lower triangular; the zeros above the diagonal are part of the 16-row strips' k range)

@@ -65,11 +65,9 @@ struct CholArgs {
     int nblk, n, N, nsys;
 };
 // Further copies of W = L^-1 that launch_chol_trinv writes besides Wp, each optional (null: not written):
-//   ex.Wp1: W diag(lam) in block layout, the pass-1 operand of k_solve2 when the stored right-hand sides are unscaled
-//           (written only when ex.lam is given; lam: [nsys][Np]);
 //   ex.Wf1 / ex.Wf2: fragment-major copies for k_solve3 (hp_solve3.cu: Wf1 = pass-1 operand, scaled by lam when ex.lam is
-//           given; Wf2 = W in pass-2 (transposed) fragment order), [nsys][solve3_frag_doubles]
-struct TrinvExtra { double* Wp1; double* Wf1; double* Wf2; const double* lam; };
+//           given (lam: [nsys][Np]); Wf2 = W in pass-2 (transposed) fragment order), [nsys][solve3_frag_doubles]
+struct TrinvExtra { double* Wf1; double* Wf2; const double* lam; };
 // M = L L^H and W = L^-1 (Wp: the padded block layout of L, [nsys][tri_blocks][2304]) in one sequence of block-column
 // launches of k_chol_w: the panel launch of column k also carries row k of W.  Returns the number of launches (1 for
 // nblk = 1, otherwise nblk + 1).
@@ -97,29 +95,6 @@ void launch_solve(const SolveArgs& a, cudaStream_t st);
 size_t solve_smem_bytes(int nblk);
 bool solve_resident_ok(int nblk, size_t max_smem);   // false: use the dense-product solve (N > 576)
 
-// ---- k_solve2 (hp_solve2.cu): persistent register-blocked solve, right-hand sides in tile layout -------------------
-struct Solve2Args {
-    const double* W1;      // [nsys][tri_blocks][2304] pass-1 operand: W, or W diag(lam) when Rt holds unscaled Rfix
-    const double* W2;      // [nsys][tri_blocks][2304] pass-2 operand: W (applied as W^H)
-    const double* Rt;      // [nsys][ntiles][nblk][2][32][16] right-hand sides in the tile's shared-memory layout (k_rhs_tile)
-    double* X;             // [nsys][Tp][Np] complex: solution [ytilde ; f]
-    double* Ppart;         // [nsys][2 ntiles][n]: sum over eight of the tile's times of |ytilde|^2
-    int nblk, n, N, Tp, ntiles, nsys, T;
-    int philox;            // 1: add xi ~ CN(0, I) (Philox, same counter layout as k_solve) to y = W1 r
-    uint32_t key0, key1, iter;
-    const int* chain_ids;
-    int chain0;
-    int stages;            // set by launch_solve2
-    int grid_limit;        // > 0: cap on the persistent grid (sub-batches sharing the GPU); 0 = one CTA per SM
-};
-void launch_solve2(const Solve2Args& a, cudaStream_t st);
-int solve2_stages(int nblk, size_t max_smem);   // W-ring depth that fits shared memory; 0 = k_solve2 cannot take this size
-void launch_rhs_tile(double* Rt, const double* Rfix, const double* wa, const double* lam, int nblk, int n, int N, int T, int Tp,
-                     int ntiles, int nsys, cudaStream_t st);
-// scalar model of the reference's truncated CG applied to the global solution X (every solve path)
-void launch_cg_scale(double* X, const double* Rfix, const double* wa, const double* lam, int n, int N, int Np, int T, int Tp,
-                     int nsys, cudaStream_t st);
-
 // ---- k_solve3 (hp_solve3.cu): independent warps, W fragments streamed from L2 into registers ------------------------
 constexpr int kS3Warps = 16;         // warps of a k_solve3 CTA (all of them compute): four per scheduler hide the L2 latency
 constexpr int kS3MaxStrips = 28;     // 16-row strips of the system (Np <= 448: two shared-memory tiles)
@@ -139,7 +114,7 @@ struct Solve3Args {
     uint32_t key0, key1, iter;
     const int* chain_ids;
     int chain0;
-    int grid_limit;
+    int grid_limit;        // > 0: cap on the persistent grid (sub-batches sharing the GPU); 0 = one CTA per SM
     int nstrip;            // 16-row strips holding rows of the system, ceil(N / 16) (0: all 2 nblk); must match the schedule
     Solve3Sched sched;
 };
@@ -147,6 +122,11 @@ void launch_solve3(const Solve3Args& a, cudaStream_t st);
 bool solve3_ok(int nblk, size_t max_smem);
 size_t solve3_frag_doubles(int nblk);               // doubles per system of Wf1 (and of Wf2)
 void solve3_make_schedule(int nblk, Solve3Sched* sc, int nstrip = 0);
+void launch_rhs_tile(double* Rt, const double* Rfix, const double* wa, const double* lam, int nblk, int n, int N, int T, int Tp,
+                     int ntiles, int nsys, cudaStream_t st);
+// scalar model of the reference's truncated CG applied to the global solution X (k_solve3, the dense-product solve)
+void launch_cg_scale(double* X, const double* Rfix, const double* wa, const double* lam, int n, int N, int Np, int T, int Tp,
+                     int nsys, cudaStream_t st);
 
 struct PostArgs {
     const double* Sf;      // [nsys][>=T][n] complex: signal in frequency space (rows t < T are read)

@@ -1,9 +1,10 @@
 // hp_solve3.cu -- k_solve3: the GCR solve  x = W^H (W r + xi)  with warps that never wait for each other inside a pass.
 //
 // Replaces the per-time preconditioned CG of the reference (gcr_fgmodes_1d, pspec.py:151-235).  k_solve (round 1) and
-// k_solve2 both reach ~62 % DMMA-pipe activity for the same reason (profiles/r2_solve2_v1_notes.md): all consumer warps
-// walk one shared W-block ring and meet at a partial-sum exchange after every block row, so they issue DMMAs in lockstep
-// and do their per-block / per-row housekeeping in lockstep too, with the pipe idle.  Here:
+// round 2's k_solve2 (since retired) both reached ~62 % DMMA-pipe activity for the same reason
+// (profiles/r2_solve2_v1_notes.md): all consumer warps walk one shared W-block ring and meet at a partial-sum exchange
+// after every block row, so they issue DMMAs in lockstep and do their per-block / per-row housekeeping in lockstep too,
+// with the pipe idle.  Here:
 //
 //   * one persistent CTA (16 warps) per SM walks the (baseline, 16-time tile) list;
 //   * the tile of right-hand sides r (TMA bulk copy, tile-native layout of k_rhs_tile) and the tile of y = W1 r + xi live
@@ -381,6 +382,94 @@ void launch_solve3(const Solve3Args& a_in, cudaStream_t st) {
     if (grid > total) grid = total;
     if (timers) k_solve3<true><<<grid, kS3Threads, smem, st>>>(a);
     else k_solve3<false><<<grid, kS3Threads, smem, st>>>(a);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// k_rhs_tile: right-hand sides in the shared-memory layout of k_solve3's tile,
+//     Rt[sys][tile][block row][plane][r][c ^ 4 (r & 3)] = (lam_row) Rfix[sys][16 tile + c][32 j + r] (+ wa)
+// Built once per chain load when the chain runs unscaled right-hand sides (Philox mode), per iteration otherwise.
+__global__ void __launch_bounds__(256) k_rhs_tile(double* __restrict__ Rt, const double* __restrict__ Rfix, const double* __restrict__ wa,
+                                                  const double* __restrict__ lam, int nblk, int n, int N, int T, int Tp) {
+    const int Np = nblk * 32;
+    const int tile = blockIdx.x, sys = blockIdx.y, t0 = tile * kTT;
+    const int ntiles = gridDim.x;
+    const double* R = Rfix + 2 * ((size_t)sys * Tp + t0) * Np;
+    const double* Wa = wa ? wa + 2 * ((size_t)sys * Tp + t0) * Np : nullptr;
+    const double* lm = lam ? lam + (size_t)sys * Np : nullptr;
+    double* out = Rt + ((size_t)sys * ntiles + tile) * nblk * kRowDoubles3;
+    // thread -> (column c, row): consecutive threads read consecutive rows of one time (coalesced 16-byte loads)
+    for (int e = threadIdx.x; e < Np * kTT; e += blockDim.x) {
+        const int c = e / Np, row = e - c * Np;
+        double vr = 0.0, vi = 0.0;
+        if (t0 + c < T && row < N) {
+            const double2 x = *reinterpret_cast<const double2*>(R + 2 * ((size_t)c * Np + row));
+            const double l = lm ? lm[row] : 1.0;
+            vr = l * x.x; vi = l * x.y;
+            if (Wa && row < n) { const double2 y = *reinterpret_cast<const double2*>(Wa + 2 * ((size_t)c * Np + row)); vr += y.x; vi += y.y; }
+        }
+        const int j = row >> 5, r = row & 31;
+        double* o = out + (size_t)j * kRowDoubles3 + r * kTT + (c ^ ((r & 3) << 2));
+        o[0] = vr;
+        o[32 * kTT] = vi;
+    }
+}
+void launch_rhs_tile(double* Rt, const double* Rfix, const double* wa, const double* lam, int nblk, int n, int N, int T, int Tp,
+                     int ntiles, int nsys, cudaStream_t st) {
+    k_rhs_tile<<<dim3(ntiles, nsys), 256, 0, st>>>(Rt, Rfix, wa, lam, nblk, n, N, T, Tp);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// k_cg_scale: the scalar model of the reference's truncated CG (pspec.py:228; DESIGN.md section 1, hp_math.h: cg_theta).
+// Every column of the exact solution is multiplied by theta(c, ||b||) with
+//     c = sum_k lam_k^2 conj(r_k) x_k + sum_j conj(r_j) x_j,   ||b||^2 = sum_k lam_k^2 |r_k|^2 + sum_j |r_j|^2
+// in the whitened variables (r = lam * Rfix + wa).  One CTA per (time, baseline); works on the global solution, so it
+// serves k_solve3 and the dense-product solve of large N (k_solve applies the model itself).
+__global__ void __launch_bounds__(128) k_cg_scale(double* __restrict__ X, const double* __restrict__ Rfix, const double* __restrict__ wa,
+                                                  const double* __restrict__ lam, int n, int N, int Np, int T, int Tp) {
+    const int t = blockIdx.x, sys = blockIdx.y;
+    if (t >= T) return;
+    const size_t off = 2 * ((size_t)sys * Tp + t) * Np;
+    double* x = X + off;
+    const double* R = Rfix + off;
+    const double* Wa = wa ? wa + off : nullptr;
+    const double* lm = lam + (size_t)sys * Np;
+    double sre = 0.0, sim = 0.0, sb = 0.0;
+    for (int row = threadIdx.x; row < N; row += blockDim.x) {
+        const double l = lm[row];
+        double vr = l * R[2 * row], vi = l * R[2 * row + 1];
+        if (Wa && row < n) { vr += Wa[2 * row]; vi += Wa[2 * row + 1]; }
+        const double wgt = row < n ? l * l : 1.0;
+        const double xr = x[2 * row], xim = x[2 * row + 1];
+        sre += wgt * (vr * xr + vi * xim);   // conj(r) x
+        sim += wgt * (vr * xim - vi * xr);
+        sb += wgt * (vr * vr + vi * vi);
+    }
+    __shared__ double red[3][4];
+    __shared__ double th[2];
+    for (int o = 16; o > 0; o >>= 1) {
+        sre += __shfl_down_sync(0xffffffffu, sre, o);
+        sim += __shfl_down_sync(0xffffffffu, sim, o);
+        sb += __shfl_down_sync(0xffffffffu, sb, o);
+    }
+    if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = sre; red[1][threadIdx.x >> 5] = sim; red[2][threadIdx.x >> 5] = sb; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        cplx c; c.re = red[0][0] + red[0][1] + red[0][2] + red[0][3]; c.im = red[1][0] + red[1][1] + red[1][2] + red[1][3];
+        const double b2 = red[2][0] + red[2][1] + red[2][2] + red[2][3];
+        const cplx v = cg_theta(c, sqrt(b2), 1e-8, 1e-6, 100000);
+        th[0] = v.re; th[1] = v.im;
+    }
+    __syncthreads();
+    const double tr = th[0], ti = th[1];
+    for (int row = threadIdx.x; row < Np; row += blockDim.x) {
+        const double xr = x[2 * row], xim = x[2 * row + 1];
+        x[2 * row] = tr * xr - ti * xim;
+        x[2 * row + 1] = tr * xim + ti * xr;
+    }
+}
+void launch_cg_scale(double* X, const double* Rfix, const double* wa, const double* lam, int n, int N, int Np, int T, int Tp,
+                     int nsys, cudaStream_t st) {
+    k_cg_scale<<<dim3(T, nsys), 128, 0, st>>>(X, Rfix, wa, lam, n, N, Np, T, Tp);
 }
 
 }  // namespace hp

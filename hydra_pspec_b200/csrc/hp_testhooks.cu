@@ -52,7 +52,7 @@ int hp_test_chol_solve(int n, int m, int T, const double* G, const double* lam, 
     hp::launch_pack_lower(dG, N, 0, dGp, N, nblk, 1, 0);
     hp::CholArgs ca{};
     ca.Gp = dGp; ca.lam = dlam; ca.Lp = dLp; ca.Linvp = dLinv; ca.info = dinfo; ca.nblk = nblk; ca.n = n; ca.N = N; ca.nsys = 1;
-    hp::launch_chol_trinv(ca, dWp, hp::TrinvExtra{nullptr, nullptr, nullptr, nullptr}, 0);
+    hp::launch_chol_trinv(ca, dWp, hp::TrinvExtra{nullptr, nullptr, nullptr}, 0);
     hp::SolveArgs sa{};
     sa.Wp = dWp; sa.lam = dlam; sa.Rfix = dR; sa.wa = dW; sa.X = dX; sa.Ssc = dS; sa.Ppart = dP;
     sa.nblk = nblk; sa.n = n; sa.N = N; sa.Tp = Tp; sa.ntiles = ntiles; sa.nsys = 1; sa.T = T; sa.cg_compat = cg_compat;
@@ -81,29 +81,27 @@ int hp_test_chol_solve(int n, int m, int T, const double* G, const double* lam, 
 }
 
 
-// The same factorisation followed by k_solve2 (hp_solve2.cu) for `nsys` systems that share G and lam but have their own
+// The same factorisation followed by k_solve3 (hp_solve3.cu) for `nsys` systems that share G and lam but have their own
 // right-hand sides Rfix[nsys][T][N] (and wa[nsys][T][n]).  wa == NULL: unscaled right-hand sides in tile layout and
-// W1 = W diag(lam) (the Philox-mode data flow, without the noise); wa != NULL: r = lam * Rfix + wa built by k_rhs_tile
-// and W1 = W.  grid_limit > 0 caps the persistent grid (several tiles per CTA at test sizes).
+// Wf1 = W diag(lam) (the Philox-mode data flow, without the noise); wa != NULL: r = lam * Rfix + wa built by k_rhs_tile
+// and Wf1 = W.  grid_limit > 0 caps the persistent grid (several tiles per CTA at test sizes).
 // X [nsys][T][N]; psum [nsys][n] = sum_t |x_k|^2 from the kernel's partial sums (or NULL).
-int hp_test_solve2(int n, int m, int T, int nsys, const double* G, const double* lam, const double* Rfix, const double* wa,
-                   int cg_compat, int grid_limit, int variant, double* X, double* psum) {
+int hp_test_solve3(int n, int m, int T, int nsys, const double* G, const double* lam, const double* Rfix, const double* wa,
+                   int cg_compat, int grid_limit, double* X, double* psum) {
     const int N = n + m, nblk = (N + 31) / 32, Np = nblk * 32, ntiles = (T + 15) / 16, Tp = ntiles * 16;
     int max_smem = 0, dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-    if (variant == 3 ? !hp::solve3_ok(nblk, (size_t)max_smem) : hp::solve2_stages(nblk, (size_t)max_smem) == 0) return HP_ERR_SIZE;
-    const int ppt = variant == 3 ? ntiles : 2 * ntiles;   // partial sums per system
+    if (!hp::solve3_ok(nblk, (size_t)max_smem)) return HP_ERR_SIZE;
     const size_t wf = hp::solve3_frag_doubles(nblk);
-    double *dWf1 = nullptr, *dWf2 = nullptr;
-    double *dG, *dGp, *dlam, *dLp, *dLinv, *dWp, *dWp1, *dR, *dW = nullptr, *dX, *dP, *dRt;
+    double *dG, *dGp, *dlam, *dLp, *dLinv, *dWp, *dR, *dW = nullptr, *dX, *dP, *dRt, *dWf1, *dWf2;
     int* dinfo;
     const size_t tri = hp::tri_blocks(nblk) * hp::kLBlkDoubles, trig = hp::tri_blocks(nblk) * hp::kBlkDoubles;
     const size_t rt_doubles = (size_t)nsys * ntiles * nblk * 2 * 32 * hp::kTT;
     cudaMalloc(&dG, 16ull * N * N); cudaMalloc(&dGp, 8 * trig); cudaMalloc(&dlam, 8ull * Np); cudaMalloc(&dLp, 8 * tri);
-    cudaMalloc(&dLinv, 8ull * nblk * hp::kLBlkDoubles); cudaMalloc(&dWp, 8 * tri); cudaMalloc(&dWp1, 8 * tri);
+    cudaMalloc(&dLinv, 8ull * nblk * hp::kLBlkDoubles); cudaMalloc(&dWp, 8 * tri);
     cudaMalloc(&dR, 16ull * nsys * Tp * Np); cudaMalloc(&dX, 16ull * nsys * Tp * Np);
-    cudaMalloc(&dP, 8ull * nsys * 2 * ntiles * n); cudaMalloc(&dinfo, 4); cudaMalloc(&dRt, 8 * rt_doubles);
+    cudaMalloc(&dP, 8ull * nsys * ntiles * n); cudaMalloc(&dinfo, 4); cudaMalloc(&dRt, 8 * rt_doubles);
     cudaMemset(dR, 0, 16ull * nsys * Tp * Np); cudaMemset(dlam, 0, 8ull * Np); cudaMemset(dX, 0xff, 16ull * nsys * Tp * Np);
     cudaMemcpy(dG, G, 16ull * N * N, cudaMemcpyHostToDevice);
     cudaMemcpy(dlam, lam, 8ull * N, cudaMemcpyHostToDevice);
@@ -117,44 +115,27 @@ int hp_test_solve2(int n, int m, int T, int nsys, const double* G, const double*
     hp::launch_pack_lower(dG, N, 0, dGp, N, nblk, 1, 0);
     hp::CholArgs ca{};
     ca.Gp = dGp; ca.lam = dlam; ca.Lp = dLp; ca.Linvp = dLinv; ca.info = dinfo; ca.nblk = nblk; ca.n = n; ca.N = N; ca.nsys = 1;
-    if (variant == 3) {
-        cudaMalloc(&dWf1, 8 * wf * nsys); cudaMalloc(&dWf2, 8 * wf * nsys);
-        cudaMemset(dWf1, 0xff, 8 * wf * nsys); cudaMemset(dWf2, 0xff, 8 * wf * nsys);   // NaN: every fragment must be written
-    }
+    cudaMalloc(&dWf1, 8 * wf * nsys); cudaMalloc(&dWf2, 8 * wf * nsys);
+    cudaMemset(dWf1, 0xff, 8 * wf * nsys); cudaMemset(dWf2, 0xff, 8 * wf * nsys);   // NaN: every fragment must be written
     // wa given: r = lam * Rfix + wa is built by k_rhs_tile and pass 1 uses the unscaled W
-    hp::launch_chol_trinv(ca, dWp, hp::TrinvExtra{dWp1, dWf1, dWf2, wa ? nullptr : dlam}, 0);
-    if (variant != 3 && wa) cudaMemcpy(dWp1, dWp, 8 * tri, cudaMemcpyDeviceToDevice);
+    hp::launch_chol_trinv(ca, dWp, hp::TrinvExtra{dWf1, dWf2, wa ? nullptr : dlam}, 0);
     for (int s = 0; s < nsys; ++s) {
         // lam is shared by the systems while k_rhs_tile indexes lam by system: build the tiles one system at a time
         hp::launch_rhs_tile(dRt + (size_t)s * ntiles * nblk * 2 * 32 * hp::kTT, dR + 2ull * s * Tp * Np,
                             dW ? dW + 2ull * s * Tp * Np : nullptr, wa ? dlam : nullptr, nblk, n, N, T, Tp, ntiles, 1, 0);
     }
     // one solve launch covers all systems and expects per-system W: replicate the one factor
-    double *dWall, *dW1all;
-    cudaMalloc(&dWall, 8 * tri * nsys); cudaMalloc(&dW1all, 8 * tri * nsys);
-    for (int s = 0; s < nsys; ++s) {
-        cudaMemcpy(dWall + tri * s, dWp, 8 * tri, cudaMemcpyDeviceToDevice);
-        cudaMemcpy(dW1all + tri * s, dWp1, 8 * tri, cudaMemcpyDeviceToDevice);
-        if (variant == 3 && s > 0) {
-            cudaMemcpy(dWf1 + wf * s, dWf1, 8 * wf, cudaMemcpyDeviceToDevice);
-            cudaMemcpy(dWf2 + wf * s, dWf2, 8 * wf, cudaMemcpyDeviceToDevice);
-        }
+    for (int s = 1; s < nsys; ++s) {
+        cudaMemcpy(dWf1 + wf * s, dWf1, 8 * wf, cudaMemcpyDeviceToDevice);
+        cudaMemcpy(dWf2 + wf * s, dWf2, 8 * wf, cudaMemcpyDeviceToDevice);
     }
-    if (variant == 3) {
-        hp::Solve3Args s3{};
-        s3.Wf1 = dWf1; s3.Wf2 = dWf2; s3.Rt = dRt; s3.X = dX; s3.Ppart = dP;
-        s3.nblk = nblk; s3.n = n; s3.N = N; s3.Tp = Tp; s3.ntiles = ntiles; s3.nsys = nsys; s3.T = T;
-        s3.philox = 0; s3.grid_limit = grid_limit;
-        s3.nstrip = (N + 15) / 16;
-        hp::solve3_make_schedule(nblk, &s3.sched, s3.nstrip);
-        hp::launch_solve3(s3, 0);
-    } else {
-    hp::Solve2Args sa{};
-    sa.W1 = dW1all; sa.W2 = dWall; sa.Rt = dRt; sa.X = dX; sa.Ppart = dP;
-    sa.nblk = nblk; sa.n = n; sa.N = N; sa.Tp = Tp; sa.ntiles = ntiles; sa.nsys = nsys; sa.T = T;
-    sa.philox = 0; sa.grid_limit = grid_limit;
-    hp::launch_solve2(sa, 0);
-    }
+    hp::Solve3Args s3{};
+    s3.Wf1 = dWf1; s3.Wf2 = dWf2; s3.Rt = dRt; s3.X = dX; s3.Ppart = dP;
+    s3.nblk = nblk; s3.n = n; s3.N = N; s3.Tp = Tp; s3.ntiles = ntiles; s3.nsys = nsys; s3.T = T;
+    s3.philox = 0; s3.grid_limit = grid_limit;
+    s3.nstrip = (N + 15) / 16;
+    hp::solve3_make_schedule(nblk, &s3.sched, s3.nstrip);
+    hp::launch_solve3(s3, 0);
     if (cg_compat)
         for (int s = 0; s < nsys; ++s)
             hp::launch_cg_scale(dX + 2ull * s * Tp * Np, dR + 2ull * s * Tp * Np, dW ? dW + 2ull * s * Tp * Np : nullptr, dlam, n, N,
@@ -164,18 +145,18 @@ int hp_test_solve2(int n, int m, int T, int nsys, const double* G, const double*
         for (int s = 0; s < nsys; ++s)
             cudaMemcpy2D(X + 2ull * s * T * N, 16ull * N, dX + 2ull * s * Tp * Np, 16ull * Np, 16ull * N, T, cudaMemcpyDeviceToHost);
         if (psum) {
-            std::vector<double> pp((size_t)nsys * ppt * n);
+            std::vector<double> pp((size_t)nsys * ntiles * n);
             cudaMemcpy(pp.data(), dP, 8 * pp.size(), cudaMemcpyDeviceToHost);
             for (int s = 0; s < nsys; ++s)
                 for (int k = 0; k < n; ++k) {
                     double acc = 0.0;
-                    for (int tl = 0; tl < ppt; ++tl) acc += pp[((size_t)s * ppt + tl) * n + k];
+                    for (int tl = 0; tl < ntiles; ++tl) acc += pp[((size_t)s * ntiles + tl) * n + k];
                     psum[(size_t)s * n + k] = acc;
                 }
         }
     }
-    cudaFree(dG); cudaFree(dGp); cudaFree(dlam); cudaFree(dLp); cudaFree(dLinv); cudaFree(dWp); cudaFree(dWp1); cudaFree(dR);
-    cudaFree(dW); cudaFree(dX); cudaFree(dP); cudaFree(dinfo); cudaFree(dRt); cudaFree(dWall); cudaFree(dW1all); cudaFree(dWf1); cudaFree(dWf2);
+    cudaFree(dG); cudaFree(dGp); cudaFree(dlam); cudaFree(dLp); cudaFree(dLinv); cudaFree(dWp); cudaFree(dR);
+    cudaFree(dW); cudaFree(dX); cudaFree(dP); cudaFree(dinfo); cudaFree(dRt); cudaFree(dWf1); cudaFree(dWf2);
     return e == cudaSuccess ? HP_OK : HP_ERR_CUDA;
 }
 

@@ -234,11 +234,11 @@ int hp_test_zgemm(int M, int N, int K, const double* A, int transA, int conjA, c
                   const double* dk, double* C);
 int hp_test_chol_solve(int n, int m, int T, const double* G, const double* lam, const double* Rfix, const double* wa,
                        int cg_compat, double* Ldense, double* X, int* info);
-/* chol + trinv + k_solve2 / k_solve3 (variant = 2 / 3; hp_solve2.cu, hp_solve3.cu) for nsys systems sharing G and lam:
+/* chol + trinv + k_solve3 (hp_solve3.cu) for nsys systems sharing G and lam:
  * Rfix [nsys][T][N], wa [nsys][T][n] or NULL, X [nsys][T][N], psum [nsys][n] = sum_t |x_k|^2 or NULL; grid_limit > 0 caps
  * the persistent grid */
-int hp_test_solve2(int n, int m, int T, int nsys, const double* G, const double* lam, const double* Rfix, const double* wa,
-                   int cg_compat, int grid_limit, int variant, double* X, double* psum);
+int hp_test_solve3(int n, int m, int T, int nsys, const double* G, const double* lam, const double* Rfix, const double* wa,
+                   int cg_compat, int grid_limit, double* X, double* psum);
 
 /* k_solve3's static strip schedule for a system of nblk 32-row blocks (host logic, no device needed):
  * n[2][nwarps] strips per pass and warp, strips[2][nwarps][max_per_warp] their 16-row strip indices */

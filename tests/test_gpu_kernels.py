@@ -45,7 +45,8 @@ def test_fourier_operator_matches_reference_definition():
         assert np.max(np.abs(got - want)) < 5e-13  # the reference's own argument is only good to ~n*eps
 
 
-@pytest.mark.parametrize("n,m,T", [(32, 0, 16), (20, 4, 5), (64, 8, 33), (120, 12, 24), (384, 32, 48)])
+@pytest.mark.parametrize("n,m,T", [(32, 0, 16), (20, 4, 5), (64, 8, 33), (120, 12, 24), (384, 32, 48),
+                                   (500, 44, 20)])   # Np = 544: k_solve takes the resident systems k_solve3 cannot
 def test_chol_solve(n, m, T):
     L = _lib()
     rng = np.random.default_rng(n + m + T)
@@ -144,18 +145,24 @@ def test_two_devices_in_one_process():
 @pytest.mark.parametrize("n,m,T,nsys,grid,use_wa,cg", [
     (32, 0, 16, 1, 0, False, 0),      # one block, one tile
     (20, 4, 5, 2, 1, True, 0),        # padded rows and times, two tiles on one persistent CTA
-    (64, 8, 33, 3, 2, False, 0),      # 3 block rows, 9 tiles on 2 CTAs (ring and exchange parities wrap)
+    (64, 8, 33, 3, 2, False, 0),      # 3 block rows, 9 tiles on 2 CTAs (mbarrier phases wrap)
     (120, 12, 24, 2, 1, True, 1),     # cg_compat through k_cg_scale
     (96, 8, 48, 4, 3, False, 0),      # 4 block rows, uneven tile split
-    (384, 32, 48, 2, 4, False, 0),    # the headline system: 13 block rows, 4-stage ring
+    (384, 32, 48, 2, 4, False, 0),    # the headline system: 13 block rows
     (384, 32, 40, 1, 0, True, 1),
-    (500, 44, 20, 1, 0, False, 0),    # Np = 544: the largest k_solve2 takes (2-stage ring)
+    (416, 32, 20, 1, 0, False, 0),    # Np = 448: the largest system k_solve3 takes (28 strips)
+    (416, 32, 17, 2, 3, True, 1),     # Np = 448 with wa and cg_compat; the second tile holds one time
+    (256, 16, 20, 2, 0, True, 0),     # N = 272: the trailing strip of pure padding is left out (272 rows in 288)
+    (40, 0, 64, 5, 7, False, 0),      # no foreground modes; 20 tiles on 7 CTAs
+    (200, 24, 48, 2, 5, False, 1),    # cg_compat with unscaled right-hand sides (Wf1 = W diag(lam))
+    (300, 20, 16, 3, 1, True, 0),     # N = 320, whole blocks; three tiles on one CTA
+    (64, 8, 1, 1, 0, False, 0),       # one time, 15 padded columns
+    (352, 32, 40, 2, 2, False, 0),    # 12 block rows, 6 tiles on 2 CTAs
+    (24, 8, 7, 3, 2, True, 0),        # one block, 3 partly filled tiles on 2 CTAs
+    (180, 12, 64, 1, 3, True, 0),     # N = 192, 4 tiles on 3 CTAs
 ])
-@pytest.mark.parametrize("variant", [2, 3])
-def test_solve2(n, m, T, nsys, grid, use_wa, cg, variant):
-    """k_solve2 / k_solve3 (persistent solves, hp_solve2.cu / hp_solve3.cu) against numpy: X, and the sum_t |x|^2 sums."""
-    if variant == 3 and n + m > 448:
-        pytest.skip("k_solve3 keeps two tiles in shared memory: Np <= 448")
+def test_solve3(n, m, T, nsys, grid, use_wa, cg):
+    """k_solve3 (persistent solve, hp_solve3.cu) against numpy: X, and the sum_t |x|^2 sums."""
     from oracle import hydra_oracle as ho  # checker only
     L = _lib()
     rng = np.random.default_rng(7 * n + m + T + nsys)
@@ -181,8 +188,8 @@ def test_solve2(n, m, T, nsys, grid, use_wa, cg, variant):
                 Xw[s, t] *= ho.cg_theta(c, b)
     X = np.empty((nsys, T, N), dtype=np.complex128)
     psum = np.empty((nsys, n))
-    L.check(L.lib().hp_test_solve2(n, m, T, nsys, L.ptr(G), L.ptr(lam), L.ptr(np.ascontiguousarray(Rfix)),
-                                   L.ptr(None if wa is None else np.ascontiguousarray(wa)), cg, grid, variant, L.ptr(X), L.ptr(psum)))
+    L.check(L.lib().hp_test_solve3(n, m, T, nsys, L.ptr(G), L.ptr(lam), L.ptr(np.ascontiguousarray(Rfix)),
+                                   L.ptr(None if wa is None else np.ascontiguousarray(wa)), cg, grid, L.ptr(X), L.ptr(psum)))
     assert rel(X, Xw) < 1e-11
     if not cg:  # (with cg_compat the engine recomputes the sums after the scaling)
         assert rel(psum, np.sum(np.abs(Xw[:, :, :n]) ** 2, axis=1)) < 1e-11

@@ -80,12 +80,27 @@ def test_large_n_philox_chain_and_reference_cg():
         assert rel(o, w) < 1e-9, k
 
 
-@pytest.mark.parametrize("nf,nm", [(544, 32), (560, 32)])
+@pytest.mark.parametrize("nf,nm", [(448, 32), (500, 44)])
+def test_resident_k_solve_chain_matches_oracle(nf, nm):
+    """Np = 480 and 544 (past k_solve3's range, resident k_solve): two iterations with injected draws match the oracle in
+    every output, signal_ps (the partial sums of |ytilde|^2) included, and a Philox chain runs."""
+    from hydra_pspec_b200 import pspec
+    vis, flags, S0, F, Ninv, prior = make_case(6, nf, nm, 4, nf, False)
+    want = ho.gibbs_sample_with_fg(vis, flags, S0, F, Ninv, prior, Niter=2, seed=4, solver="direct", symmetric_flags=True)
+    got = pspec.gibbs_sample_with_fg(vis, flags, S0, F, Ninv, prior, Niter=2, seed=4, verbose=False, solver="exact")
+    for o, w, k in zip(got[:6], want, KEYS):
+        assert rel(o, w) < 1e-9, k
+    out = pspec.gibbs_sample_with_fg(vis, flags, S0, F, Ninv, prior, Niter=3, seed=4, verbose=False, rng="philox")
+    assert np.all(np.isfinite(out[2])) and np.all(out[2] > 0) and np.all(np.isfinite(out[5]))
+
+
+@pytest.mark.parametrize("nf,nm", [(448, 32), (512, 32), (544, 32), (560, 32)])
 def test_resident_tile_boundary_residual(nf, nm):
-    """N = 576 is the largest system k_solve keeps resident in shared memory (Np = 576); N = 592 is the first that takes
-    the dense-product solve.  Size-independent property on both sides of the boundary: the solution satisfies the
-    reference's A x = b for every time (map_estimate: no fluctuation terms), and the two paths agree on a common
-    sub-problem through the chi^2 of the fit."""
+    """Np = 480 and 544 are past k_solve3's range (Np <= 448) and take the resident k_solve; N = 576 is the largest system
+    k_solve keeps resident in shared memory (Np = 576); N = 592 is the first that takes the dense-product solve.
+    Size-independent property on both sides of each boundary: the solution satisfies the reference's A x = b for every
+    time (map_estimate: no fluctuation terms), and the two paths agree on a common sub-problem through the chi^2 of the
+    fit."""
     from hydra_pspec_b200 import pspec
     rng = np.random.default_rng(nf)
     nt = 20

@@ -7,7 +7,7 @@ time of every chain.  Its distribution is Gaussian with
 
 (the reference's GCR, pspec.py:151-235, draws exactly this through omega_a / omega_b).  The tests pool >= 4000 draws:
 the sample covariance must equal Sigma within Monte-Carlo error -- which exercises the Philox counter layout over block
-rows / time tiles / chains of k_solve2, of the dense-product solve (k_add_noise) and of the per-time kernel -- and the
+rows / time tiles / chains of k_solve3, of the dense-product solve (k_add_noise) and of the per-time kernel -- and the
 cross-time, cross-chain and cross-draw covariances must vanish (a wrong counter mapping gives correlated xi).  GPU only.
 """
 import numpy as np
@@ -40,7 +40,7 @@ def nrm(C, Sigma):
     return np.max(np.abs(C) / np.outer(d, d))
 
 
-@pytest.mark.parametrize("variant", ["solve2", "dense_solve", "time_flags", "time_flags_direct"])
+@pytest.mark.parametrize("variant", ["solve3", "dense_solve", "time_flags", "time_flags_direct"])
 def test_philox_gcr_covariance_multiblock(variant, monkeypatch):
     from hydra_pspec_b200 import pspec
     # per-time flags: the low-rank form (k_solve3 + k_pt_lowrank with its own zeta draws; default) and one factorisation
