@@ -103,16 +103,15 @@ __global__ void k_build_rhs(double* R, const double* Rfix, const double* wa, con
     R[off] = vr; R[off + 1] = vi;
 }
 // y += xi, xi ~ CN(0, I): same Philox counter layout as k_solve
-__global__ void k_add_noise(double* Y, int N, int Np, int T, int Tp, uint32_t key0, uint32_t key1, uint32_t iter,
-                            const int* __restrict__ chain_ids) {
+__global__ void k_add_noise(double* Y, int N, int Np, int T, int Tp, hp::DrawKey dk) {
     const size_t sys = blockIdx.y;
     long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (e >= (long long)T * Np) return;
     const int t = (int)(e / Np), row = (int)(e % Np);
     if (row >= N) return;
-    hp::u32x4 ctr; ctr.x = (uint32_t)row; ctr.y = (uint32_t)t; ctr.z = iter; ctr.w = (uint32_t)chain_ids[sys];
+    hp::u32x4 ctr; ctr.x = (uint32_t)row; ctr.y = (uint32_t)t; ctr.z = dk.iter; ctr.w = (uint32_t)__ldg(dk.chain_ids + sys);
     double n0, n1;
-    hp::normal_pair_fast(hp::philox4x32_10(ctr, key0, key1 ^ 0xA5A5A5A5u), n0, n1);
+    hp::normal_pair_fast(hp::philox4x32_10(ctr, dk.key0, dk.key1 ^ 0xA5A5A5A5u), n0, n1);
     double* y = Y + 2 * (sys * (size_t)Tp * Np + (size_t)e);
     y[0] += n0 * 0.70710678118654752440; y[1] += n1 * 0.70710678118654752440;
 }
@@ -233,6 +232,10 @@ struct Basis {
 
 enum { CLS_CHOL = 0, CLS_SOLVE = 1, CLS_TRANSFORM = 2, CLS_POST = 3, CLS_SAMPLE = 4, CLS_LOWRANK = 5 };
 
+// The paths an engine takes through the solve and the post-processing, chosen once by select_paths (DESIGN.md section 3)
+enum class Solve { Solve3, Resident, Dense, PtLowRank, PtDirect };
+enum class Post { Fft2, Fft, Dense };
+
 }  // namespace
 
 struct hp_engine {
@@ -253,10 +256,14 @@ struct hp_engine {
     double *wT = nullptr, *Hpt = nullptr, *niT = nullptr, *Bsel = nullptr, *ptScratch = nullptr;  // per-time flags
     int* ptSame = nullptr;   // [C][Tp]: flags of time t equal those of t - 1
     int pt_ctas = 0;
+    Solve solve = Solve::Solve3;
+    Post post = Post::Fft2;
+    int ppart_tiles = 1;     // partial sums of beta per chain that the solve leaves in Ppart (k_sample adds them)
+    bool uses_solve3() const { return solve == Solve::Solve3 || solve == Solve::PtLowRank; }
     // per-time flags in low-rank form (hp_ptlow.cu): the shared system of the channels unflagged at any time goes through
     // chol / trinv / k_solve3 with n extra right-hand sides (rows Tp0 .. of Rfix / X), k_pt_lowrank corrects every time
-    bool pt_low = false;     // engine runs the low-rank form (cleared when a chain has a time with > kPtLowMaxRank extra flags)
-    int Tp0 = 0;             // padded number of times; Tp = Tp0 + padded Nfreqs when pt_low was possible at creation
+    int Tp0 = 0;             // padded number of times; Tp = Tp0 + padded Nfreqs when the engine was created as PtLowRank
+    bool lowrank_rows() const { return Tp != Tp0; }   // the extra right-hand sides of the low-rank form exist
     int pt_kcap = 0;         // largest number of extra flagged channels of any loaded (chain, time)
     double* Pm = nullptr;    // [C][n][n] complex
     uint16_t* ptFidx = nullptr;   // [C][T][kPtLowMaxRank]
@@ -266,8 +273,6 @@ struct hp_engine {
     std::vector<uint8_t> pt_loaded;   // per chain: loaded with per-time flags
     int gd_slots = 1;
     std::vector<uint8_t> pending;         // chains whose G / Rfix products are still to be built (flush_pending)
-    bool big_solve = false;               // N too large for k_solve's resident tile: dense k_zgemm2 products with W
-    bool solve3 = false;                  // k_solve3 (independent warps, W fragments streamed into registers) takes the solve
     double *Wf1 = nullptr, *Wf2 = nullptr;   // fragment-major W for k_solve3 (k_chol_w writes them)
     hp::Solve3Sched sched3{};
     double *Wd = nullptr, *Yb = nullptr;
@@ -283,13 +288,10 @@ struct hp_engine {
     void* arena = nullptr;   // one device allocation holds every buffer below
     size_t arena_bytes = 0;
     hp::FftPlan plan{};
-    hp::FftPlan plan2f{}, plan2r{};   // k_post_fft2: forward plan and the same radices in reverse order
-    bool fft2_ok = false;
-    bool fft_ok = false;
     int ntilesE = 0, ktp = 8;
     double *tw = nullptr, *tw2 = nullptr, *Empart = nullptr, *Eupart = nullptr;
     std::vector<uint8_t> flagged;  // per chain: any channel flagged
-    std::vector<uint8_t> have_omega;
+    bool any_omega = false;   // injected omega draws were set for some chain (hp_engine_set_draws)
     bool any_flagged = false;
     int ring = 1;     // device slots of the big per-iteration outputs (cfg.ring_iters, or max_iters)
     std::vector<cudaEvent_t> copy_done;   // run_to_host: the device-to-host copies out of ring slot s have completed
@@ -400,7 +402,52 @@ void want_basis(hp_engine* e, ArenaPlan& ap, Basis& b) {
     ap.want(&b.Gp, C * hp::tri_blocks(e->nblk) * hp::kBlkDoubles);
     ap.want(&b.Rfix, 2 * C * e->Tp * e->Np);
     if (e->cfg.rng_mode == HP_RNG_INJECTED) ap.want(&b.wa, 2 * C * e->Tp * e->Np);
-    if (e->solve3) ap.want(&b.Rt, 2 * C * e->Tp * e->Np);
+    if (e->uses_solve3()) ap.want(&b.Rt, 2 * C * e->Tp * e->Np);
+}
+
+// Chooses the engine's solve and post-processing paths from its configuration and the device's shared memory, and what
+// follows from them: the padded times of the low-rank form, k_solve3's schedule, the granularity of the beta partial sums
+// and the FFT tiling.  Refuses the per-time-flag configurations that no path takes.
+int select_paths(hp_engine* e, size_t max_smem) {
+    const hp_config& cfg = e->cfg;
+    e->ktp = hp::postfft_ktp(e->n, e->m, max_smem);
+    if (!hp::make_fft_plan(e->n, &e->plan) || e->ktp == 0 || cfg.force_dense_transforms) {
+        e->post = Post::Dense;
+    } else if (hp::postfft2_ok(e->n) &&
+               hp::postfft2_smem_bytes(e->n, e->m) <= max_smem / (e->n >= 512 ? 1 : 2)) {   // one CTA per SM from 512 channels on
+        e->post = Post::Fft2;
+        e->ktp = 8;   // k_post_fft2 handles eight times per CTA
+    } else {
+        e->post = Post::Fft;
+    }
+    e->ntilesE = hp::postfft_tiles(e->T, e->ktp > 0 ? e->ktp : 8);
+    const bool s3 = hp::solve3_ok(e->nblk, max_smem);
+    if (cfg.time_flags) {
+        // low-rank form on top of k_solve3 unless HP_PT_DIRECT=1 (A/B runs, tests of k_pt_cholsolve)
+        const char* pd = getenv("HP_PT_DIRECT");
+        const bool low = !(pd && pd[0] == '1') && !cfg.force_dense_solve && s3 && e->n < 65536;
+        e->solve = low ? Solve::PtLowRank : Solve::PtDirect;
+        // a general (non-delay-diagonal) S_initial is possible in the low-rank form only: k_pt_cholsolve relies on the
+        // circulant signal block of the delay basis
+        if (cfg.dense_noise || cfg.cg_compat || cfg.force_dense_transforms || (cfg.general_basis0 && !low))
+            return fail(HP_ERR_ARG, "per-time flags need diagonal noise, the exact solver and an FFT-able Nfreqs (and a delay-diagonal "
+                                    "S_initial unless Nfreqs + Nmodes <= 448)");
+        if (hp::pt_smem_bytes(e->nblk, e->n) > max_smem || e->post == Post::Dense)
+            return fail(HP_ERR_SIZE, "per-time flags: Nfreqs too large for the shared-memory working set, or without an FFT plan");
+    } else if (cfg.force_dense_solve || !hp::solve_resident_ok(e->nblk, max_smem)) {
+        e->solve = Solve::Dense;
+    } else {
+        e->solve = s3 ? Solve::Solve3 : Solve::Resident;
+    }
+    if (e->solve == Solve::PtLowRank) {
+        e->Tp += hp::kTT * ((e->n + hp::kTT - 1) / hp::kTT);
+        e->ntiles = e->Tp / hp::kTT;
+    }
+    if (e->uses_solve3()) hp::solve3_make_schedule(e->nblk, &e->sched3, (e->N + 15) / 16);
+    // k_solve and k_solve3 leave one partial sum per 16-time tile; the other paths, and k_solve3 followed by the reference-CG
+    // scaling, one per chain (k_colsumsq)
+    e->ppart_tiles = (e->solve == Solve::Resident || (e->solve == Solve::Solve3 && !cfg.cg_compat)) ? e->ntiles : 1;
+    return HP_OK;
 }
 }  // namespace
 
@@ -467,47 +514,16 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     e->Tp0 = e->Tp;
     int max_smem = 0;
     cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device);
-    e->big_solve = cfg->force_dense_solve || !hp::solve_resident_ok(e->nblk, (size_t)max_smem);
-    {
-        // k_solve3 where it fits (Np <= 448), else round-1 k_solve while W stays resident (Np <= 576), else the dense products
-        e->solve3 = !e->big_solve && !cfg->time_flags && hp::solve3_ok(e->nblk, (size_t)max_smem);
-        // per-time flags: low-rank form on top of k_solve3 unless HP_PT_DIRECT=1 (A/B runs, tests of k_pt_cholsolve)
-        const char* pd = getenv("HP_PT_DIRECT");
-        if (cfg->time_flags && !(pd && pd[0] == '1') && !cfg->force_dense_solve && hp::solve3_ok(e->nblk, (size_t)max_smem) &&
-            e->n < 65536) {
-            e->pt_low = true;
-            e->solve3 = true;
-            e->Tp0 = e->Tp;
-            e->Tp += hp::kTT * ((e->n + hp::kTT - 1) / hp::kTT);
-            e->ntiles = e->Tp / hp::kTT;
-        }
-        if (e->solve3) hp::solve3_make_schedule(e->nblk, &e->sched3, (e->N + 15) / 16);
-    }
-    // a general (non-delay-diagonal) S_initial is possible in the low-rank form only: k_pt_cholsolve relies on the circulant
-    // signal block of the delay basis
-    if (cfg->time_flags && (cfg->dense_noise || cfg->cg_compat || cfg->force_dense_transforms || (cfg->general_basis0 && !e->pt_low))) {
+    if (const int rc = select_paths(e, (size_t)max_smem)) {
         delete e;
-        return fail(HP_ERR_ARG, "per-time flags need diagonal noise, the exact solver and an FFT-able Nfreqs (and a delay-diagonal "
-                                "S_initial unless Nfreqs + Nmodes <= 448)");
-    }
-    if (cfg->time_flags && (hp::pt_smem_bytes(e->nblk, e->n) > (size_t)max_smem || !hp::make_fft_plan(e->n, &e->plan) ||
-                            hp::postfft_ktp(e->n, e->m, (size_t)max_smem) == 0)) {
-        delete e;
-        return fail(HP_ERR_SIZE, "per-time flags: Nfreqs too large for the shared-memory working set, or without an FFT plan");
+        return rc;
     }
     if (cfg->stream) e->st = (cudaStream_t)cfg->stream;
     else { CU_TRY(cudaStreamCreateWithFlags(&e->st, cudaStreamNonBlocking)); e->own_stream = true; }
     const size_t C = e->C, n = e->n, m = e->m, Np = e->Np, Tp = e->Tp, T = e->T, I = cfg->max_iters;
     e->ring = (cfg->ring_iters > 0 && cfg->ring_iters < cfg->max_iters) ? cfg->ring_iters : cfg->max_iters;
     const size_t R = e->ring;
-    e->ktp = hp::postfft_ktp(e->n, e->m, (size_t)max_smem);
-    e->fft_ok = hp::make_fft_plan(e->n, &e->plan) && e->ktp > 0 &&
-                !cfg->force_dense_transforms;
-    e->fft2_ok = e->fft_ok && hp::make_fft2_plan(e->n, &e->plan2f, &e->plan2r) &&
-                 hp::postfft2_smem_bytes(e->n, e->m) <= (size_t)max_smem / (e->n >= 512 ? 1 : 2);   // one CTA per SM from 512 channels on
-    if (e->fft2_ok) e->ktp = 8;   // k_post_fft2 handles eight times per CTA
-    e->ntilesE = hp::postfft_tiles(e->T, e->ktp > 0 ? e->ktp : 8);
-    const bool dense = !e->fft_ok;                       // dense-transform scratch
+    const bool dense = e->post == Post::Dense;           // dense-transform scratch
     const bool need_ssc = dense || cfg->general_basis0;  // lam * ytilde as input of the dense back-transform
     ArenaPlan ap;
     ap.want(&e->Fop, 2 * n * n); ap.want(&e->U, 2 * n * n);
@@ -520,7 +536,7 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     ap.want(&e->Lp, C * hp::tri_blocks(e->nblk) * hp::kLBlkDoubles);
     ap.want(&e->Linvp, C * e->nblk * hp::kLBlkDoubles);
     ap.want(&e->Wp, C * hp::tri_blocks(e->nblk) * hp::kLBlkDoubles);
-    if (e->solve3) { ap.want(&e->Wf1, C * hp::solve3_frag_doubles(e->nblk)); ap.want(&e->Wf2, C * hp::solve3_frag_doubles(e->nblk)); }
+    if (e->uses_solve3()) { ap.want(&e->Wf1, C * hp::solve3_frag_doubles(e->nblk)); ap.want(&e->Wf2, C * hp::solve3_frag_doubles(e->nblk)); }
     ap.want(&e->info, C);
     ap.want(&e->chain_ids, C);
     ap.want(&e->X, 2 * C * Tp * Np);
@@ -528,7 +544,7 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     ap.want(&e->Ppart, C * e->ntiles * n); ap.want(&e->Sf, 2 * C * Tp * n);
     if (dense) { ap.want(&e->Wm, 2 * C * Tp * n); ap.want(&e->Tmp, 2 * C * Tp * n); ap.want(&e->Em, C * n); ap.want(&e->Eu, C * n); }
     ap.want(&e->lnp1, C * Tp);
-    if (e->big_solve && !cfg->time_flags) { ap.want(&e->Wd, 2 * C * Np * Np); ap.want(&e->Yb, 2 * C * Tp * Np); }
+    if (e->solve == Solve::Dense) { ap.want(&e->Wd, 2 * C * Np * Np); ap.want(&e->Yb, 2 * C * Tp * Np); }
     if (cfg->time_flags) {
         e->pt_ctas = hp::pt_grid(e->C, e->T);
         ap.want(&e->wT, C * Tp * n);
@@ -537,7 +553,7 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
         ap.want(&e->niT, Tp * n);
         ap.want(&e->Bsel, 2 * n * (1 + m));
         ap.want(&e->ptScratch, (size_t)e->pt_ctas * hp::pt_scratch_doubles_per_cta(e->nblk));
-        if (e->pt_low) {
+        if (e->solve == Solve::PtLowRank) {
             ap.want(&e->Pm, 2 * C * n * n);
             ap.want(&e->ptFidx, C * T * hp::kPtLowMaxRank);
             ap.want(&e->ptFcnt, C * T);
@@ -559,7 +575,7 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     ap.want(&e->stage, 2 * (T * n > n * n ? T * n : n * n));
     ap.want(&e->vecn, 4 * n);
     ap.want(&e->tw, 2 * n);
-    if (e->fft2_ok) ap.want(&e->tw2, 4 * n);
+    if (e->post == Post::Fft2) ap.want(&e->tw2, 4 * n);
     ap.want(&e->Empart, C * e->ntilesE * n); ap.want(&e->Eupart, C * e->ntilesE * n);
     {
         cudaError_t ce = ap.commit(&e->arena, &e->arena_bytes, cfg->device, e->st);
@@ -574,7 +590,6 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     e->hpt_built.assign(C, 0);
     e->pt_loaded.assign(C, 0);
     e->pending.assign(C, 0);
-    e->have_omega.assign(C, 0);
     {
         int ns = cfg->substreams > 1 ? (cfg->substreams < (int)C ? cfg->substreams : (int)C) : 1;
         if (ns > 1) {
@@ -594,7 +609,7 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     hp::launch_fourier_operator(e->Fop, e->n, 1.0, e->st);
     hp::launch_fourier_operator(e->U, e->n, 1.0 / std::sqrt((double)e->n), e->st);
     hp::launch_twiddles(e->tw, e->n, e->st);
-    if (e->tw2 && !hp::launch_fft2_tables(e->tw2, e->tw, e->n, e->st)) e->tw2 = nullptr;
+    if (e->post == Post::Fft2) hp::launch_fft2_tables(e->tw2, e->tw, e->n, e->st);
     if (cudaStreamSynchronize(e->st) != cudaSuccess || cudaGetLastError() != cudaSuccess) {
         hp_engine_destroy(e);
         return fail(HP_ERR_CUDA, "engine initialisation kernels failed");
@@ -666,14 +681,14 @@ static int build_basis_products(hp_engine* e, Basis& b, int c) {
     }
     hp::launch_zgemm(r, e->st);
     // low-rank form of per-time flags: the columns of A = D B^H sqrt(wbar N^-1) are n more right-hand sides (rows Tp0 + x)
-    if (e->ptFidx) hp::launch_pt_arows(b.Rfix + 2 * (size_t)c * e->Tp * Np, Bm, e->ni + (size_t)c * n, n, Np, e->Tp0, e->st);
+    if (e->lowrank_rows()) hp::launch_pt_arows(b.Rfix + 2 * (size_t)c * e->Tp * Np, Bm, e->ni + (size_t)c * n, n, Np, e->Tp0, e->st);
     if (b.Rt && e->cfg.rng_mode == HP_RNG_PHILOX)
         hp::launch_rhs_tile(b.Rt + 2 * (size_t)c * e->Tp * Np, b.Rfix + 2 * (size_t)c * e->Tp * Np, nullptr, nullptr, e->nblk, e->n, e->N,
-                            e->ptFidx ? e->Tp : e->T, e->Tp, e->ntiles, 1, e->st);
+                            e->lowrank_rows() ? e->Tp : e->T, e->Tp, e->ntiles, 1, e->st);
     // the operands of k_pt_cholsolve are built only when the engine runs (or falls back to) one factorisation per time
     if (e->cfg.time_flags && &b == &e->bF) {
         e->hpt_built[c] = 0;
-        if (!e->pt_low) { const int rc = build_hpt(e, c); if (rc != HP_OK) return rc; }
+        if (e->solve == Solve::PtDirect) { const int rc = build_hpt(e, c); if (rc != HP_OK) return rc; }
     }
     CU_TRY(cudaGetLastError());
     return HP_OK;
@@ -713,7 +728,7 @@ static int build_basis_products_batch(hp_engine* e, Basis& b, int c0, int nc) {
 
 static int flush_pending(hp_engine* e) {
     const int C = e->C;
-    if (e->cfg.time_flags && !e->pt_low)   // fell back to one factorisation per time after some chains were loaded
+    if (e->solve == Solve::PtDirect)   // fell back to one factorisation per time after some chains were loaded
         for (int c = 0; c < C; ++c)
             if (e->pt_loaded[c] && !e->hpt_built[c]) { const int rc = build_hpt(e, c); if (rc != HP_OK) return rc; }
     for (int c = 0; c < C;) {
@@ -769,7 +784,7 @@ static int load_chain_impl(hp_engine* e, int c, const double* vis, const uint8_t
         std::vector<int> same(Tp, 0);
         for (int t = 1; t < T; ++t) same[t] = std::memcmp(flags + (size_t)t * n, flags + (size_t)(t - 1) * n, n) == 0 ? 1 : 0;
         CU_TRY(cudaMemcpyAsync(e->ptSame + (size_t)c * Tp, same.data(), (size_t)Tp * sizeof(int), cudaMemcpyHostToDevice, st));
-        if (e->ptFidx) {
+        if (e->lowrank_rows()) {
             // channels flagged at time t beyond the all-times mask
             std::vector<uint16_t> fidx((size_t)T * hp::kPtLowMaxRank, 0);
             std::vector<int> fcnt(T, 0);
@@ -791,8 +806,8 @@ static int load_chain_impl(hp_engine* e, int c, const double* vis, const uint8_t
             e->pt_kcap = 0;
             for (int v : e->pt_kmax) if (v > e->pt_kcap) e->pt_kcap = v;
             // a time with more extra flags than the low-rank kernel takes: the whole engine uses k_pt_cholsolve
-            e->pt_low = e->pt_kcap <= hp::kPtLowMaxRank;
-            if (!e->pt_low && e->cfg.general_basis0)
+            e->solve = e->pt_kcap <= hp::kPtLowMaxRank ? Solve::PtLowRank : Solve::PtDirect;
+            if (e->solve == Solve::PtDirect && e->cfg.general_basis0)
                 return fail(HP_ERR_SIZE, "per-time flags with a general S_initial: a time has more than 64 channels flagged beyond the "
                                          "all-times mask (only the low-rank form of the per-time solve takes a general first basis)");
         }
@@ -914,7 +929,7 @@ int hp_engine_set_draws(hp_engine* e, int c, const double* omega_a, const double
             hp::launch_zgemm(a, st);
             CU_TRY(cudaStreamSynchronize(st));
         }
-        e->have_omega[c] = 1;
+        e->any_omega = true;
     }
     CU_TRY(cudaStreamSynchronize(st));
     CU_TRY(cudaGetLastError());
@@ -965,180 +980,200 @@ static void enqueue_dense_lnp1(hp_engine* e, const Sub& sb) {
     e->prof_end(CLS_TRANSFORM, 2, sb.st);
 }
 
-// GCR step (gcr_fgmodes) and everything of gibbs_step_fgmodes up to the power-spectrum draw:
-// chol + solve + back-transform + residual statistics.  `b` is the basis in use.
-static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb, uint32_t draw_iter) {
-    const bool philox = e->cfg.rng_mode == HP_RNG_PHILOX;
-    const bool general = &b == &e->b0;
-    const size_t n = e->n, m = e->m, Np = e->Np, Tp = e->Tp;
-    const size_t tri = hp::tri_blocks(e->nblk);
-    const bool fused_inverse = e->fft_ok && !general;  // s = U^H (lam ytilde) inside k_post_fft
-    const bool pt = e->cfg.time_flags != 0;
-    bool any_omega = false;
-    for (auto h : e->have_omega) any_omega |= (h != 0);
-    const bool pt_low = pt && e->pt_low;
-    if (pt && !pt_low) {
-        // one factorisation + solve per (chain, time); sub-batches share the SMs, each gets its share of the
-        // persistent grid and of the scratch slots
-        const int nsub = e->C > 0 ? (e->C + sb.nc - 1) / sb.nc : 1;
-        int grid = e->pt_ctas / (nsub > 0 ? nsub : 1);
-        if (grid < 1) grid = 1;
-        const int slot0 = (int)(((long long)sb.c0 * e->pt_ctas) / e->C);
-        if (slot0 + grid > e->pt_ctas) grid = e->pt_ctas - slot0;
-        e->prof_begin(CLS_SOLVE, sb.st);
-        cudaMemsetAsync(e->info + sb.c0, 0, sizeof(int) * sb.nc, sb.st);
-        hp::PtArgs pa{};
-        pa.H = OFFS(e->Hpt, 2 * Tp * (1 + m) * Np); pa.lam = OFFS(e->lam, Np); pa.Rfix = OFFS(b.Rfix, 2 * Tp * Np);
-        pa.wa = (!philox && any_omega) ? OFFS(b.wa, 2 * Tp * Np) : nullptr;
-        pa.X = OFFS(e->X, 2 * Tp * Np);
-        pa.same_prev = OFFS(e->ptSame, Tp);
-        pa.scratch = e->ptScratch + (size_t)slot0 * hp::pt_scratch_doubles_per_cta(e->nblk);
-        pa.info = e->info + sb.c0;
-        pa.nblk = e->nblk; pa.n = e->n; pa.m = e->m; pa.N = e->N; pa.T = e->T; pa.Tp = e->Tp; pa.nsys = sb.nc;
-        pa.philox_wa = philox ? 1 : 0;
-        pa.key0 = (uint32_t)e->cfg.seed; pa.key1 = (uint32_t)(e->cfg.seed >> 32); pa.iter = draw_iter;
-        pa.chain_ids = OFFS(e->chain_ids, 1); pa.chain0 = sb.c0;
-        hp::launch_pt_cholsolve(pa, grid, sb.st);
-        // beta partial sums: Ppart[sys][0][k] = sum_t |ytilde_k|^2
-        hp::launch_colsumsq(OFFS(e->X, 2 * Tp * Np), OFFS(e->Ppart, (size_t)e->ntiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
-        e->prof_end(CLS_SOLVE, 2, sb.st);
-    } else {
-    e->prof_begin(CLS_CHOL, sb.st);
-    hp::CholArgs ca{};
-    ca.Gp = OFFS(b.Gp, tri * hp::kBlkDoubles); ca.lam = OFFS(e->lam, Np); ca.Lp = OFFS(e->Lp, tri * hp::kLBlkDoubles);
-    ca.Linvp = OFFS(e->Linvp, (size_t)e->nblk * hp::kLBlkDoubles); ca.info = e->info + sb.c0;
-    ca.nblk = e->nblk; ca.n = e->n; ca.N = e->N; ca.nsys = sb.nc;
-    // Philox mode: the stored right-hand-side tiles are the unscaled Rfix, so pass 1 multiplies by W diag(lam)
-    const hp::TrinvExtra ex{OFFS(e->Wf1, hp::solve3_frag_doubles(e->nblk)), OFFS(e->Wf2, hp::solve3_frag_doubles(e->nblk)),
-                            philox ? OFFS(e->lam, Np) : nullptr};
-    const int nchol = hp::launch_chol_trinv(ca, OFFS(e->Wp, tri * hp::kLBlkDoubles), ex, sb.st);
-    e->prof_end(CLS_CHOL, nchol, sb.st);
+// Whether the next computed iteration is accumulated into the posterior moments: after hp_engine_set_summary the first
+// burn_in iterations are skipped, then every thin-th one is taken.  Decided on the host once per iteration, for all
+// sub-batches alike, and so is whether it closes a batch of the batch means (the count reaches j * batch).
+struct SumStep {
+    double invk = 0.0;   // 1 / (accumulated iterations including this one); 0: not accumulated
+    double jj1 = -1.0;   // j (j - 1) when the iteration closes batch j; < 0: it closes none
+};
+static SumStep summary_step(hp_engine* e) {
+    auto& s = e->sum;
+    SumStep r;
+    if (!s.what) return r;
+    const long long k = s.seen++ - s.burn_in;
+    if (k < 0 || k % s.thin != 0) return r;
+    r.invk = 1.0 / (double)(++s.count);
+    if (s.batch > 0 && s.count % s.batch == 0) {
+        const double j = (double)(s.count / s.batch);
+        r.jj1 = j * (j - 1.0);
+    }
+    return r;
+}
 
-    if (e->big_solve) {
-        // x = W^H (W r + xi) as two dense products (W unpacked to a dense lower-triangular matrix): the path for
-        // Nfreqs + Nmodes beyond k_solve's shared-memory resident tile (BASELINE.json configs[4])
-        e->prof_begin(CLS_SOLVE, sb.st);
-        const long long NN = (long long)e->Np * e->Np, TN = (long long)e->Tp * e->Np;
-        double* Wd = OFFS(e->Wd, 2 * Np * Np);
-        double* Yb = OFFS(e->Yb, 2 * Tp * Np);
-        double* X = OFFS(e->X, 2 * Tp * Np);
-        k_unpack_lower<<<dim3(nblocks(NN), sb.nc), 256, 0, sb.st>>>(OFFS(e->Wp, tri * hp::kLBlkDoubles), Wd, e->nblk,
-                                                                   tri * hp::kLBlkDoubles);
-        k_build_rhs<<<dim3(nblocks(TN), sb.nc), 256, 0, sb.st>>>(X, OFFS(b.Rfix, 2 * Tp * Np),
-                                                                (!philox && any_omega) ? OFFS(b.wa, 2 * Tp * Np) : nullptr,
-                                                                OFFS(e->lam, Np), e->n, e->Np, e->T, e->Tp);
-        hp::ZgemmArgs y{};   // Y[t][i] = sum_j r[t][j] W[i][j]
-        y.A = X; y.sAi = e->Np; y.sAk = 1; y.bsA = TN;
-        y.B = Wd; y.sBk = 1; y.sBj = e->Np; y.bsB = NN;
-        y.C = Yb; y.sCi = e->Np; y.sCj = 1; y.bsC = TN;
-        y.M = e->T; y.N = e->Np; y.K = e->Np; y.alpha = 1.0; y.batch = sb.nc;
-        y.tri = 1;           // B[k = j][col = i] = W[i][j] = 0 for j > i
-        hp::launch_zgemm(y, sb.st);
-        int nl = 4;
-        if (philox) {
-            k_add_noise<<<dim3(nblocks((long long)e->T * e->Np), sb.nc), 256, 0, sb.st>>>(
-                Yb, e->N, e->Np, e->T, e->Tp, (uint32_t)e->cfg.seed, (uint32_t)(e->cfg.seed >> 32), draw_iter, OFFS(e->chain_ids, 1));
-            ++nl;
-        }
-        hp::ZgemmArgs x{};   // X[t][i] = sum_j y[t][j] conj(W[j][i])
-        x.A = Yb; x.sAi = e->Np; x.sAk = 1; x.bsA = TN;
-        x.B = Wd; x.sBk = e->Np; x.sBj = 1; x.bsB = NN; x.conjB = 1;
-        x.C = X; x.sCi = e->Np; x.sCj = 1; x.bsC = TN;
-        x.M = e->T; x.N = e->Np; x.K = e->Np; x.alpha = 1.0; x.batch = sb.nc;
-        x.tri = 2;           // B[k = j][col = i] = conj(W[j][i]) = 0 for j < i
-        hp::launch_zgemm(x, sb.st);
-        if (e->cfg.cg_compat) {
-            hp::launch_cg_scale(X, OFFS(b.Rfix, 2 * Tp * Np), (!philox && any_omega) ? OFFS(b.wa, 2 * Tp * Np) : nullptr, OFFS(e->lam, Np),
-                                e->n, e->N, e->Np, e->T, e->Tp, sb.nc, sb.st);
-            ++nl;
-        }
-        hp::launch_colsumsq(X, OFFS(e->Ppart, (size_t)e->ntiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
-        ++nl;
-        if (!fused_inverse) {
-            k_make_ssc<<<dim3(nblocks((long long)e->T * e->n), sb.nc), 256, 0, sb.st>>>(OFFS(e->Ssc, 2 * Tp * n), X, OFFS(e->lam, Np),
-                                                                                       e->n, e->Np, e->T, e->Tp);
-            ++nl;
-        }
-        e->prof_end(CLS_SOLVE, nl, sb.st);
-    } else if (e->solve3) {
-        // k_solve3: right-hand sides in tile layout (Philox: the unscaled tiles built at load time, Wf1 = W diag(lam);
-        // injected draws: r = lam * Rfix + wa rebuilt per solve, Wf1 = W)
-        e->prof_begin(CLS_SOLVE, sb.st);
-        int nl = 1;
-        const double* wa_sb = (!philox && any_omega) ? OFFS(b.wa, 2 * Tp * Np) : nullptr;
-        if (!philox) {
-            hp::launch_rhs_tile(OFFS(b.Rt, 2 * Tp * Np), OFFS(b.Rfix, 2 * Tp * Np), wa_sb, OFFS(e->lam, Np), e->nblk, e->n, e->N,
-                                pt_low ? e->Tp : e->T, e->Tp, e->ntiles, sb.nc, sb.st);
-            ++nl;
-        }
-        hp::Solve3Args sa{};
-        sa.Wf1 = OFFS(e->Wf1, hp::solve3_frag_doubles(e->nblk)); sa.Wf2 = OFFS(e->Wf2, hp::solve3_frag_doubles(e->nblk));
-        sa.Rt = OFFS(b.Rt, 2 * Tp * Np);
-        sa.X = OFFS(e->X, 2 * Tp * Np);
-        sa.Ppart = OFFS(e->Ppart, (size_t)e->ntiles * n);
-        sa.nblk = e->nblk; sa.n = e->n; sa.N = e->N; sa.Tp = e->Tp; sa.ntiles = e->ntiles; sa.nsys = sb.nc; sa.T = e->T;
-        sa.philox = philox ? 1 : 0;
-        sa.key0 = (uint32_t)e->cfg.seed; sa.key1 = (uint32_t)(e->cfg.seed >> 32); sa.iter = draw_iter;
-        sa.chain_ids = OFFS(e->chain_ids, 1); sa.chain0 = sb.c0;
-        sa.sched = e->sched3; sa.nstrip = (e->N + 15) / 16;
-        hp::launch_solve3(sa, sb.st);
-        if (pt_low) {
-            // per-time flags: rows Tp0 + x of X now hold R = M_0^-1 A.  P = A^H R, then the rank-k_t correction of every time
-            e->prof_end(CLS_SOLVE, nl, sb.st);
-            nl = 0;
-            e->prof_begin(CLS_LOWRANK, sb.st);
-            hp::ZgemmArgs pz{};
-            pz.A = OFFS(b.Rfix, 2 * Tp * Np) + 2 * (size_t)e->Tp0 * Np; pz.sAi = e->Np; pz.sAk = 1; pz.bsA = (long long)e->Tp * e->Np;
-            pz.conjA = 1; pz.dk = OFFS(e->lam, Np); pz.bsD = e->Np;
-            pz.B = sa.X + 2 * (size_t)e->Tp0 * Np; pz.sBk = 1; pz.sBj = e->Np; pz.bsB = (long long)e->Tp * e->Np;
-            pz.C = OFFS(e->Pm, 2 * n * n); pz.sCi = e->n; pz.sCj = 1; pz.bsC = (long long)e->n * e->n;
-            pz.M = e->n; pz.N = e->n; pz.K = e->N; pz.alpha = 1.0; pz.batch = sb.nc;
-            pz.lower_out = 1;   // k_pt_lowrank reads the lower triangle of P only
-            hp::launch_zgemm(pz, sb.st);
-            hp::PtLowArgs la{};
-            la.Rfix = OFFS(b.Rfix, 2 * Tp * Np); la.wa = wa_sb; la.lam = OFFS(e->lam, Np); la.X = sa.X; la.Pm = OFFS(e->Pm, 2 * n * n);
-            la.fidx = e->ptFidx + (size_t)sb.c0 * e->T * hp::kPtLowMaxRank; la.fcnt = e->ptFcnt + (size_t)sb.c0 * e->T;
-            la.info = e->info + sb.c0;
-            la.n = e->n; la.N = e->N; la.Np = e->Np; la.T = e->T; la.Tp = e->Tp; la.Tp0 = e->Tp0; la.nsys = sb.nc; la.nblk = e->nblk;
-            la.kcap = e->pt_kcap; la.philox = philox ? 1 : 0;
-            la.key0 = (uint32_t)e->cfg.seed; la.key1 = (uint32_t)(e->cfg.seed >> 32); la.iter = draw_iter;
-            la.chain_ids = OFFS(e->chain_ids, 1); la.chain0 = sb.c0;
-            hp::launch_pt_lowrank(la, sb.st);
-            hp::launch_colsumsq(sa.X, OFFS(e->Ppart, (size_t)e->ntiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
-            e->prof_end(CLS_LOWRANK, 3, sb.st);
-            e->prof_begin(CLS_SOLVE, sb.st);   // (empty for per-time flags: no reference-CG mode, fused inverse transform)
-        }
-        if (e->cfg.cg_compat) {
-            hp::launch_cg_scale(sa.X, OFFS(b.Rfix, 2 * Tp * Np), wa_sb, OFFS(e->lam, Np), e->n, e->N, e->Np, e->T, e->Tp, sb.nc, sb.st);
-            hp::launch_colsumsq(sa.X, OFFS(e->Ppart, (size_t)e->ntiles * n), e->T, e->Tp, e->n, sb.nc, sb.st, e->Np);
-            nl += 2;
-        }
-        if (!fused_inverse) {
-            k_make_ssc<<<dim3(nblocks((long long)e->T * e->n), sb.nc), 256, 0, sb.st>>>(OFFS(e->Ssc, 2 * Tp * n), sa.X, OFFS(e->lam, Np),
-                                                                                       e->n, e->Np, e->T, e->Tp);
-            ++nl;
-        }
-        e->prof_end(CLS_SOLVE, nl, sb.st);
-    } else {
+// What one iteration (or GCR step) uses, decided on the host once for all sub-batches: the general first basis on the
+// first iteration, the draw counter of the GCR fluctuations (fixed in Philox mode unless refresh_omega) and, with
+// `summary`, the posterior-moment step (summary_step)
+struct IterStep { bool general; uint32_t draw_iter; SumStep sum; };
+static IterStep iter_step(hp_engine* e, bool summary) {
+    IterStep r;
+    r.general = e->cfg.general_basis0 && e->iter == 0;
+    r.draw_iter = (e->cfg.rng_mode == HP_RNG_PHILOX && !e->cfg.refresh_omega) ? 0u : e->draw_counter++;
+    if (summary) r.sum = summary_step(e);
+    return r;
+}
+
+// the draw identity of sub-batch sb at draw counter `iter`
+static hp::DrawKey draw_key(const hp_engine* e, const Sub& sb, uint32_t iter) {
+    return hp::DrawKey{(uint32_t)e->cfg.seed, (uint32_t)(e->cfg.seed >> 32), iter, OFFS(e->chain_ids, 1)};
+}
+
+// Ppart[sys][0][k] = sum_t |ytilde_k|^2 from the solution X
+static void launch_beta_sums(hp_engine* e, const Sub& sb) {
+    hp::launch_colsumsq(OFFS(e->X, 2 * (size_t)e->Tp * e->Np), OFFS(e->Ppart, (size_t)e->ntiles * e->n), e->T, e->Tp, e->n, sb.nc,
+                        sb.st, e->Np);
+}
+static void launch_make_ssc(hp_engine* e, const Sub& sb) {
+    k_make_ssc<<<dim3(nblocks((long long)e->T * e->n), sb.nc), 256, 0, sb.st>>>(
+        OFFS(e->Ssc, 2 * (size_t)e->Tp * e->n), OFFS(e->X, 2 * (size_t)e->Tp * e->Np), OFFS(e->lam, (size_t)e->Np), e->n, e->Np, e->T, e->Tp);
+}
+
+// The solve paths.  Each leaves the solution [ytilde ; f] in X, e->ppart_tiles partial sums of beta = sum_t |ytilde|^2 per
+// chain in Ppart, and with `ssc` lam * ytilde in Ssc.  wa: Q^H omega_a of the injected draws, or null.
+// x = W^H (W r + xi) as two dense products (W unpacked to a dense lower-triangular matrix): the path for Nfreqs + Nmodes
+// beyond k_solve's shared-memory resident tile (BASELINE.json configs[4])
+static void solve_dense(hp_engine* e, Basis& b, const Sub& sb, const hp::DrawKey& dk, const double* wa, bool ssc) {
+    const size_t Np = e->Np, Tp = e->Tp, tri = hp::tri_blocks(e->nblk);
+    e->prof_begin(CLS_SOLVE, sb.st);
+    const long long NN = (long long)e->Np * e->Np, TN = (long long)e->Tp * e->Np;
+    double* Wd = OFFS(e->Wd, 2 * Np * Np);
+    double* Yb = OFFS(e->Yb, 2 * Tp * Np);
+    double* X = OFFS(e->X, 2 * Tp * Np);
+    k_unpack_lower<<<dim3(nblocks(NN), sb.nc), 256, 0, sb.st>>>(OFFS(e->Wp, tri * hp::kLBlkDoubles), Wd, e->nblk,
+                                                               tri * hp::kLBlkDoubles);
+    k_build_rhs<<<dim3(nblocks(TN), sb.nc), 256, 0, sb.st>>>(X, OFFS(b.Rfix, 2 * Tp * Np), wa, OFFS(e->lam, Np), e->n, e->Np, e->T,
+                                                            e->Tp);
+    hp::ZgemmArgs y{};   // Y[t][i] = sum_j r[t][j] W[i][j]
+    y.A = X; y.sAi = e->Np; y.sAk = 1; y.bsA = TN;
+    y.B = Wd; y.sBk = 1; y.sBj = e->Np; y.bsB = NN;
+    y.C = Yb; y.sCi = e->Np; y.sCj = 1; y.bsC = TN;
+    y.M = e->T; y.N = e->Np; y.K = e->Np; y.alpha = 1.0; y.batch = sb.nc;
+    y.tri = 1;           // B[k = j][col = i] = W[i][j] = 0 for j > i
+    hp::launch_zgemm(y, sb.st);
+    const bool philox = e->cfg.rng_mode == HP_RNG_PHILOX;
+    if (philox) k_add_noise<<<dim3(nblocks((long long)e->T * e->Np), sb.nc), 256, 0, sb.st>>>(Yb, e->N, e->Np, e->T, e->Tp, dk);
+    hp::ZgemmArgs x{};   // X[t][i] = sum_j y[t][j] conj(W[j][i])
+    x.A = Yb; x.sAi = e->Np; x.sAk = 1; x.bsA = TN;
+    x.B = Wd; x.sBk = e->Np; x.sBj = 1; x.bsB = NN; x.conjB = 1;
+    x.C = X; x.sCi = e->Np; x.sCj = 1; x.bsC = TN;
+    x.M = e->T; x.N = e->Np; x.K = e->Np; x.alpha = 1.0; x.batch = sb.nc;
+    x.tri = 2;           // B[k = j][col = i] = conj(W[j][i]) = 0 for j < i
+    hp::launch_zgemm(x, sb.st);
+    if (e->cfg.cg_compat) hp::launch_cg_scale(X, OFFS(b.Rfix, 2 * Tp * Np), wa, OFFS(e->lam, Np), e->n, e->N, e->Np, e->T, e->Tp, sb.nc, sb.st);
+    launch_beta_sums(e, sb);
+    if (ssc) launch_make_ssc(e, sb);
+    // unpack, right-hand sides, two products, beta sums (+ noise, CG scaling, Ssc)
+    e->prof_end(CLS_SOLVE, 5 + philox + (e->cfg.cg_compat != 0) + ssc, sb.st);
+}
+
+// k_solve3: right-hand sides in tile layout (Philox: the unscaled tiles built at load time, Wf1 = W diag(lam); injected draws:
+// r = lam * Rfix + wa rebuilt per solve, Wf1 = W)
+static void solve_solve3(hp_engine* e, Basis& b, const Sub& sb, const hp::DrawKey& dk, const double* wa, bool ssc) {
+    const size_t n = e->n, Np = e->Np, Tp = e->Tp;
+    const bool philox = e->cfg.rng_mode == HP_RNG_PHILOX;
+    e->prof_begin(CLS_SOLVE, sb.st);
+    if (!philox)
+        hp::launch_rhs_tile(OFFS(b.Rt, 2 * Tp * Np), OFFS(b.Rfix, 2 * Tp * Np), wa, OFFS(e->lam, Np), e->nblk, e->n, e->N,
+                            e->lowrank_rows() ? e->Tp : e->T, e->Tp, e->ntiles, sb.nc, sb.st);
+    hp::Solve3Args sa{};
+    sa.Wf1 = OFFS(e->Wf1, hp::solve3_frag_doubles(e->nblk)); sa.Wf2 = OFFS(e->Wf2, hp::solve3_frag_doubles(e->nblk));
+    sa.Rt = OFFS(b.Rt, 2 * Tp * Np);
+    sa.X = OFFS(e->X, 2 * Tp * Np);
+    sa.Ppart = OFFS(e->Ppart, (size_t)e->ntiles * n);
+    sa.nblk = e->nblk; sa.n = e->n; sa.N = e->N; sa.Tp = e->Tp; sa.ntiles = e->ntiles; sa.nsys = sb.nc; sa.T = e->T;
+    sa.philox = philox ? 1 : 0;
+    sa.dk = dk;
+    sa.sched = e->sched3; sa.nstrip = (e->N + 15) / 16;
+    hp::launch_solve3(sa, sb.st);
+    if (e->cfg.cg_compat) {
+        hp::launch_cg_scale(sa.X, OFFS(b.Rfix, 2 * Tp * Np), wa, OFFS(e->lam, Np), e->n, e->N, e->Np, e->T, e->Tp, sb.nc, sb.st);
+        launch_beta_sums(e, sb);
+    }
+    if (ssc) launch_make_ssc(e, sb);
+    e->prof_end(CLS_SOLVE, (philox ? 1 : 2) + 2 * (e->cfg.cg_compat != 0) + ssc, sb.st);
+}
+
+static void solve_resident(hp_engine* e, Basis& b, const Sub& sb, const hp::DrawKey& dk, const double* wa, bool ssc) {
+    const size_t n = e->n, Np = e->Np, Tp = e->Tp, tri = hp::tri_blocks(e->nblk);
     e->prof_begin(CLS_SOLVE, sb.st);
     hp::SolveArgs sa{};
     sa.Wp = OFFS(e->Wp, tri * hp::kLBlkDoubles); sa.lam = OFFS(e->lam, Np);
     sa.Rfix = OFFS(b.Rfix, 2 * Tp * Np);
-    sa.wa = (!philox && any_omega) ? OFFS(b.wa, 2 * Tp * Np) : nullptr;
-    sa.X = OFFS(e->X, 2 * Tp * Np); sa.Ssc = fused_inverse ? nullptr : OFFS(e->Ssc, 2 * Tp * n);
+    sa.wa = wa;
+    sa.X = OFFS(e->X, 2 * Tp * Np); sa.Ssc = ssc ? OFFS(e->Ssc, 2 * Tp * n) : nullptr;
     sa.Ppart = OFFS(e->Ppart, (size_t)e->ntiles * n);
     sa.nblk = e->nblk; sa.n = e->n; sa.N = e->N; sa.Tp = e->Tp; sa.ntiles = e->ntiles; sa.nsys = sb.nc; sa.T = e->T;
-    sa.philox_wa = philox ? 1 : 0;
+    sa.philox_wa = e->cfg.rng_mode == HP_RNG_PHILOX ? 1 : 0;
     sa.cg_compat = e->cfg.cg_compat;
-    sa.key0 = (uint32_t)e->cfg.seed; sa.key1 = (uint32_t)(e->cfg.seed >> 32); sa.iter = draw_iter;
-    sa.chain_ids = OFFS(e->chain_ids, 1); sa.chain0 = sb.c0;
+    sa.dk = dk;
     hp::launch_solve(sa, sb.st);
     e->prof_end(CLS_SOLVE, 1, sb.st);
-    }
-    }
+}
 
+// per-time flags, low-rank form: k_solve3 leaves R = M_0^-1 A in rows Tp0 + x of X (no reference-CG mode with per-time
+// flags).  P = A^H R, then the rank-k_t correction of every time
+static void solve_pt_lowrank(hp_engine* e, Basis& b, const Sub& sb, const hp::DrawKey& dk, const double* wa, bool ssc) {
+    const size_t n = e->n, Np = e->Np, Tp = e->Tp;
+    solve_solve3(e, b, sb, dk, wa, false);
+    e->prof_begin(CLS_LOWRANK, sb.st);
+    double* X = OFFS(e->X, 2 * Tp * Np);
+    hp::ZgemmArgs pz{};
+    pz.A = OFFS(b.Rfix, 2 * Tp * Np) + 2 * (size_t)e->Tp0 * Np; pz.sAi = e->Np; pz.sAk = 1; pz.bsA = (long long)e->Tp * e->Np;
+    pz.conjA = 1; pz.dk = OFFS(e->lam, Np); pz.bsD = e->Np;
+    pz.B = X + 2 * (size_t)e->Tp0 * Np; pz.sBk = 1; pz.sBj = e->Np; pz.bsB = (long long)e->Tp * e->Np;
+    pz.C = OFFS(e->Pm, 2 * n * n); pz.sCi = e->n; pz.sCj = 1; pz.bsC = (long long)e->n * e->n;
+    pz.M = e->n; pz.N = e->n; pz.K = e->N; pz.alpha = 1.0; pz.batch = sb.nc;
+    pz.lower_out = 1;   // k_pt_lowrank reads the lower triangle of P only
+    hp::launch_zgemm(pz, sb.st);
+    hp::PtLowArgs la{};
+    la.Rfix = OFFS(b.Rfix, 2 * Tp * Np); la.wa = wa; la.lam = OFFS(e->lam, Np); la.X = X; la.Pm = OFFS(e->Pm, 2 * n * n);
+    la.fidx = e->ptFidx + (size_t)sb.c0 * e->T * hp::kPtLowMaxRank; la.fcnt = e->ptFcnt + (size_t)sb.c0 * e->T;
+    la.info = e->info + sb.c0;
+    la.n = e->n; la.N = e->N; la.Np = e->Np; la.T = e->T; la.Tp = e->Tp; la.Tp0 = e->Tp0; la.nsys = sb.nc; la.nblk = e->nblk;
+    la.kcap = e->pt_kcap; la.philox = e->cfg.rng_mode == HP_RNG_PHILOX ? 1 : 0;
+    la.dk = dk;
+    hp::launch_pt_lowrank(la, sb.st);
+    launch_beta_sums(e, sb);
+    e->prof_end(CLS_LOWRANK, 3, sb.st);
+    e->prof_begin(CLS_SOLVE, sb.st);   // lam * ytilde for a general first basis, else empty
+    if (ssc) launch_make_ssc(e, sb);
+    e->prof_end(CLS_SOLVE, ssc ? 1 : 0, sb.st);
+}
+
+// per-time flags, one factorisation + solve per (chain, time); sub-batches share the SMs, each gets its share of the
+// persistent grid and of the scratch slots.  Never asked for Ssc: a general first basis needs the low-rank form
+// (select_paths, load_chain_impl refuse it here), and per-time flags always have an FFT plan
+static void solve_pt_direct(hp_engine* e, Basis& b, const Sub& sb, const hp::DrawKey& dk, const double* wa) {
+    const size_t m = e->m, Np = e->Np, Tp = e->Tp;
+    const int nsub = e->C > 0 ? (e->C + sb.nc - 1) / sb.nc : 1;
+    int grid = e->pt_ctas / (nsub > 0 ? nsub : 1);
+    if (grid < 1) grid = 1;
+    const int slot0 = (int)(((long long)sb.c0 * e->pt_ctas) / e->C);
+    if (slot0 + grid > e->pt_ctas) grid = e->pt_ctas - slot0;
+    e->prof_begin(CLS_SOLVE, sb.st);
+    cudaMemsetAsync(e->info + sb.c0, 0, sizeof(int) * sb.nc, sb.st);
+    hp::PtArgs pa{};
+    pa.H = OFFS(e->Hpt, 2 * Tp * (1 + m) * Np); pa.lam = OFFS(e->lam, Np); pa.Rfix = OFFS(b.Rfix, 2 * Tp * Np);
+    pa.wa = wa;
+    pa.X = OFFS(e->X, 2 * Tp * Np);
+    pa.same_prev = OFFS(e->ptSame, Tp);
+    pa.scratch = e->ptScratch + (size_t)slot0 * hp::pt_scratch_doubles_per_cta(e->nblk);
+    pa.info = e->info + sb.c0;
+    pa.nblk = e->nblk; pa.n = e->n; pa.m = e->m; pa.N = e->N; pa.T = e->T; pa.Tp = e->Tp; pa.nsys = sb.nc;
+    pa.philox_wa = e->cfg.rng_mode == HP_RNG_PHILOX ? 1 : 0;
+    pa.dk = dk;
+    hp::launch_pt_cholsolve(pa, grid, sb.st);
+    launch_beta_sums(e, sb);
+    e->prof_end(CLS_SOLVE, 2, sb.st);
+}
+
+// s = U^H (lam ytilde) (fused into k_post_fft / k_post_fft2, or with `ssc` a dense back-transform of Ssc), foreground
+// amplitudes, residual statistics and the sums of |U s|^2, |U (w s)|^2 that k_sample reads (sample_energies)
+static void enqueue_post(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb, Post post, bool ssc) {
+    const bool general = &b == &e->b0;
+    const size_t n = e->n, m = e->m, Np = e->Np, Tp = e->Tp;
     double* sf = o.sf + 2 * (size_t)sb.c0 * (size_t)o.sf_bs;
-    if (!fused_inverse) {
+    if (ssc) {
         // s = Q (lam * ytilde) as a dense product (general eigenbasis, or Nfreqs without an FFT plan)
         e->prof_begin(CLS_TRANSFORM, sb.st);
         hp::ZgemmArgs t{};
@@ -1154,37 +1189,34 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
     double* fg = o.fg ? o.fg + (size_t)sb.c0 * (size_t)o.fg_bs : nullptr;
     double* chisq = o.chisq ? o.chisq + (size_t)sb.c0 * (size_t)o.chisq_bs : nullptr;
 
-    if (e->fft_ok) {
-        e->prof_begin(CLS_POST, sb.st);
+    e->prof_begin(CLS_POST, sb.st);
+    if (post == Post::Dense) {
+        // dense fallback for Nfreqs with a large prime factor
+        hp::PostArgs pa{};
+        pa.Sf = sf; pa.sf_bs = o.sf_bs; pa.X = OFFS(e->X, 2 * Tp * Np); pa.Ft = OFFS(e->Ft, 2 * (m ? m : 1) * n);
+        pa.wd = OFFS(e->wd, 2 * Tp * n); pa.w = OFFS(e->w, n); pa.ninvd = OFFS(e->ninvd, n);
+        pa.fg_out = fg; pa.fg_bs = o.fg_bs; pa.chisq_out = chisq; pa.chisq_bs = o.chisq_bs;
+        pa.Wm = e->any_flagged ? OFFS(e->Wm, 2 * Tp * n) : nullptr; pa.Rm = e->cfg.dense_noise ? OFFS(e->Rm, 2 * Tp * n) : nullptr;
+        pa.lnp1 = OFFS(e->lnp1, Tp);
+        pa.n = e->n; pa.m = e->m; pa.Np = e->Np; pa.T = e->T; pa.Tp = e->Tp; pa.nsys = sb.nc;
+        hp::launch_post(pa, sb.st);
+    } else {
         hp::PostFftArgs pa{};
         pa.plan = e->plan; pa.tw = e->tw; pa.tw2 = e->tw2; pa.X = OFFS(e->X, 2 * Tp * Np); pa.lam = OFFS(e->lam, Np); pa.Sf = sf; pa.sf_bs = o.sf_bs;
         pa.Ft = OFFS(e->Ft, 2 * (m ? m : 1) * n); pa.wd = OFFS(e->wd, 2 * Tp * n); pa.w = OFFS(e->w, n); pa.ninvd = OFFS(e->ninvd, n);
         pa.w_bs = e->n; pa.w_ts = 0;
-        if (pt) { pa.w = OFFS(e->wT, Tp * n); pa.w_bs = (long long)e->Tp * e->n; pa.w_ts = e->n; }
+        if (e->cfg.time_flags) { pa.w = OFFS(e->wT, Tp * n); pa.w_bs = (long long)e->Tp * e->n; pa.w_ts = e->n; }
         pa.fg_out = fg; pa.fg_bs = o.fg_bs; pa.chisq_out = chisq; pa.chisq_bs = o.chisq_bs;
         pa.lnp1 = OFFS(e->lnp1, Tp); pa.Rm = e->cfg.dense_noise ? OFFS(e->Rm, 2 * Tp * n) : nullptr;
         pa.Empart = e->any_flagged ? OFFS(e->Empart, (size_t)e->ntilesE * n) : nullptr;
         pa.Eupart = general ? OFFS(e->Eupart, (size_t)e->ntilesE * n) : nullptr;
-        pa.m = e->m; pa.Np = e->Np; pa.T = e->T; pa.Tp = e->Tp; pa.nsys = sb.nc; pa.do_inverse = fused_inverse ? 1 : 0; pa.ktp = e->ktp;
-        if (!(e->fft2_ok && pa.do_inverse && !pa.Eupart && hp::launch_post_fft2(pa, e->plan2f, e->plan2r, sb.st)))
-            hp::launch_post_fft(pa, sb.st);
-        e->prof_end(CLS_POST, 1, sb.st);
-        if (e->cfg.dense_noise) enqueue_dense_lnp1(e, sb);
-        return;
+        pa.m = e->m; pa.Np = e->Np; pa.T = e->T; pa.Tp = e->Tp; pa.nsys = sb.nc; pa.do_inverse = ssc ? 0 : 1; pa.ktp = e->ktp;
+        if (post == Post::Fft2) hp::launch_post_fft2(pa, sb.st);
+        else hp::launch_post_fft(pa, sb.st);
     }
-    // dense fallback for Nfreqs with a large prime factor
-    e->prof_begin(CLS_POST, sb.st);
-    hp::PostArgs pa{};
-    pa.Sf = sf; pa.sf_bs = o.sf_bs; pa.X = OFFS(e->X, 2 * Tp * Np); pa.Ft = OFFS(e->Ft, 2 * (m ? m : 1) * n);
-    pa.wd = OFFS(e->wd, 2 * Tp * n); pa.w = OFFS(e->w, n); pa.ninvd = OFFS(e->ninvd, n);
-    pa.fg_out = fg; pa.fg_bs = o.fg_bs; pa.chisq_out = chisq; pa.chisq_bs = o.chisq_bs;
-    pa.Wm = e->any_flagged ? OFFS(e->Wm, 2 * Tp * n) : nullptr; pa.Rm = e->cfg.dense_noise ? OFFS(e->Rm, 2 * Tp * n) : nullptr;
-    pa.lnp1 = OFFS(e->lnp1, Tp);
-    pa.n = e->n; pa.m = e->m; pa.Np = e->Np; pa.T = e->T; pa.Tp = e->Tp; pa.nsys = sb.nc;
-    hp::launch_post(pa, sb.st);
     e->prof_end(CLS_POST, 1, sb.st);
     if (e->cfg.dense_noise) enqueue_dense_lnp1(e, sb);
-    if (e->any_flagged || general) {
+    if (post == Post::Dense && (e->any_flagged || general)) {
         e->prof_begin(CLS_TRANSFORM, sb.st);
         int nl2 = 0;
         hp::ZgemmArgs t{};
@@ -1206,6 +1238,49 @@ static void enqueue_gcr(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb,
         }
         e->prof_end(CLS_TRANSFORM, nl2, sb.st);
     }
+}
+
+// Where enqueue_post left sum_t |U s|^2 (Eu, general-basis iteration) and sum_t |U (w s)|^2 (Em, flagged channels) for
+// k_sample: per-tile partial sums from k_post_fft / k_post_fft2, one sum per chain from the dense transforms
+static void sample_energies(hp_engine* e, const Sub& sb, hp::SampleArgs& sp) {
+    const size_t n = e->n;
+    const bool tiles = e->post != Post::Dense;
+    sp.ntilesE = tiles ? e->ntilesE : 0;
+    sp.Eu = tiles ? OFFS(e->Eupart, (size_t)e->ntilesE * n) : OFFS(e->Eu, n);
+    sp.Em = e->any_flagged ? (tiles ? OFFS(e->Empart, (size_t)e->ntilesE * n) : OFFS(e->Em, n)) : nullptr;
+}
+
+// GCR step (gcr_fgmodes) and everything of gibbs_step_fgmodes up to the power-spectrum draw:
+// chol + solve + back-transform + residual statistics
+static void enqueue_gcr(hp_engine* e, const IterOut& o, const Sub& sb, const IterStep& step) {
+    Basis& b = step.general ? e->b0 : e->bF;
+    const hp::DrawKey dk = draw_key(e, sb, step.draw_iter);
+    // the general-basis first iteration needs Eupart, which k_post_fft2 does not write; the post-processing fuses the inverse
+    // transform otherwise, and the solve leaves lam * ytilde in Ssc for a dense back-transform only when it does not
+    const Post post = (step.general && e->post == Post::Fft2) ? Post::Fft : e->post;
+    const bool ssc = post == Post::Dense || step.general;
+    const bool philox = e->cfg.rng_mode == HP_RNG_PHILOX;
+    const double* wa = (!philox && e->any_omega) ? OFFS(b.wa, 2 * (size_t)e->Tp * e->Np) : nullptr;
+    if (e->solve != Solve::PtDirect) {
+        const size_t Np = e->Np, tri = hp::tri_blocks(e->nblk);
+        e->prof_begin(CLS_CHOL, sb.st);
+        hp::CholArgs ca{};
+        ca.Gp = OFFS(b.Gp, tri * hp::kBlkDoubles); ca.lam = OFFS(e->lam, Np); ca.Lp = OFFS(e->Lp, tri * hp::kLBlkDoubles);
+        ca.Linvp = OFFS(e->Linvp, (size_t)e->nblk * hp::kLBlkDoubles); ca.info = e->info + sb.c0;
+        ca.nblk = e->nblk; ca.n = e->n; ca.N = e->N; ca.nsys = sb.nc;
+        // Philox mode: the stored right-hand-side tiles are the unscaled Rfix, so pass 1 multiplies by W diag(lam)
+        const hp::TrinvExtra ex{OFFS(e->Wf1, hp::solve3_frag_doubles(e->nblk)), OFFS(e->Wf2, hp::solve3_frag_doubles(e->nblk)),
+                                philox ? OFFS(e->lam, Np) : nullptr};
+        e->prof_end(CLS_CHOL, hp::launch_chol_trinv(ca, OFFS(e->Wp, tri * hp::kLBlkDoubles), ex, sb.st), sb.st);
+    }
+    switch (e->solve) {
+        case Solve::Solve3: solve_solve3(e, b, sb, dk, wa, ssc); break;
+        case Solve::Resident: solve_resident(e, b, sb, dk, wa, ssc); break;
+        case Solve::Dense: solve_dense(e, b, sb, dk, wa, ssc); break;
+        case Solve::PtLowRank: solve_pt_lowrank(e, b, sb, dk, wa, ssc); break;
+        case Solve::PtDirect: solve_pt_direct(e, b, sb, dk, wa); break;
+    }
+    enqueue_post(e, b, o, sb, post, ssc);
 }
 
 // sub-batches of the engine: [c0, c0 + nc) on stream st (the engine's own stream when there is one range)
@@ -1240,47 +1315,21 @@ int hp_engine_gcr(hp_engine* e) {
     if (e->ahead > 0) return fail(HP_ERR_ARG, kAheadMsg);
     CU_TRY(cudaSetDevice(e->cfg.device));
     { int rcf = flush_pending(e); if (rcf != HP_OK) return rcf; }
-    Basis& b = (e->cfg.general_basis0 && e->iter == 0) ? e->b0 : e->bF;
+    const IterStep step = iter_step(e, false);
     IterOut o{e->Sf, (long long)e->Tp * e->n, nullptr, 0, nullptr, 0};
-    const bool philox = e->cfg.rng_mode == HP_RNG_PHILOX;
-    const uint32_t draw_iter = (philox && !e->cfg.refresh_omega) ? 0u : e->draw_counter++;
     auto subs = make_subs(e);
     fork_subs(e, subs);
-    for (auto& sb : subs) enqueue_gcr(e, b, o, sb, draw_iter);
+    for (auto& sb : subs) enqueue_gcr(e, o, sb, step);
     join_subs(e, subs);
     CU_TRY(cudaGetLastError());
     return HP_OK;
 }
 
-// Whether the next computed iteration is accumulated into the posterior moments: after hp_engine_set_summary the first
-// burn_in iterations are skipped, then every thin-th one is taken.  Decided on the host once per iteration, for all
-// sub-batches alike, and so is whether it closes a batch of the batch means (the count reaches j * batch).
-struct SumStep {
-    double invk = 0.0;   // 1 / (accumulated iterations including this one); 0: not accumulated
-    double jj1 = -1.0;   // j (j - 1) when the iteration closes batch j; < 0: it closes none
-};
-static SumStep summary_step(hp_engine* e) {
-    auto& s = e->sum;
-    SumStep r;
-    if (!s.what) return r;
-    const long long k = s.seen++ - s.burn_in;
-    if (k < 0 || k % s.thin != 0) return r;
-    r.invk = 1.0 / (double)(++s.count);
-    if (s.batch > 0 && s.count % s.batch == 0) {
-        const double j = (double)(s.count / s.batch);
-        r.jj1 = j * (j - 1.0);
-    }
-    return r;
-}
-
-// one Gibbs iteration of all chains (gibbs_step_fgmodes, pspec.py:377-490), enqueued on e->st
 // one Gibbs iteration (gibbs_step_fgmodes, pspec.py:377-490) of the chains of one sub-batch
-// sum.invk > 0: accumulate the iteration into the posterior moments (SumStep)
-static void enqueue_iteration_sub(hp_engine* e, const Sub& sb, int it, uint32_t iter, uint32_t draw_iter, bool general,
-                                  const SumStep& sum) {
+// step.sum.invk > 0: accumulate the iteration into the posterior moments (SumStep)
+static void enqueue_iteration_sub(hp_engine* e, const Sub& sb, int it, uint32_t iter, const IterStep& step) {
     const size_t n = e->n, m = e->m, T = e->T, Tp = e->Tp, I = e->cfg.max_iters, Np = e->Np;
     const bool philox = e->cfg.rng_mode == HP_RNG_PHILOX;
-    Basis& b = general ? e->b0 : e->bF;
     IterOut o{};
     const size_t R = e->ring, slot = (size_t)it % R;   // big outputs: ring slot; signal_ps / ln_post: one entry per iteration
     // ring layout [slot][chain][...]: one iteration's array of all chains is contiguous (one plain copy to the host)
@@ -1289,9 +1338,9 @@ static void enqueue_iteration_sub(hp_engine* e, const Sub& sb, int it, uint32_t 
     o.sf_bs = e->cr_out ? (long long)(T * n) : (long long)(Tp * n);
     o.fg = e->fg_out ? e->fg_out + 2 * slot * Cn * T * m : nullptr; o.fg_bs = 2 * (long long)(T * m);
     o.chisq = e->chisq_out ? e->chisq_out + slot * Cn * T * n : nullptr; o.chisq_bs = (long long)(T * n);
-    enqueue_gcr(e, b, o, sb, draw_iter);
+    enqueue_gcr(e, o, sb, step);
 
-    if (sum.invk > 0.0) {
+    if (step.sum.invk > 0.0) {
         // signal_cr from the slot the iteration wrote; fg_amps straight from the solution X (rows t < T, columns n .. n + m),
         // where HP_BUF_LAST_FG reads it too, so that it needs no HP_KEEP_FG
         const auto& s = e->sum;
@@ -1310,26 +1359,22 @@ static void enqueue_iteration_sub(hp_engine* e, const Sub& sb, int it, uint32_t 
             if (s.batch > 0) { fgb.snap = s.fg_snap + 2 * (size_t)sb.c0 * s.ld_fg; fgb.m2 = s.fg_m2bm + (size_t)sb.c0 * s.ld_fg; }
         }
         // only the iterations that close a batch run the longer k_moments_batch; the launch count is the same
-        e->launches += sum.jj1 >= 0.0 ? hp::launch_moments_batch(cr, fg, crb, fgb, sum.invk, sum.jj1, sb.st)
-                                      : hp::launch_moments(cr, fg, sum.invk, sb.st);
+        e->launches += step.sum.jj1 >= 0.0 ? hp::launch_moments_batch(cr, fg, crb, fgb, step.sum.invk, step.sum.jj1, sb.st)
+                                           : hp::launch_moments(cr, fg, step.sum.invk, sb.st);
     }
 
     e->prof_begin(CLS_SAMPLE, sb.st);
     hp::SampleArgs sp{};
-    sp.Ppart = OFFS(e->Ppart, (size_t)e->ntiles * n);
-    sp.ntilesE = e->fft_ok ? e->ntilesE : 0;
-    sp.Eu = e->fft_ok ? OFFS(e->Eupart, (size_t)e->ntilesE * n) : OFFS(e->Eu, n);
-    sp.Em = e->any_flagged ? (e->fft_ok ? OFFS(e->Empart, (size_t)e->ntilesE * n) : OFFS(e->Em, n)) : nullptr;
+    sp.Ppart = OFFS(e->Ppart, (size_t)e->ntiles * n); sp.ntiles = e->ppart_tiles;
+    sample_energies(e, sb, sp);
     sp.lnp1 = OFFS(e->lnp1, Tp); sp.lnp1_dense = nullptr; sp.prior = OFFS(e->prior, 2 * n);
     sp.draws = philox ? nullptr : OFFS(e->sdraws, I * n) + (size_t)it * n; sp.draws_bs = (long long)(I * n);
     sp.ps = OFFS(e->ps, n); sp.lam = OFFS(e->lam, Np);
     sp.ps_out = OFFS(e->ps_out, I * n) + (size_t)it * n; sp.ps_bs = (long long)(I * n);
     sp.lnpost_out = OFFS(e->lnpost_out, I) + it; sp.lnpost_bs = (long long)I;
     sp.n = e->n; sp.Np = e->Np; sp.T = e->T; sp.Tp = e->Tp; sp.nsys = sb.nc;
-    sp.ntiles = (e->cfg.time_flags || e->big_solve || (e->solve3 && e->cfg.cg_compat)) ? 1 : e->ntiles;  // 1: one partial sum per chain (k_colsumsq)
-    sp.beta_mode = general ? 1 : 0; sp.philox = philox ? 1 : 0;
-    sp.key0 = (uint32_t)e->cfg.seed; sp.key1 = (uint32_t)(e->cfg.seed >> 32); sp.iter = iter;
-    sp.chain_ids = OFFS(e->chain_ids, 1); sp.chain0 = sb.c0;
+    sp.beta_mode = step.general ? 1 : 0; sp.philox = philox ? 1 : 0;
+    sp.dk = draw_key(e, sb, iter);
     hp::launch_sample(sp, sb.st);
     e->prof_end(CLS_SAMPLE, 1, sb.st);
 }
@@ -1340,14 +1385,11 @@ static void enqueue_iteration_sub(hp_engine* e, const Sub& sb, int it, uint32_t 
 extern "C++" {
 template <typename F>
 static void enqueue_iterations(hp_engine* e, int niter, F&& after_iter) {
-    const bool philox = e->cfg.rng_mode == HP_RNG_PHILOX;
     auto subs = make_subs(e);
     fork_subs(e, subs);
     for (int k = 0; k < niter; ++k) {
-        const bool general = e->cfg.general_basis0 && e->iter == 0;
-        const uint32_t draw_iter = (philox && !e->cfg.refresh_omega) ? 0u : e->draw_counter++;
-        const SumStep sum = summary_step(e);
-        for (auto& sb : subs) enqueue_iteration_sub(e, sb, e->out_pos, (uint32_t)e->iter, draw_iter, general, sum);
+        const IterStep step = iter_step(e, true);
+        for (auto& sb : subs) enqueue_iteration_sub(e, sb, e->out_pos, (uint32_t)e->iter, step);
         e->iter++;
         e->out_pos++;
         if (after_iter(k)) { join_subs(e, subs); after_iter(-1 - k); if (k + 1 < niter) fork_subs(e, subs); }
@@ -1381,7 +1423,6 @@ int hp_engine_run_to_host(hp_engine* e, int niter, const hp_host_sink* sink) {
     const size_t n = e->n, m = e->m, T = e->T, I = e->cfg.max_iters, HI = sink->iters, R = e->ring, C = (size_t)e->C;
     const int first = e->out_pos;
     const bool big = sink->signal_cr || (sink->fg_amps && m) || sink->chisq;
-    const bool philox = e->cfg.rng_mode == HP_RNG_PHILOX;
     auto subs = make_subs(e);
     const size_t nsub = subs.size();
     if (e->ahead > 0 && (!big || e->it_done.size() < R * nsub))
@@ -1406,13 +1447,11 @@ int hp_engine_run_to_host(hp_engine* e, int niter, const hp_host_sink* sink) {
     // compute iteration `it` (the next one of the chain) into its ring slot; records it_done[slot][*]
     auto compute_next = [&](size_t it) {
         const size_t slot = it % R;
-        const bool general = e->cfg.general_basis0 && e->iter == 0;
-        const uint32_t draw_iter = (philox && !e->cfg.refresh_omega) ? 0u : e->draw_counter++;
-        const SumStep sum = summary_step(e);
+        const IterStep step = iter_step(e, true);
         for (size_t i = 0; i < nsub; ++i) {
             // the slot was last used by iteration it - R: wait for its copies unless they completed in an earlier call
             if (big && it >= R + (size_t)first) cudaStreamWaitEvent(subs[i].st, e->copy_done[slot], 0);
-            enqueue_iteration_sub(e, subs[i], (int)it, (uint32_t)e->iter, draw_iter, general, sum);
+            enqueue_iteration_sub(e, subs[i], (int)it, (uint32_t)e->iter, step);
             if (big) cudaEventRecord(e->it_done[slot * nsub + i], subs[i].st);
         }
         e->iter++;
@@ -1521,7 +1560,7 @@ int hp_engine_rewind(hp_engine* e) {
 long long hp_engine_launch_count(const hp_engine* e) { return e ? e->launches : -1; }
 int hp_engine_pt_form(const hp_engine* e, int* low_rank, int* max_rank) {
     if (!e) return fail(HP_ERR_ARG, "null engine");
-    if (low_rank) *low_rank = (e->cfg.time_flags && e->pt_low) ? 1 : 0;
+    if (low_rank) *low_rank = e->solve == Solve::PtLowRank ? 1 : 0;
     if (max_rank) *max_rank = e->pt_kcap;
     return HP_OK;
 }

@@ -169,28 +169,9 @@ __device__ __forceinline__ void build_twiddle_tables(double2* dst, const double2
 
 }  // namespace
 
-// Nfreqs covered by k_post_fft2 (compile-time plans): 128 = 4.4.4.2, 256 = 8.8.4, 384 = 6.4.4.4, 512 = 8.8.4.2, 1024 = 8.8.4.4.  The FftPlan outputs carry
-// the forward / reverse radices for reference; the kernel has them as template parameters.
-bool make_fft2_plan(int n, FftPlan* fwd, FftPlan* rev) {
-    int rad[4], nf;
-    if (n == 384) { rad[0] = 6; rad[1] = 4; rad[2] = 4; rad[3] = 4; nf = 4; }
-    else if (n == 1024) { rad[0] = 8; rad[1] = 8; rad[2] = 4; rad[3] = 4; nf = 4; }
-    else if (n == 512) { rad[0] = 8; rad[1] = 8; rad[2] = 4; rad[3] = 2; nf = 4; }
-    else if (n == 256) { rad[0] = 8; rad[1] = 8; rad[2] = 4; rad[3] = 1; nf = 3; }
-    else if (n == 128) { rad[0] = 4; rad[1] = 4; rad[2] = 4; rad[3] = 2; nf = 4; }
-    else return false;
-    for (int dir = 0; dir < 2; ++dir) {
-        FftPlan* p = dir ? rev : fwd;
-        p->n = n; p->nf = nf;
-        int Ns = 1;
-        for (int i = 0; i < nf; ++i) {
-            p->radix[i] = dir ? rad[nf - 1 - i] : rad[i];
-            p->magic[i] = Ns > 1 ? (uint32_t)((0x100000000ull + (uint64_t)Ns - 1) / (uint64_t)Ns) : 0u;
-            Ns *= p->radix[i];
-        }
-    }
-    return true;
-}
+// Nfreqs covered by k_post_fft2: its radices are template parameters, 128 = 4.4.4.2, 256 = 8.8.4, 384 = 6.4.4.4,
+// 512 = 8.8.4.2, 1024 = 8.8.4.4
+bool postfft2_ok(int n) { return n == 128 || n == 256 || n == 384 || n == 512 || n == 1024; }
 
 size_t postfft2_smem_bytes(int n, int m) {
     const int mk = ((m + 3) / 4) * 4;
@@ -245,19 +226,12 @@ __global__ void __launch_bounds__(32 * kTP2, (E >= 16 ? 1 : HP_FFT2_CTAS)) k_pos
             v[e] = make_double2(sg * y.x, -sg * y.y);
         }
     }
-    if (a.tw2) {
-        // the tables were built once per engine: a straight, coalesced copy (the per-CTA build is ~760 scattered 16-byte gathers
-        // with index arithmetic in front of every CTA's first pass)
-        const double2* t2 = reinterpret_cast<const double2*>(a.tw2);
-        const int cnt = a.Empart ? 2 * n : n;
-        for (int e = tid; e < cnt; e += kThreads) tw[e] = t2[e];
-    } else {
-        build_twiddle_tables<E, P0, P1, P2, P3>(tw, twg, tid, kThreads);
-        if (a.Empart) {
-            if constexpr (P3 > 1) build_twiddle_tables<E, P3, P2, P1, P0>(tw + n, twg, tid, kThreads);
-            else build_twiddle_tables<E, P2, P1, P0, 1>(tw + n, twg, tid, kThreads);
-        }
-    }
+    // the tables were built once per engine: a straight, coalesced copy (the per-CTA build is ~760 scattered 16-byte gathers
+    // with index arithmetic in front of every CTA's first pass)
+    const double2* t2 = reinterpret_cast<const double2*>(a.tw2);
+    const int cnt = a.Empart ? 2 * n : n;
+#pragma unroll 8   // the compiler's default unrolling hoists these loads over the first pass: 6 more registers at 1024 channels
+    for (int e = tid; e < cnt; e += kThreads) tw[e] = t2[e];
     for (int e = tid; e < kTP2 * ldf; e += kThreads) {
         const int tt = e / ldf, j = e - tt * ldf;
         double2 f = make_double2(0.0, 0.0);
@@ -407,7 +381,7 @@ __global__ void __launch_bounds__(256) k_fft2_tables(double2* tw2, const double2
 }
 }  // namespace
 
-bool launch_fft2_tables(double* tw2, const double* tw, int n, cudaStream_t st) {
+void launch_fft2_tables(double* tw2, const double* tw, int n, cudaStream_t st) {
     double2* o = reinterpret_cast<double2*>(tw2);
     const double2* t = reinterpret_cast<const double2*>(tw);
     if (n == 128) k_fft2_tables<4, 4, 4, 4, 2><<<1, 256, 0, st>>>(o, t);
@@ -415,14 +389,10 @@ bool launch_fft2_tables(double* tw2, const double* tw, int n, cudaStream_t st) {
     else if (n == 384) k_fft2_tables<12, 6, 4, 4, 4><<<1, 256, 0, st>>>(o, t);
     else if (n == 512) k_fft2_tables<16, 8, 8, 4, 2><<<1, 256, 0, st>>>(o, t);
     else if (n == 1024) k_fft2_tables<32, 8, 8, 4, 4><<<1, 256, 0, st>>>(o, t);
-    else return false;
-    return true;
 }
 
-// true: the launch was taken by k_post_fft2
-bool launch_post_fft2(const PostFftArgs& a, const FftPlan& fwd, const FftPlan& rev, cudaStream_t st) {
-    (void)rev;
-    const int n = fwd.n;
+void launch_post_fft2(const PostFftArgs& a, cudaStream_t st) {
+    const int n = a.plan.n;
     const size_t smem = postfft2_smem_bytes(n, a.m);
     static size_t attr_dev[kMaxDev][5] = {{0}};
     const int slot = n == 128 ? 0 : (n == 256 ? 1 : (n == 384 ? 2 : (n == 512 ? 3 : 4)));
@@ -443,10 +413,7 @@ bool launch_post_fft2(const PostFftArgs& a, const FftPlan& fwd, const FftPlan& r
     } else if (n == 1024) {
         if (smem > attr) { cudaFuncSetAttribute(k_post_fft2<32, 8, 8, 4, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); attr = smem; }
         k_post_fft2<32, 8, 8, 4, 4><<<grid, 32 * kTP2, smem, st>>>(a);
-    } else {
-        return false;
     }
-    return true;
 }
 
 }  // namespace hp

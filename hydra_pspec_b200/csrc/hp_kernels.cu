@@ -423,7 +423,7 @@ __global__ void __launch_bounds__(1024) k_sample(SampleArgs a) {
     const double* prior = a.prior + (size_t)sys * 2 * n;
     const double* draws = a.draws ? a.draws + (size_t)sys * a.draws_bs : nullptr;
     const double alpha = (double)a.T - 1.0;  // pspec.py:108
-    const uint32_t chain = a.chain_ids ? (uint32_t)a.chain_ids[sys] : (uint32_t)(a.chain0 + sys);
+    const uint32_t chain = a.philox ? (uint32_t)a.dk.chain_ids[sys] : 0u;
 
     double lp2 = 0.0;  // sum_k E_k / Lambda'_k
     for (int k0 = 0; k0 < n; k0 += 1024) {
@@ -445,7 +445,7 @@ __global__ void __launch_bounds__(1024) k_sample(SampleArgs a) {
             has_prior = prior[k] > 0.0 || prior[n + k] > 0.0;  // pspec.py:114
             if (!has_prior) {
                 if (!a.philox) newps = draws[k] * beta;  // invgamma.rvs(a=alpha) * beta, pspec.py:125
-                else newps = beta / gamma_mt(alpha, (uint32_t)k, a.iter, chain, a.key0, a.key1 ^ 0x5A5A5A5Au);
+                else newps = beta / gamma_mt(alpha, (uint32_t)k, a.dk.iter, chain, a.dk.key0, a.dk.key1 ^ 0x5A5A5A5Au);
             }
         }
         // prior-bounded bins: inversion sampling, one bin at a time, grid evaluated by the CTA
@@ -492,8 +492,8 @@ __global__ void __launch_bounds__(1024) k_sample(SampleArgs a) {
             double u;
             if (!a.philox) u = draws[kk];
             else {
-                u32x4 ctr; ctr.x = (uint32_t)kk; ctr.y = a.iter; ctr.z = 0xFFFFu; ctr.w = chain;
-                u32x4 r = philox4x32_10(ctr, a.key0, a.key1 ^ 0x5A5A5A5Au);
+                u32x4 ctr; ctr.x = (uint32_t)kk; ctr.y = a.dk.iter; ctr.z = 0xFFFFu; ctr.w = chain;
+                u32x4 r = philox4x32_10(ctr, a.dk.key0, a.dk.key1 ^ 0x5A5A5A5Au);
                 u = u53(r.x, r.y);
             }
             // bracket: lo = last kept with cdf <= u ; hi = first kept with cdf > u

@@ -56,6 +56,10 @@ void launch_pack_lower(const double* dense, long long ld, long long bs, double* 
                        int batch, cudaStream_t st);
 
 // ---- per-iteration kernels ---------------------------------------------------------------
+// Identity of a launch's Philox draws: the key (the engine seed), the draw counter and the global chain id of every
+// system, chain_ids[nsys] (read only when the kernel draws).  Each kernel builds its own counters from it.
+struct DrawKey { uint32_t key0, key1, iter; const int* chain_ids; };
+
 struct CholArgs {
     const double* Gp;      // [nsys][tri_blocks][2048]
     const double* lam;     // [nsys][Np]   (lambda for rows < n, 1 for fg rows, 0 for padding)
@@ -87,9 +91,7 @@ struct SolveArgs {
     int stages;            // ring depth (set by launch_solve)
     int rows_per_round;    // times staged through the ring area per round (set by launch_solve)
     int cg_compat;         // 1: scale each column by the scalar CG model (hp_math.h:cg_theta)
-    uint32_t key0, key1, iter;
-    const int* chain_ids;  // [nsys] global chain id for the philox counter (or null -> chain0 + sys index)
-    int chain0;
+    DrawKey dk;
 };
 void launch_solve(const SolveArgs& a, cudaStream_t st);
 size_t solve_smem_bytes(int nblk);
@@ -111,9 +113,7 @@ struct Solve3Args {
     double* Ppart;         // [nsys][ntiles][n]
     int nblk, n, N, Tp, ntiles, nsys, T;
     int philox;
-    uint32_t key0, key1, iter;
-    const int* chain_ids;
-    int chain0;
+    DrawKey dk;
     int grid_limit;        // > 0: cap on the persistent grid (sub-batches sharing the GPU); 0 = one CTA per SM
     int nstrip;            // 16-row strips holding rows of the system, ceil(N / 16) (0: all 2 nblk); must match the schedule
     Solve3Sched sched;
@@ -162,9 +162,7 @@ struct PtArgs {
     int* info;             // [nsys], zeroed by the caller; atomicMax(k + 1) on a non-positive pivot in block column k
     int nblk, n, m, N, T, Tp, nsys;
     int philox_wa;
-    uint32_t key0, key1, iter;
-    const int* chain_ids;
-    int chain0;
+    DrawKey dk;
 };
 size_t pt_smem_bytes(int nblk, int n);
 size_t pt_scratch_doubles_per_cta(int nblk);
@@ -187,9 +185,7 @@ struct PtLowArgs {
     int* info;             // [nsys]: atomicMax(nblk + 1) when a K_t is not positive definite
     int n, N, Np, T, Tp, Tp0, nsys, nblk, kcap;   // kcap: largest count in fcnt (shared-memory sizing)
     int philox;
-    uint32_t key0, key1, iter;
-    const int* chain_ids;
-    int chain0;
+    DrawKey dk;
 };
 size_t pt_lowrank_smem_bytes(int kcap, int warps);
 void launch_pt_lowrank(const PtLowArgs& a, cudaStream_t st);
@@ -211,9 +207,7 @@ struct SampleArgs {
     int n, Np, T, Tp, ntiles, nsys;
     int beta_mode, philox;
     int ntilesE;           // > 0: Em / Eu are per-tile partial sums [nsys][ntilesE][n]
-    uint32_t key0, key1, iter;
-    const int* chain_ids;
-    int chain0;
+    DrawKey dk;
     long long ps_bs, lnpost_bs, draws_bs;
 };
 void launch_sample(const SampleArgs& a, cudaStream_t st);
@@ -230,7 +224,7 @@ struct PostFftArgs {
     FftPlan plan;
     const double* tw;
     const double* tw2;     // k_post_fft2: per-pass twiddle tables of the forward plan ([0, n)) and of the reverse plan ([n, 2 n)),
-                           //   built once per engine (launch_fft2_tables); null: every CTA derives them from tw
+                           //   built once per engine (launch_fft2_tables)
     const double* X;       // [nsys][Tp][Np]
     const double* lam;     // [nsys][Np]
     double* Sf;            // [nsys][..][n] frequency-space signal: written (do_inverse) or read
@@ -248,10 +242,10 @@ struct PostFftArgs {
 };
 void launch_post_fft(const PostFftArgs& a, cudaStream_t st);
 // k_post_fft2 (hp_fft2.cu): register-resident FFTs, one shared-memory buffer; needs do_inverse = 1 and Eupart = NULL
-bool make_fft2_plan(int n, FftPlan* fwd, FftPlan* rev);   // false: Nfreqs not covered (k_post_fft takes it)
+bool postfft2_ok(int n);   // false: Nfreqs not covered (k_post_fft takes it)
 size_t postfft2_smem_bytes(int n, int m);
-bool launch_post_fft2(const PostFftArgs& a, const FftPlan& fwd, const FftPlan& rev, cudaStream_t st);
-bool launch_fft2_tables(double* tw2, const double* tw, int n, cudaStream_t st);   // tw2: 4 n doubles; false: Nfreqs not covered
+void launch_post_fft2(const PostFftArgs& a, cudaStream_t st);   // a.plan.n: an Nfreqs of postfft2_ok
+void launch_fft2_tables(double* tw2, const double* tw, int n, cudaStream_t st);   // tw2: 4 n doubles; n: an Nfreqs of postfft2_ok
 
 // k_moments (hp_moments.cu): Welford update of per-chain posterior moments from one iteration's samples.
 // Element i < L of chain c is src[c * src_cs + (i / w) * rs + i % w] (complex); its accumulators are mean[c * ld + i]

@@ -277,11 +277,11 @@ __global__ void __launch_bounds__(kPT, 2) k_pt_cholsolve(PtArgs a) {
 
         // ---- fluctuation term: y += xi, xi ~ CN(0, I)   (same counter layout as k_solve)
         if (a.philox_wa) {
-            const uint32_t chain = a.chain_ids ? (uint32_t)a.chain_ids[sys] : (uint32_t)(a.chain0 + sys);
+            const uint32_t chain = (uint32_t)a.dk.chain_ids[sys];
             for (int row = tid; row < N; row += kPT) {
-                u32x4 ctr; ctr.x = (uint32_t)row; ctr.y = (uint32_t)t; ctr.z = a.iter; ctr.w = chain;
+                u32x4 ctr; ctr.x = (uint32_t)row; ctr.y = (uint32_t)t; ctr.z = a.dk.iter; ctr.w = chain;
                 double n0, n1;
-                normal_pair_fast(philox4x32_10(ctr, a.key0, a.key1 ^ 0xA5A5A5A5u), n0, n1);
+                normal_pair_fast(philox4x32_10(ctr, a.dk.key0, a.dk.key1 ^ 0xA5A5A5A5u), n0, n1);
                 yr[row] += n0 * 0.70710678118654752440;
                 yi[row] += n1 * 0.70710678118654752440;
             }

@@ -167,11 +167,11 @@ __global__ void __launch_bounds__(256, HP_PTLOW_MINB) k_pt_lowrank(PtLowArgs a) 
         }
         if (bad && lane == 0) atomicMax(a.info + sys, a.nblk + 1);
         if (a.philox) {
-            const uint32_t chain = a.chain_ids ? (uint32_t)a.chain_ids[sys] : (uint32_t)(a.chain0 + sys);
+            const uint32_t chain = (uint32_t)a.dk.chain_ids[sys];
             for (int e = lane; e < k; e += 32) {
-                u32x4 ctr; ctr.x = 0x80000000u + (uint32_t)e; ctr.y = (uint32_t)t; ctr.z = a.iter; ctr.w = chain;
+                u32x4 ctr; ctr.x = 0x80000000u + (uint32_t)e; ctr.y = (uint32_t)t; ctr.z = a.dk.iter; ctr.w = chain;
                 double x0, x1;
-                normal_pair(philox4x32_10(ctr, a.key0, a.key1 ^ 0xA5A5A5A5u), x0, x1);
+                normal_pair(philox4x32_10(ctr, a.dk.key0, a.dk.key1 ^ 0xA5A5A5A5u), x0, x1);
                 wv[e].x += x0 * 0.70710678118654752440; wv[e].y += x1 * 0.70710678118654752440;
             }
             __syncwarp();

@@ -222,7 +222,7 @@ __global__ void __launch_bounds__(544) k_solve(SolveArgs a) {
     rc.Rfix = a.Rfix + 2 * (size_t)sys * a.Tp * Np;
     rc.wa = a.wa ? a.wa + 2 * (size_t)sys * a.Tp * Np : nullptr;
     rc.lam = lam; rc.Np = Np; rc.n = a.n; rc.N = a.N; rc.T = a.T; rc.t0 = tile * kTT;
-    const uint32_t chain = a.chain_ids ? (uint32_t)a.chain_ids[sys] : (uint32_t)(a.chain0 + sys);
+    const uint32_t chain = a.philox_wa ? (uint32_t)a.dk.chain_ids[sys] : 0u;
     const int g = lane >> 2, q = lane & 3;
     // Warp tile: rows 8 ti.., columns 8 tj...  The two column groups (tj = 0, 1) never touch each
     // other's columns; they share only the ring.
@@ -325,8 +325,8 @@ __global__ void __launch_bounds__(544) k_solve(SolveArgs a) {
         {
             const int row = 32 * i + 8 * ti + g, c = 8 * tj + 2 * q + kh;
             if (a.philox_wa && row < a.N && rc.t0 + c < a.T) {
-                u32x4 ctr; ctr.x = (uint32_t)row; ctr.y = (uint32_t)(rc.t0 + c); ctr.z = a.iter; ctr.w = chain;
-                normal_pair_fast(philox4x32_10(ctr, a.key0, a.key1 ^ 0xA5A5A5A5u), xi0, xi1);
+                u32x4 ctr; ctr.x = (uint32_t)row; ctr.y = (uint32_t)(rc.t0 + c); ctr.z = a.dk.iter; ctr.w = chain;
+                normal_pair_fast(philox4x32_10(ctr, a.dk.key0, a.dk.key1 ^ 0xA5A5A5A5u), xi0, xi1);
                 xi0 *= 0.70710678118654752440; xi1 *= 0.70710678118654752440;
             }
         }

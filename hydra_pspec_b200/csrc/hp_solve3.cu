@@ -225,7 +225,7 @@ __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
     uint32_t it = 0;
     for (int w = blockIdx.x; w < total; w += gridDim.x, ++it) {
         const int sys = w / a.ntiles, tile = w - sys * a.ntiles, t0 = tile * kTT;
-        const uint32_t chain = a.chain_ids ? (uint32_t)a.chain_ids[sys] : (uint32_t)(a.chain0 + sys);
+        const uint32_t chain = a.philox ? (uint32_t)a.dk.chain_ids[sys] : 0u;
         mbar_wait(rhs_full, it & 1);
         S3_T(6);
         // ------------------------------------------------------------------ pass 1:  y = W1 r (+ xi)
@@ -270,12 +270,12 @@ __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
 #else
                         if (a.philox && row < a.N && t0 + col < a.T) {
 #endif
-                            u32x4 ctr; ctr.x = (uint32_t)row; ctr.y = (uint32_t)(t0 + col); ctr.z = a.iter; ctr.w = chain;
+                            u32x4 ctr; ctr.x = (uint32_t)row; ctr.y = (uint32_t)(t0 + col); ctr.z = a.dk.iter; ctr.w = chain;
                             double x0, x1;
 #ifdef HP_PHILOX_DOUBLE   // experiment (profiles/r2_summary.md): what full double-precision Box-Muller costs this kernel
-                            normal_pair(philox4x32_10(ctr, a.key0, a.key1 ^ 0xA5A5A5A5u), x0, x1);
+                            normal_pair(philox4x32_10(ctr, a.dk.key0, a.dk.key1 ^ 0xA5A5A5A5u), x0, x1);
 #else
-                            normal_pair_fast(philox4x32_10(ctr, a.key0, a.key1 ^ 0xA5A5A5A5u), x0, x1);
+                            normal_pair_fast(philox4x32_10(ctr, a.dk.key0, a.dk.key1 ^ 0xA5A5A5A5u), x0, x1);
 #endif
                             vr += x0 * 0.70710678118654752440; vi += x1 * 0.70710678118654752440;
                         }
