@@ -13,7 +13,6 @@
 // work arrays), so every access is coalesced; V stays unitary to round-off by construction.
 #include "hp_kernels.cuh"
 #include "../../include/hydra_pspec_b200.h"
-#include <cstdlib>
 #include <vector>
 
 namespace hp {
@@ -254,8 +253,6 @@ extern "C" int hp_eigh_batch(int device, int n, int batch, const double* S, doub
         cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
         int bw = (int)((size_t)(max_smem > 8192 ? max_smem - 8192 : 0) / ((size_t)4 * n * 16));
         if (bw > 8) bw = 8;
-        const char* ub = getenv("HP_EIGH_UNBLOCKED");   // A/B runs
-        if (ub && ub[0] == '1') bw = 0;
         const int nb = bw >= 2 ? (n + bw - 1) / bw : 0, nbe = nb + (nb & 1);
         const size_t bsmem = (size_t)4 * bw * n * 16;
         if (bw >= 2) cudaFuncSetAttribute(hp::k_eigh_block_round, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem);

@@ -423,9 +423,8 @@ int select_paths(hp_engine* e, size_t max_smem) {
     e->ntilesE = hp::postfft_tiles(e->T, e->ktp > 0 ? e->ktp : 8);
     const bool s3 = hp::solve3_ok(e->nblk, max_smem);
     if (cfg.time_flags) {
-        // low-rank form on top of k_solve3 unless HP_PT_DIRECT=1 (A/B runs, tests of k_pt_cholsolve)
-        const char* pd = getenv("HP_PT_DIRECT");
-        const bool low = !(pd && pd[0] == '1') && !cfg.force_dense_solve && s3 && e->n < 65536;
+        // low-rank form on top of k_solve3 unless force_dense_solve asks for one factorisation per time
+        const bool low = !cfg.force_dense_solve && s3 && e->n < 65536;
         e->solve = low ? Solve::PtLowRank : Solve::PtDirect;
         // a general (non-delay-diagonal) S_initial is possible in the low-rank form only: k_pt_cholsolve relies on the
         // circulant signal block of the delay basis

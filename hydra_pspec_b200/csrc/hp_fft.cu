@@ -15,18 +15,8 @@
 #include "hp_kernels.cuh"
 #include "hp_math.h"
 #include "hp_mma.cuh"
-#include <cstdlib>
 
 namespace hp {
-
-// Phase timers of k_post_fft (build with -DHP_POST_TIMERS; profiles/scripts/post_timers.py): clock64 deltas of thread 0
-// of every CTA.  [0] tables + f + X load  [1] FFT 1  [2] post-twiddle + Sf store  [3] F f (DMMA)  [4] residual  [5] FFT 2 + E
-#ifdef HP_POST_TIMERS
-__device__ unsigned long long g_post_cycles[8];
-#define PO_T(idx) do { if (tid == 0) { long long _n = clock64(); tacc[idx] += _n - tlast; tlast = _n; } } while (0)
-#else
-#define PO_T(idx) do { } while (0)
-#endif
 
 namespace {
 
@@ -175,9 +165,6 @@ size_t postfft_smem_bytes(int n, int m, int ktp) {
     return sizeof(double2) * ((size_t)2 * ktp * n + n + (size_t)ktp * (mk + 1)) + 64 * sizeof(double);
 }
 int postfft_ktp(int n, int m, size_t max_smem) {
-    static int forced = -1;   // HP_POSTFFT_KTP=4|8: experiments
-    if (forced < 0) { const char* e = getenv("HP_POSTFFT_KTP"); forced = e ? atoi(e) : 0; }
-    if ((forced == 4 || forced == 8) && postfft_smem_bytes(n, m, forced) <= max_smem) return forced;
     for (int ktp = 8; ktp >= 4; ktp /= 2)
         if (postfft_smem_bytes(n, m, ktp) <= max_smem) return ktp;
     return 0;
@@ -210,9 +197,6 @@ __global__ void __launch_bounds__(32 * kTP, kTP == 8 ? 2 : 1) k_post_fft(PostFft
         for (size_t off = (size_t)tid * 128; off < bytes; off += kThreads * 128)
             asm volatile("prefetch.global.L2 [%0];" ::"l"(wdp + off));
     }
-#ifdef HP_POST_TIMERS
-    long long tacc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tlast = clock64();
-#endif
     for (int j = tid; j < n; j += kThreads) tw[j] = twg[j];
     for (int e = tid; e < kTP * ldf; e += kThreads) {
         int t = e / ldf, j = e - t * ldf;
@@ -252,9 +236,7 @@ __global__ void __launch_bounds__(32 * kTP, kTP == 8 ? 2 : 1) k_post_fft(PostFft
             }
         }
         __syncthreads();
-        PO_T(0);
         double2* res = fft_forward(buf0, buf1, kTP, a.plan, tw);
-        PO_T(1);
         {
             const int t = warp;
             const bool live = t0 + t < a.T;
@@ -277,7 +259,6 @@ __global__ void __launch_bounds__(32 * kTP, kTP == 8 ? 2 : 1) k_post_fft(PostFft
     }
     double2* obuf = sbuf == buf0 ? buf1 : buf0;
     __syncthreads();
-    PO_T(2);
     // foreground model F f on the tensor pipe:  obuf[t][x] = sum_j f[t][j] Ft[j][x]
     // A = f tile (8 x m) stays in registers for all column tiles; the B fragments of a tile come
     // straight from global (L2-resident Ft) as one 16-byte load per k-step, issued as a batch and
@@ -330,7 +311,6 @@ __global__ void __launch_bounds__(32 * kTP, kTP == 8 ? 2 : 1) k_post_fft(PostFft
             for (int e = tid; e < kTP * n; e += kThreads) obuf[e] = make_double2(0.0, 0.0);
     }
     __syncthreads();
-    PO_T(3);
     // residual, chi^2, ln-posterior partial, masked signal
     {
         const double* wd = a.wd + 2 * ((size_t)sys * a.Tp + t0) * n;
@@ -380,7 +360,6 @@ __global__ void __launch_bounds__(32 * kTP, kTP == 8 ? 2 : 1) k_post_fft(PostFft
         }
     }
     __syncthreads();
-    PO_T(4);
     // |U (w s)|^2 summed over the tile's times (second term of ln_post, pspec.py:479-483)
     if (a.Empart) {
         double2* res = fft_forward(obuf, sbuf, kTP, a.plan, tw);
@@ -393,10 +372,6 @@ __global__ void __launch_bounds__(32 * kTP, kTP == 8 ? 2 : 1) k_post_fft(PostFft
         }
     }
     __syncthreads();
-    PO_T(5);
-#ifdef HP_POST_TIMERS
-    if (tid == 0) for (int i = 0; i < 8; ++i) atomicAdd(&g_post_cycles[i], (unsigned long long)tacc[i]);
-#endif
     // |U s|^2 (unmasked) for the general-basis iteration: reload s from global
     if (a.Eupart) {
         __syncthreads();
@@ -419,14 +394,6 @@ __global__ void __launch_bounds__(32 * kTP, kTP == 8 ? 2 : 1) k_post_fft(PostFft
         }
     }
 }
-
-#ifdef HP_POST_TIMERS
-extern "C" void hp_post_timers(unsigned long long* out, int reset) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_post_cycles, sizeof(unsigned long long) * 8);
-    if (reset) { unsigned long long z[8] = {0}; cudaMemcpyToSymbol(g_post_cycles, z, sizeof(z)); }
-}
-#endif
 
 int postfft_tiles(int T, int ktp) { return (T + ktp - 1) / ktp; }
 

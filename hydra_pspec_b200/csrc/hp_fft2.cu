@@ -21,16 +21,13 @@
 #include "hp_kernels.cuh"
 #include "hp_math.h"
 #include "hp_mma.cuh"
-#include <cstdlib>
 
 namespace hp {
 
 namespace {
 
 constexpr int kTP2 = 8;   // times per CTA = warps per CTA
-#ifndef HP_FFT2_CTAS
-#define HP_FFT2_CTAS 2     // resident CTAs per SM the register budget is sized for
-#endif
+constexpr int kFft2Ctas = 2;   // resident CTAs per SM the register budget is sized for
 
 __device__ __forceinline__ double2 cmul(double2 a, double2 b) { return make_double2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
 __device__ __forceinline__ double2 cadd(double2 a, double2 b) { return make_double2(a.x + b.x, a.y + b.y); }
@@ -181,7 +178,7 @@ size_t postfft2_smem_bytes(int n, int m) {
 
 // E = Nfreqs / 32; forward radices P0 P1 P2 (P3); the second transform runs them in reverse order
 template <int E, int P0, int P1, int P2, int P3>
-__global__ void __launch_bounds__(32 * kTP2, (E >= 16 ? 1 : HP_FFT2_CTAS)) k_post_fft2(PostFftArgs a) {
+__global__ void __launch_bounds__(32 * kTP2, (E >= 16 ? 1 : kFft2Ctas)) k_post_fft2(PostFftArgs a) {
     constexpr int kThreads = 32 * kTP2;
     constexpr int n = 32 * E, ld = n + n / 8 + 1;
     constexpr int RL = P3 > 1 ? P3 : P2;      // last forward radix = first reverse radix

@@ -26,14 +26,6 @@
 #include "hp_diag.cuh"
 
 namespace hp {
-// Phase timers of k_pt_cholsolve (build with -DHP_PT_TIMERS; profiles/scripts/pt_timers.py): clock64 deltas of thread 0
-// of every CTA, accumulated per phase.
-#ifdef HP_PT_TIMERS
-__device__ unsigned long long g_pt_cycles[8];
-#define PT_T(idx) do { if (tid == 0) { long long _n = clock64(); tacc[idx] += _n - tlast; tlast = _n; } } while (0)
-#else
-#define PT_T(idx) do { } while (0)
-#endif
 namespace {
 
 constexpr int kPT = 512;  // 16 warps: one 8x8 tile of a 32x32 block each
@@ -80,9 +72,6 @@ __global__ void __launch_bounds__(kPT, 2) k_pt_cholsolve(PtArgs a) {
     double* Lp = a.scratch + (size_t)blockIdx.x * (tri + nblk) * kLBlkDoubles;
     double* Vp = Lp + tri * kLBlkDoubles;
     const long long nitems = (long long)a.nsys * a.T;
-#ifdef HP_PT_TIMERS
-    long long tacc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tlast = clock64();
-#endif
 
     // Every CTA walks a contiguous range of (system, time) pairs.  Consecutive times of a baseline often carry the
     // same flag vector (persistent RFI channels): `same_prev[sys][t]` marks a time whose mask equals that of t - 1,
@@ -109,7 +98,6 @@ __global__ void __launch_bounds__(kPT, 2) k_pt_cholsolve(PtArgs a) {
         for (int e = tid; e < n; e += kPT) { double2 c = H[e]; chr[e] = c.x; chi[e] = c.y; }
         __syncthreads();
         int bad = 0;
-        PT_T(0);  // item prologue
 
         if (reuse) {
             // ---- forward substitution only, y_k = V_kk (r_k - sum_{j<k} L_kj y_j), with the factor of the previous time
@@ -192,7 +180,6 @@ __global__ void __launch_bounds__(kPT, 2) k_pt_cholsolve(PtArgs a) {
                     }
                     __syncthreads();  // stage st may be overwritten by the load issued in the next iteration
                 }
-                PT_T(1);  // j loop
                 warp_zgemm3m_finish<1, 1, false, true>(P3m, cr, ci);
                 // C = M_ik - acc with M generated on the fly
 #pragma unroll
@@ -221,12 +208,10 @@ __global__ void __launch_bounds__(kPT, 2) k_pt_cholsolve(PtArgs a) {
                     Ai[r * kLdBlk + c] = vi - ci[0][0][e];
                 }
                 __syncthreads();
-                PT_T(2);  // generation
                 if (i == k) {
                     // ---- Cholesky of the 32x32 diagonal block and its inverse, blocked 8x8 (hp_diag.cuh)
                     if (diag_chol_inverse_block(Ar, Ai, Vr, Vi, tid, kPT)) bad = k + 1;
                     __syncthreads();
-                    PT_T(3);  // diagonal block
                     // ---- y_k = V (r_k - sum_{j<k} L_kj y_j)
                     for (int o = 8; o > 0; o >>= 1) {
                         fr += __shfl_xor_sync(0xffffffffu, fr, o);
@@ -254,7 +239,6 @@ __global__ void __launch_bounds__(kPT, 2) k_pt_cholsolve(PtArgs a) {
                         Lb[e] = s.A[0][e];
                         Vb[e] = s.V[e];
                     }
-                    PT_T(4);  // y_k + store
                 } else {
                     // L_ik = C . V^H
                     double dr[1][1][2], di[1][1][2];
@@ -268,7 +252,6 @@ __global__ void __launch_bounds__(kPT, 2) k_pt_cholsolve(PtArgs a) {
                     const int r = 8 * ti + g, c = 8 * tj + 2 * q;
                     *reinterpret_cast<double2*>(Lb + r * kLdBlk + c) = make_double2(dr[0][0][0], dr[0][0][1]);
                     *reinterpret_cast<double2*>(Lb + kLPlane + r * kLdBlk + c) = make_double2(di[0][0][0], di[0][0][1]);
-                    PT_T(5);  // trsm
                 }
             }
         }
@@ -351,14 +334,9 @@ __global__ void __launch_bounds__(kPT, 2) k_pt_cholsolve(PtArgs a) {
             }
             __syncthreads();
         }
-        PT_T(6);  // noise + backward substitution
         double2* X = reinterpret_cast<double2*>(a.X) + ((size_t)sys * a.Tp + t) * Np;
         for (int e = tid; e < Np; e += kPT) X[e] = make_double2(yr[e], yi[e]);
-        PT_T(7);
     }
-#ifdef HP_PT_TIMERS
-    if (tid == 0) for (int i = 0; i < 8; ++i) atomicAdd(&g_pt_cycles[i], (unsigned long long)tacc[i]);
-#endif
 }
 
 }  // namespace
@@ -378,13 +356,6 @@ int pt_grid(int nsys, int T) {
     return (int)(items < ctas ? items : ctas);
 }
 
-#ifdef HP_PT_TIMERS
-extern "C" void hp_pt_timers(unsigned long long* out, int reset) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_pt_cycles, sizeof(unsigned long long) * 8);
-    if (reset) { unsigned long long z[8] = {0}; cudaMemcpyToSymbol(g_pt_cycles, z, sizeof(z)); }
-}
-#endif
 void launch_pt_cholsolve(const PtArgs& a, int grid, cudaStream_t st) {
     const size_t smem = pt_smem_bytes(a.nblk, a.n);
     static size_t attr_dev[kMaxDev] = {0};

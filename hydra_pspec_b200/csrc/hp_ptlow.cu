@@ -49,11 +49,9 @@ __global__ void __launch_bounds__(256) k_pt_arows(double* __restrict__ Rfix, con
 // Shared memory: a CTA-wide table that maps a packed lower-triangle index e to (row, column) (the inverse of
 // tri(r) + c: lets a warp spread a triangle of entries over its lanes), then per warp the packed K_t, three k-vectors
 // (c / z, w, 1 / L_jj) and the channel list.
-#ifndef HP_PTLOW_MINB
-#define HP_PTLOW_MINB 2   // resident CTAs per SM the register budget is sized for
-#endif
+constexpr int kPtLowMinBlocks = 2;   // resident CTAs per SM the register budget is sized for
 template <int kNJ>
-__global__ void __launch_bounds__(256, HP_PTLOW_MINB) k_pt_lowrank(PtLowArgs a) {
+__global__ void __launch_bounds__(256, kPtLowMinBlocks) k_pt_lowrank(PtLowArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
     const int kcap = a.kcap, ntri = tri(kcap);

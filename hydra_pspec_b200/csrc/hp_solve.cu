@@ -21,15 +21,8 @@
 #include "hp_kernels.cuh"
 #include "hp_math.h"
 #include "hp_mma.cuh"
-#include <cstdlib>
 
 namespace hp {
-
-// Phase timers of k_solve (build with -DHP_SOLVE_TIMERS; profiles/scripts/solve_timers.py): clock64 deltas of consumer
-// thread 0 of every CTA.  [0] staging  [1] pass 1  [2] pass 2  [3] epilogue  [4] ring waits  [5] row exchange + barrier
-#ifdef HP_SOLVE_TIMERS
-__device__ unsigned long long g_solve_cycles[8];
-#endif
 
 namespace {
 
@@ -234,12 +227,6 @@ __global__ void __launch_bounds__(544) k_solve(SolveArgs a) {
     const int ti = wt >> 1, tj = wt & 1;
     const int bcol = (8 * tj + g) ^ (q << 2);  // this lane's B-fragment column in the swizzled tile
 
-#ifdef HP_SOLVE_TIMERS
-    long long tacc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tlast = clock64();
-#define SV_T(idx) do { if (tid == 0) { long long _n = clock64(); tacc[idx] += _n - tlast; tlast = _n; } } while (0)
-#else
-#define SV_T(idx) do { } while (0)
-#endif
     // stage the right-hand sides:  tile[row][col] = lam_row Rfix[t0 + col][row] (+ wa).  The rows arrive
     // in the ring area by TMA (asynchronous, full DRAM burst instead of a load-use chain); a warp
     // instruction then moves 8 consecutive rows x 4 times: conflict-free 16-byte reads, at most 2-way
@@ -276,13 +263,7 @@ __global__ void __launch_bounds__(544) k_solve(SolveArgs a) {
 
     uint32_t slot = 0, parity = 0;  // ring slot being consumed and its phase parity
     auto acquire = [&]() -> const double* {
-#ifdef HP_SOLVE_TIMERS
-        long long t0_ = clock64();
         mbar_wait(&full[slot], parity);
-        if (tid == 0) tacc[4] += clock64() - t0_;
-#else
-        mbar_wait(&full[slot], parity);
-#endif
         return ring + (size_t)slot * kLBlkDoubles;
     };
     auto release = [&]() {
@@ -297,9 +278,6 @@ __global__ void __launch_bounds__(544) k_solve(SolveArgs a) {
     // block row i before it is overwritten in place (later rows of the pass never read it).
     uint32_t rowpar = 0;
     auto exchange = [&](double (&acc)[3][2], double (&P)[3]) {
-#ifdef HP_SOLVE_TIMERS
-        long long t0_ = clock64();
-#endif
         double* buf = scratch + (size_t)rowpar * kScratchDoubles;
         double* mine = buf + (((size_t)kh * 8 + wt) * 32 + lane) * 3;          // what I hand over
         const double* theirs = buf + (((size_t)(kh ^ 1) * 8 + wt) * 32 + lane) * 3;  // what my partner hands me
@@ -309,12 +287,8 @@ __global__ void __launch_bounds__(544) k_solve(SolveArgs a) {
 #pragma unroll
         for (int p = 0; p < 3; ++p) P[p] = (kh ? acc[p][1] : acc[p][0]) + theirs[p];
         rowpar ^= 1;
-#ifdef HP_SOLVE_TIMERS
-        if (tid == 0) tacc[5] += clock64() - t0_;
-#endif
     };
 
-    SV_T(0);
     // ------------------------------------------------------------------ pass 1:  y = W r (+ xi)
     for (int i = nblk - 1; i >= 0; --i) {
         double acc[3][2] = {{0, 0}, {0, 0}, {0, 0}};
@@ -356,7 +330,6 @@ __global__ void __launch_bounds__(544) k_solve(SolveArgs a) {
     }
     group_sync(tj);  // y complete and visible within the column group
 
-    SV_T(1);
     // ------------------------------------------------------------------ pass 2:  x = W^H y
     for (int i = 0; i < nblk; ++i) {
         double acc[3][2] = {{0, 0}, {0, 0}, {0, 0}};
@@ -385,7 +358,6 @@ __global__ void __launch_bounds__(544) k_solve(SolveArgs a) {
     }
     consumer_sync();  // both column groups done; the ring is idle from here on
 
-    SV_T(2);
     // ------------------------------------------------------------------ epilogue
     if (a.cg_compat) {
         // c = b^H x*, ||b||^2 in the reference's (unwhitened) variables:
@@ -445,19 +417,7 @@ __global__ void __launch_bounds__(544) k_solve(SolveArgs a) {
             if (cl == 0 && row < a.n) Pp[row] = p;
         }
     }
-    SV_T(3);
-#ifdef HP_SOLVE_TIMERS
-    if (tid == 0) for (int i = 0; i < 8; ++i) atomicAdd(&g_solve_cycles[i], (unsigned long long)tacc[i]);
-#endif
 }
-
-#ifdef HP_SOLVE_TIMERS
-extern "C" void hp_solve_timers(unsigned long long* out, int reset) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_solve_cycles, sizeof(unsigned long long) * 8);
-    if (reset) { unsigned long long z[8] = {0}; cudaMemcpyToSymbol(g_solve_cycles, z, sizeof(z)); }
-}
-#endif
 
 void launch_solve(const SolveArgs& a_in, cudaStream_t st) {
     SolveArgs a = a_in;

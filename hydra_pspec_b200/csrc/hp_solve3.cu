@@ -28,7 +28,6 @@
 #include "hp_mma.cuh"
 #include "hp_async.cuh"
 #include <algorithm>
-#include <cstdlib>
 #include <vector>
 
 namespace hp {
@@ -41,24 +40,17 @@ constexpr int kW3 = kS3Warps;                 // consumer warps (all warps of th
 constexpr int kS3Threads = 32 * kW3;
 constexpr int kRowDoubles3 = 2 * 32 * kTT;    // one block row of a tile: [plane][32 rows][16 columns, XOR-swizzled]
 constexpr int kFragDoubles = 128;             // one k-step of one strip in fragment-major order: 32 lanes x 4 doubles
-#ifndef HP_S3_L1_PREFETCH
-#define HP_S3_L1_PREFETCH 2                   // k-steps of L1 prefetch distance (0: loads bypass L1, no prefetch)
-#endif
+constexpr int kL1Prefetch = 2;                // k-steps of L1 prefetch distance
 
 __device__ __forceinline__ double4 ldg_frag(const double* p) {
     // streaming fragment ([row group][lane][re, im]: two 16-byte loads, each 512 contiguous bytes per warp); every byte is
     // used once per CTA, keep it out of L1.  Volatile asm: the load keeps its place between the (volatile) DMMAs, after the
     // first DMMA of a k-step has waited for the previous load -- one load group in flight per warp.
     double4 v;
-#if HP_S3_L1_PREFETCH > 0
-    // loads through L1: the group HP_S3_L1_PREFETCH k-steps ahead was requested into L1 by a prefetch (no destination
-    // register, hence no scoreboard): more fragment data in flight without the scoreboard aliasing.  5.27 -> 5.15 ms.
+    // loads through L1: the group kL1Prefetch k-steps ahead was requested into L1 by a prefetch (no destination register,
+    // hence no scoreboard): more fragment data in flight without the scoreboard aliasing.  5.27 -> 5.15 ms.
     asm volatile("ld.global.ca.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p));
     asm volatile("ld.global.ca.v2.f64 {%0, %1}, [%2];" : "=d"(v.z), "=d"(v.w) : "l"(p + 64));
-#else
-    asm volatile("ld.global.cg.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p));
-    asm volatile("ld.global.cg.v2.f64 {%0, %1}, [%2];" : "=d"(v.z), "=d"(v.w) : "l"(p + 64));
-#endif
     return v;
 }
 
@@ -137,12 +129,6 @@ void solve3_make_schedule(int nblk, Solve3Sched* sc, int nstrip) {
     }
 }
 
-// Phase timers (HP_S3_TIMERS=1; profiles/scripts/solve3_timers.py), clock64 deltas of lane 0 of every warp:
-//  [0] pass 1 strips  [1] Philox + y store  [2] barrier (y complete)  [3] pass 2 strips  [4] x store  [5] waiting for the
-//  y buffer  [6] waiting for right-hand sides  [7] whole loop
-__device__ unsigned long long g_solve3_cycles[8];
-
-template <bool kTimers>
 __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int nblk = a.nblk, Np = nblk * 32;
@@ -203,12 +189,10 @@ __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
         const double4 v = ldg_frag(pf_p);
         pf_p += kFragDoubles;
         --pf_left;
-#if HP_S3_L1_PREFETCH > 0
-        if (pf_left >= HP_S3_L1_PREFETCH) {   // the group HP_S3_L1_PREFETCH k-steps after the one just requested
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(pf_p + (HP_S3_L1_PREFETCH - 1) * kFragDoubles));
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(pf_p + (HP_S3_L1_PREFETCH - 1) * kFragDoubles + 64));
+        if (pf_left >= kL1Prefetch) {   // the group kL1Prefetch k-steps after the one just requested
+            asm volatile("prefetch.global.L1 [%0];" ::"l"(pf_p + (kL1Prefetch - 1) * kFragDoubles));
+            asm volatile("prefetch.global.L1 [%0];" ::"l"(pf_p + (kL1Prefetch - 1) * kFragDoubles + 64));
         }
-#endif
         return v;
     };
     // Exactly one fragment load is in flight per warp (issued before the DMMAs of the current k-step, consumed by the next):
@@ -216,18 +200,12 @@ __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
     // (profiles/r2_solve2_v1_notes.md); the L2 latency is hidden by the four warps of a scheduler instead.
     double4 acur = pf_next();
 
-    long long tacc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tlast = 0;
-    if (kTimers) tlast = clock64();
-#define S3_T(idx) do { if (kTimers) { const long long now_ = clock64(); tacc[idx] += now_ - tlast; tlast = now_; } } while (0)
-    const long long tloop0 = tlast;
-
     double P[3][2][2][2];
     uint32_t it = 0;
     for (int w = blockIdx.x; w < total; w += gridDim.x, ++it) {
         const int sys = w / a.ntiles, tile = w - sys * a.ntiles, t0 = tile * kTT;
         const uint32_t chain = a.philox ? (uint32_t)a.dk.chain_ids[sys] : 0u;
         mbar_wait(rhs_full, it & 1);
-        S3_T(6);
         // ------------------------------------------------------------------ pass 1:  y = W1 r (+ xi)
         for (int e = 0; e < n1; ++e) {
             const int s = a.sched.strip[0][warp][e];
@@ -251,8 +229,7 @@ __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
                 load_b(bf[0], tileR, (t + 2 < nk) ? t + 2 : 0, bo0, bo1);
                 mma_rest<false>(P, anx, bf[1]);
             }
-            S3_T(0);
-            if (e == 0 && it > 0) { mbar_wait(yfree, (it - 1) & 1); S3_T(5); }   // the previous tile's pass 2 is done with y
+            if (e == 0 && it > 0) mbar_wait(yfree, (it - 1) & 1);   // the previous tile's pass 2 is done with y
             // y = (P0 - P1) + i (P2 - P0 - P1) + xi  ->  tile Y
 #pragma unroll
             for (int wi = 0; wi < 2; ++wi) {
@@ -265,18 +242,10 @@ __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
                         const int col = 8 * wj + 2 * q + x;
                         double vr = P[0][wi][wj][x] - P[1][wi][wj][x];
                         double vi = P[2][wi][wj][x] - P[0][wi][wj][x] - P[1][wi][wj][x];
-#ifdef HP_S3_EXPERIMENT_NO_NOISE   // timing experiment only (wrong statistics): what the Philox draws cost
-                        if (false) {
-#else
                         if (a.philox && row < a.N && t0 + col < a.T) {
-#endif
                             u32x4 ctr; ctr.x = (uint32_t)row; ctr.y = (uint32_t)(t0 + col); ctr.z = a.dk.iter; ctr.w = chain;
                             double x0, x1;
-#ifdef HP_PHILOX_DOUBLE   // experiment (profiles/r2_summary.md): what full double-precision Box-Muller costs this kernel
-                            normal_pair(philox4x32_10(ctr, a.dk.key0, a.dk.key1 ^ 0xA5A5A5A5u), x0, x1);
-#else
                             normal_pair_fast(philox4x32_10(ctr, a.dk.key0, a.dk.key1 ^ 0xA5A5A5A5u), x0, x1);
-#endif
                             vr += x0 * 0.70710678118654752440; vi += x1 * 0.70710678118654752440;
                         }
                         const int c = col ^ ((rl & 3) << 2);
@@ -284,13 +253,9 @@ __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
                         trow[c + 32 * kTT] = vi;
                     }
             }
-            S3_T(1);
         }
         if (n1 == 0 && it > 0) mbar_wait(yfree, (it - 1) & 1);   // keep the phase bookkeeping of idle warps in step
-#ifndef HP_S3_EXPERIMENT_NO_BARRIER   // timing experiment only (wrong results): what the per-tile barrier costs
         consumer_sync3();   // y complete; r is dead
-#endif
-        S3_T(2);
         if (tid == 0 && w + (int)gridDim.x < total) {
             // the next tile's right-hand sides land while pass 2 runs
             mbar_arrive_expect_tx(rhs_full, tile_bytes);
@@ -320,7 +285,6 @@ __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
                 load_b(bf[0], tileY, (t + 2 < nk) ? k0 + t + 2 : 0, bo0, bo1);
                 mma_rest<true>(P, anx, bf[1]);
             }
-            S3_T(3);
             // x = (P0 + P1) + i (P2 - P0 + P1)   (conj(A) B)
 #pragma unroll
             for (int wi = 0; wi < 2; ++wi) {
@@ -340,48 +304,31 @@ __global__ void __launch_bounds__(kS3Threads, 1) k_solve3(Solve3Args a) {
                 psum += __shfl_xor_sync(0xffffffffu, psum, 2);
                 if (q == 0 && row < a.n) Pp[row] = psum;
             }
-            S3_T(4);
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(yfree);
     }
-    if (kTimers) {
-        tacc[7] = clock64() - tloop0;
-        if (lane == 0)
-            for (int i = 0; i < 8; ++i) atomicAdd(&g_solve3_cycles[i], (unsigned long long)tacc[i]);
-    }
-#undef S3_T
-}
-
-extern "C" void hp_solve3_timers(unsigned long long* out, int reset) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_solve3_cycles, sizeof(unsigned long long) * 8);
-    if (reset) { unsigned long long z[8] = {0}; cudaMemcpyToSymbol(g_solve3_cycles, z, sizeof(z)); }
 }
 
 void launch_solve3(const Solve3Args& a_in, cudaStream_t st) {
     Solve3Args a = a_in;
-    static int num_sm = 0, timers = -1;
+    static int num_sm = 0;
     if (!num_sm) {
         int dev = 0;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&num_sm, cudaDevAttrMultiProcessorCount, dev);
-        const char* ev = getenv("HP_S3_TIMERS");
-        timers = (ev && ev[0] == '1') ? 1 : 0;
     }
     const size_t smem = solve3_smem_bytes(a.nblk);
     static size_t attr_dev[kMaxDev] = {0};
     size_t& attr_smem = attr_dev[current_device_slot()];
     if (smem > attr_smem) {
-        cudaFuncSetAttribute(k_solve3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaFuncSetAttribute(k_solve3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(k_solve3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         attr_smem = smem;
     }
     const int total = a.ntiles * a.nsys;
     int grid = a.grid_limit > 0 ? a.grid_limit : num_sm;
     if (grid > total) grid = total;
-    if (timers) k_solve3<true><<<grid, kS3Threads, smem, st>>>(a);
-    else k_solve3<false><<<grid, kS3Threads, smem, st>>>(a);
+    k_solve3<<<grid, kS3Threads, smem, st>>>(a);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

@@ -65,11 +65,12 @@ typedef struct hp_config {
     int force_dense_transforms; /* 1: apply the Fourier operator as dense products even when Nfreqs has
                             an FFT plan (the path used for Nfreqs with a prime factor > 31); tests */
     int force_dense_solve; /* 1: run the GCR solve as dense products with W = L^-1 even when the shared-memory
-                            resident k_solve tile fits (the path Nfreqs + Nmodes > 576 takes in any case); tests */
+                            resident k_solve tile fits (the path Nfreqs + Nmodes > 576 takes in any case); with
+                            time_flags = 1: one factorisation per time (csrc/hp_pertime.cu) instead of the
+                            low-rank form; tests */
     int time_flags;      /* 1: flags are per time, [Ntimes][Nfreqs] (an extension: the reference collapses them to
-                            "flagged at any time", run-hydra-pspec.py:520-526).  Every (baseline, time) pair is then
-                            factored and solved on its own (csrc/hp_pertime.cu).  Needs a delay-diagonal S_initial,
-                            diagonal noise, cg_compat = 0 */
+                            "flagged at any time", run-hydra-pspec.py:520-526).  hp_engine_pt_form reports which
+                            form of the per-time solve runs.  Needs diagonal noise, cg_compat = 0 */
     int ring_iters;      /* device slots of the big per-iteration outputs (signal_cr, fg_amps, chisq): 0 = max_iters
                             (every iteration stays readable with hp_engine_read); R > 0: a ring of R slots, iteration i
                             lives in slot i % R until iteration i + R overwrites it.  hp_engine_run_to_host streams
@@ -210,7 +211,7 @@ int hp_engine_set_profile(hp_engine* e, int on);
 /* Per-time flags (cfg.time_flags): which form of the per-time solve the engine runs for the chains loaded so far.
  *   *low_rank = 1: one shared factorisation per chain + a rank-k_t correction per time (csrc/hp_ptlow.cu); 0: one
  *   factorisation per (chain, time) (csrc/hp_pertime.cu: a time has more than 64 channels flagged beyond the chain's
- *   all-times mask, Nfreqs + Nmodes > 448, or HP_PT_DIRECT=1).  *max_rank = largest k_t of the loaded chains.
+ *   all-times mask, Nfreqs + Nmodes > 448, or cfg.force_dense_solve).  *max_rank = largest k_t of the loaded chains.
  * Replaces nothing in the reference (it has no per-time flags, pspec.py:428); either pointer may be NULL. */
 int hp_engine_pt_form(const hp_engine* e, int* low_rank, int* max_rank);
 /* Total kernel launches issued by hp_engine_run / hp_engine_gcr so far. */

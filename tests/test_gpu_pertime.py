@@ -51,11 +51,10 @@ def make_case(nt, nf, nm, frac, seed):
 @pytest.fixture(params=["lowrank", "direct"])
 def pt_form(request, monkeypatch):
     """Both forms of the per-time solve: the low-rank correction of one shared factorisation (hp_ptlow.cu, default) and
-    one factorisation per time (hp_pertime.cu: HP_PT_DIRECT=1, read at engine creation)."""
+    one factorisation per time (hp_pertime.cu: the engine's force_dense_solve field)."""
+    from hydra_pspec_b200 import pspec
     if request.param == "direct":
-        monkeypatch.setenv("HP_PT_DIRECT", "1")
-    else:
-        monkeypatch.delenv("HP_PT_DIRECT", raising=False)
+        monkeypatch.setattr(pspec, "_FORCE_DENSE_SOLVE", True)
     return request.param
 
 
@@ -146,9 +145,9 @@ def test_per_time_unsupported_combinations_raise():
 @pytest.mark.parametrize("nt,nf,nm,frac,seed", [(7, 32, 4, 0.1, 81), (9, 96, 8, 0.15, 82), (5, 128, 0, 0.2, 83)])
 def test_per_time_flags_with_general_S_initial(nt, nf, nm, frac, seed, monkeypatch):
     """A non-delay-diagonal S_initial (first iteration in its eigenbasis) together with per-time flags: taken by the low-rank
-    form (any first basis; hp_ptlow.cu), refused by the direct form (k_pt_cholsolve relies on the circulant signal block)."""
+    form (any first basis; hp_ptlow.cu), refused by the direct form (force_dense_solve; k_pt_cholsolve relies on the
+    circulant signal block)."""
     from hydra_pspec_b200 import pspec, _lib
-    monkeypatch.delenv("HP_PT_DIRECT", raising=False)
     vis, flags, S0, F, Ninv, prior = make_case(nt, nf, nm, frac, seed)
     rng = np.random.default_rng(seed)
     G = crandn(rng, nf, nf)
@@ -157,7 +156,7 @@ def test_per_time_flags_with_general_S_initial(nt, nf, nm, frac, seed, monkeypat
     out = pspec.gibbs_sample_with_fg(vis, flags, Sg, F, Ninv, prior, Niter=3, seed=5, verbose=False)
     for o, r, k in zip(out[:6], ref, KEYS):
         assert rel(o, r) < (1e-8 if k == "chisq" else 5e-10), k
-    monkeypatch.setenv("HP_PT_DIRECT", "1")
+    monkeypatch.setattr(pspec, "_FORCE_DENSE_SOLVE", True)
     with pytest.raises(_lib.HydraLibError):
         pspec.gibbs_sample_with_fg(vis, flags, Sg, F, Ninv, prior, Niter=1, seed=5, verbose=False)
 
@@ -221,25 +220,19 @@ def test_per_time_rank_limit_selects_the_form(frac, expect_lowrank):
         assert rel(o, r) < (1e-8 if k == "chisq" else TOL), k
 
 
-def test_per_time_forms_agree_at_config2_shape():
+def test_per_time_forms_agree_at_config2_shape(monkeypatch):
     """BASELINE.json configs[2] shape (Nfreq=256, Nfg=16, 5 % per-time flags on top of a 5 % all-times mask), 64 times, four
-    chains in one engine: low-rank form == one factorisation per time to round-off (injected draws, two iterations)."""
-    import os
+    chains in one engine: low-rank form == one factorisation per time (force_dense_solve) to round-off (injected draws, two
+    iterations)."""
     from hydra_pspec_b200 import pspec
     bls = []
     for c in range(4):
         vis, flags, S0, F, Ninv, prior = make_case(64, 256, 16, 0.05, 70 + c)
         flags[:, np.random.default_rng(c).choice(256, 12, replace=False)] = False
         bls.append(dict(vis=vis, flags=flags, S_initial=S0, fgmodes=F, Ninv=Ninv, ps_prior=prior))
-    old = os.environ.pop("HP_PT_DIRECT", None)
-    try:
-        low = pspec.gibbs_sample_batch(bls, Niter=2, seed=5, rng="numpy", solver="exact")
-        os.environ["HP_PT_DIRECT"] = "1"
-        direct = pspec.gibbs_sample_batch(bls, Niter=2, seed=5, rng="numpy", solver="exact")
-    finally:
-        os.environ.pop("HP_PT_DIRECT", None)
-        if old is not None:
-            os.environ["HP_PT_DIRECT"] = old
+    low = pspec.gibbs_sample_batch(bls, Niter=2, seed=5, rng="numpy", solver="exact")
+    monkeypatch.setattr(pspec, "_FORCE_DENSE_SOLVE", True)
+    direct = pspec.gibbs_sample_batch(bls, Niter=2, seed=5, rng="numpy", solver="exact")
     for a, b in zip(low, direct):
         for x, y, k in zip(a[:6], b[:6], KEYS):
             assert rel(x, y) < (1e-8 if k == "chisq" else TOL), k

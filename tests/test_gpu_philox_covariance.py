@@ -41,14 +41,8 @@ def nrm(C, Sigma):
 
 
 @pytest.mark.parametrize("variant", ["solve3", "dense_solve", "time_flags", "time_flags_direct"])
-def test_philox_gcr_covariance_multiblock(variant, monkeypatch):
+def test_philox_gcr_covariance_multiblock(variant):
     from hydra_pspec_b200 import pspec
-    # per-time flags: the low-rank form (k_solve3 + k_pt_lowrank with its own zeta draws; default) and one factorisation
-    # per time (k_pt_cholsolve)
-    if variant == "time_flags_direct":
-        monkeypatch.setenv("HP_PT_DIRECT", "1")
-    else:
-        monkeypatch.delenv("HP_PT_DIRECT", raising=False)
     nt, nf, nm, nch, ndraw = 48, 96, 8, 4, 4000          # N = 104: 4 block rows; 3 time tiles; 4 chains
     rng = np.random.default_rng(2024)
     F = np.linalg.qr(crandn(rng, nf, nm))[0]
@@ -65,8 +59,10 @@ def test_philox_gcr_covariance_multiblock(variant, monkeypatch):
         masks = np.ones((1, nf), dtype=bool)
         masks[0, [5, 40, 41, 77]] = False
         flags = masks[0]
+    # per-time flags: the low-rank form (k_solve3 + k_pt_lowrank with its own zeta draws; default) and, with
+    # force_dense_solve, one factorisation per time (k_pt_cholsolve)
     eng = pspec.GibbsEngine(nch, nt, nf, nm, max_iters=1, rng="philox", refresh_omega=True, keep=(), seed=99,
-                            time_flags=per_time, force_dense_solve=(variant == "dense_solve"))
+                            time_flags=per_time, force_dense_solve=variant in ("dense_solve", "time_flags_direct"))
     for c in range(nch):
         eng.load_chain(c, vis[c] * flags, flags, F, ninv_diag, ps / nf)
     post = [posterior(ps, mk, F, ninv_diag) for mk in masks]

@@ -80,7 +80,7 @@ CASES = {
     "dense_solve": dict(force_dense_solve=True),
     "dense_noise": dict(dense=True),
     "per_time_lowrank": dict(per_time=True),
-    "per_time_direct": dict(per_time=True),
+    "per_time_direct": dict(per_time=True, force_dense_solve=True),
     "general_basis0": dict(general=True),
     "no_fg_modes": dict(m=0),
     "odd_rows_prime_nfreqs": dict(T=41, n=37, m=3),   # odd T n and T m (padded accumulator rows); no FFT plan for 37
@@ -88,10 +88,8 @@ CASES = {
 
 
 @pytest.mark.parametrize("case", list(CASES))
-def test_moments_match_samples(case, monkeypatch):
+def test_moments_match_samples(case):
     """5 chains in 2 sub-batches, 13 iterations, burn_in 3, thin 2: the moments are those of samples [3::2]."""
-    if case == "per_time_direct":
-        monkeypatch.setenv("HP_PT_DIRECT", "1")
     eng = make_engine(**CASES[case])
     try:
         if case.startswith("per_time"):

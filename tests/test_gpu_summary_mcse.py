@@ -39,11 +39,9 @@ def check_against(got, key, samples, b):
 
 
 @pytest.mark.parametrize("case", list(CASES))
-def test_mcse_matches_numpy(case, monkeypatch):
+def test_mcse_matches_numpy(case):
     """5 chains in 2 sub-batches, 40 iterations, burn_in 3, thin 2, batch 4: k = 19 samples [3::2], 4 complete batches and
     a partial batch of 3."""
-    if case == "per_time_direct":
-        monkeypatch.setenv("HP_PT_DIRECT", "1")
     eng = make_engine(niter=40, **CASES[case])
     try:
         eng.set_summary(("cr", "fg"), burn_in=3, thin=2, batch=4)
