@@ -45,6 +45,7 @@ _SIGNATURES = {
     "hp_engine_load_chain": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p]),
     "hp_engine_load_chain_dense": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 9),
+    "hp_engine_load_chain_time_noise": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 7),
     "hp_engine_set_draws": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "hp_engine_run": (C.c_int, [C.c_void_p, C.c_int]),
     "hp_engine_run_to_host": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(HPHostSink)]),

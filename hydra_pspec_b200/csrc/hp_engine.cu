@@ -62,6 +62,33 @@ __global__ void k_rowscale(double* out, const double* W, const double* v, int ro
     if (e >= (long long)rows * n) return;
     out[e] = W[e] * v[e % n];
 }
+// out[e] = W[e] * V[e]: per-time flags times per-time noise weights
+__global__ void k_mul_elem(double* out, const double* W, const double* V, long long count) {
+    long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (e >= count) return;
+    out[e] = W[e] * V[e];
+}
+// A[e] *= W[e] sqrt(V[e])  (A complex): the injected noise draw of per-time noise, (w_t N_t^-1)^1/2 omega_b
+__global__ void k_mask_sqrt_elem(double* A, const double* W, const double* V, long long count) {
+    long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (e >= count) return;
+    const double s = W[e] * sqrt(V[e]);
+    A[2 * e] *= s;
+    A[2 * e + 1] *= s;
+}
+// D[e] = A[e] * V[e]  (A, D complex, V real)
+__global__ void k_scale_elem(double* D, const double* A, const double* V, long long count) {
+    long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (e >= count) return;
+    D[2 * e] = A[2 * e] * V[e];
+    D[2 * e + 1] = A[2 * e + 1] * V[e];
+}
+// out[t][x] = v[x] for t < T: the per-time noise rows of a chain loaded with one diagonal
+__global__ void k_bcast_rows(double* out, const double* v, int T, int n) {
+    long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (e >= (long long)T * n) return;
+    out[e] = v[e % n];
+}
 // Bsel[x][0] = Bmat[x][0],  Bsel[x][1 + j] = Bmat[x][n + j]
 __global__ void k_select_cols(double* Bsel, const double* Bmat, int n, int m, int Np) {
     long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
@@ -254,7 +281,14 @@ struct hp_engine {
     double *wd = nullptr, *w = nullptr, *ninvd = nullptr, *ni = nullptr, *nu = nullptr, *Ft = nullptr, *prior = nullptr;
     double *Lp = nullptr, *Linvp = nullptr, *Wp = nullptr;
     double *wT = nullptr, *Hpt = nullptr, *niT = nullptr, *Bsel = nullptr, *ptScratch = nullptr;  // per-time flags
-    int* ptSame = nullptr;   // [C][Tp]: flags of time t equal those of t - 1
+    int* ptSame = nullptr;   // [C][Tp]: flags (and per-time noise weights) of time t equal those of t - 1
+    // per-time noise (hp_engine_load_chain_time_noise): diag(N_t^-1) of every chain and time, [C][Tp0][n], its own allocation
+    // made when the first such chain is loaded (the arena of an engine that never sees one does not grow).  Once it exists,
+    // the rows of every chain are kept current (a chain loaded with one diagonal gets it broadcast over its times), so that
+    // the post-processing can read the chi^2 / ln-posterior weights of a sub-batch with one stride
+    double* ninvT = nullptr;
+    std::vector<uint8_t> tn_loaded;   // per chain: loaded with per-time noise
+    bool any_tn() const { for (auto v : tn_loaded) if (v) return true; return false; }
     int pt_ctas = 0;
     Solve solve = Solve::Solve3;
     Post post = Post::Fft2;
@@ -482,6 +516,7 @@ int hp_engine_destroy(hp_engine* e) {
     arena_release(e->arena, e->arena_bytes, e->cfg.device);
     for (double* p : {e->sum.cr_mean, e->sum.cr_m2, e->sum.fg_mean, e->sum.fg_m2, e->sum.cr_snap, e->sum.cr_m2bm, e->sum.fg_snap,
                       e->sum.fg_m2bm}) if (p) cudaFree(p);
+    if (e->ninvT) cudaFree(e->ninvT);
     if (e->copy_st) cudaStreamDestroy(e->copy_st);
     for (auto x : e->sub_st) cudaStreamDestroy(x);
     if (e->fork_ev) cudaEventDestroy(e->fork_ev);
@@ -588,6 +623,7 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
     e->pt_kmax.assign(C, 0);
     e->hpt_built.assign(C, 0);
     e->pt_loaded.assign(C, 0);
+    e->tn_loaded.assign(C, 0);
     e->pending.assign(C, 0);
     {
         int ns = cfg->substreams > 1 ? (cfg->substreams < (int)C ? cfg->substreams : (int)C) : 1;
@@ -619,11 +655,16 @@ int hp_engine_create(const hp_config* cfg, hp_engine** out) {
 
 // Per-time flags, one factorisation per time (hp_pertime.cu): H_t = [Q|F]^H (w_t N^-1) [q_0 | F] for every time of chain c --
 // column 0 is the generator chat_t of the circulant signal block, the rest are the foreground columns of G_t.  Built from what
-// load_chain left on the device (Bmat, wT, ninvd), so it can be deferred until the direct form is actually needed.
+// load_chain left on the device (Bmat, wT, ninvd or, with per-time noise, ninvT: w_t N_t^-1), so it can be deferred until
+// the direct form is actually needed.
 static int build_hpt(hp_engine* e, int c) {
     const int n = e->n, m = e->m, N = e->N, Np = e->Np, T = e->T;
     const double* Bm = e->bF.Bmat + 2 * (size_t)c * n * Np;
-    k_rowscale<<<nblocks((long long)T * n), 256, 0, e->st>>>(e->niT, e->wT + (size_t)c * e->Tp * n, e->ninvd + (size_t)c * n, T, n);
+    if (e->tn_loaded[c])
+        k_mul_elem<<<nblocks((long long)T * n), 256, 0, e->st>>>(e->niT, e->wT + (size_t)c * e->Tp * n, e->ninvT + (size_t)c * e->Tp0 * n,
+                                                                 (long long)T * n);
+    else
+        k_rowscale<<<nblocks((long long)T * n), 256, 0, e->st>>>(e->niT, e->wT + (size_t)c * e->Tp * n, e->ninvd + (size_t)c * n, T, n);
     k_select_cols<<<nblocks((long long)n * (1 + m)), 256, 0, e->st>>>(e->Bsel, Bm, n, m, Np);
     hp::ZgemmArgs h{};
     h.A = Bm; h.sAi = 1; h.sAk = Np; h.bsA = 0; h.conjA = 1;
@@ -673,6 +714,12 @@ static int build_basis_products(hp_engine* e, Basis& b, int c) {
         y.M = T; y.N = n; y.K = n; y.alpha = 1.0; y.batch = 1;
         hp::launch_zgemm(y, e->st);
         r.A = e->Yd + 2 * (size_t)c * e->Tp * n; r.sAi = n; r.sAk = 1;
+    } else if (e->cfg.time_flags && e->tn_loaded[c]) {
+        // per-time noise: (w_t N_t^-1)(w_t d_t) = N_t^-1 (w_t d_t) element by element, staged (wd stays the masked data: the
+        // residual of the post-processing reads it)
+        k_scale_elem<<<nblocks((long long)T * n), 256, 0, e->st>>>(e->stage, e->wd + 2 * (size_t)c * e->Tp * n,
+                                                                   e->ninvT + (size_t)c * e->Tp0 * n, (long long)T * n);
+        r.A = e->stage; r.sAi = n; r.sAk = 1; r.conjA = 0;
     } else {
         r.A = e->wd + 2 * (size_t)c * e->Tp * n; r.sAi = n; r.sAk = 1; r.conjA = 0;
         // wd is already masked and w^2 = w: per-time flags use the unmasked diagonal
@@ -743,9 +790,11 @@ static int flush_pending(hp_engine* e) {
     return HP_OK;
 }
 
+// ninv_t: per-time noise, [T][n] (hp_engine_load_chain_time_noise), or null; ninv_diag is then its per-channel maximum over
+// the times, which nothing reads while the chain carries per-time noise
 static int load_chain_impl(hp_engine* e, int c, const double* vis, const uint8_t* flags, const double* fgmodes,
                            const double* ninv_diag, const double* ninv_dense, const double* nih_dense, const double* basis0,
-                           const double* lam0sq, const double* ps_prior) {
+                           const double* lam0sq, const double* ps_prior, const double* ninv_t = nullptr) {
     if (!e || !vis || !flags || !ninv_diag || !lam0sq || (e->m > 0 && !fgmodes))
         return fail(HP_ERR_ARG, "hp_engine_load_chain: null argument");
     if ((e->cfg.dense_noise != 0) != (ninv_dense != nullptr))
@@ -757,6 +806,18 @@ static int load_chain_impl(hp_engine* e, int c, const double* vis, const uint8_t
     const int n = e->n, m = e->m, N = e->N, Np = e->Np, T = e->T, Tp = e->Tp;
     cudaStream_t st = e->st;
     const bool pt = e->cfg.time_flags != 0;   // flags: [Ntimes][Nfreqs]
+    if (pt && (ninv_t || e->ninvT)) {
+        // per-time noise: the weights of every chain and time live in ninvT from the first such chain on
+        if (!e->ninvT) {
+            CU_TRY(dalloc(&e->ninvT, (size_t)e->C * e->Tp0 * n));
+            CU_TRY(cudaStreamSynchronize(0));   // dalloc zeroes on the legacy stream, which the engine's streams do not wait for
+            for (int c2 = 0; c2 < e->C; ++c2)   // chains loaded before with one diagonal: broadcast it over their times
+                if (c2 != c && e->pt_loaded[c2])
+                    k_bcast_rows<<<nblocks((long long)T * n), 256, 0, st>>>(e->ninvT + (size_t)c2 * e->Tp0 * n, e->ninvd + (size_t)c2 * n, T, n);
+        }
+        if (ninv_t) CU_TRY(cudaMemcpyAsync(e->ninvT + (size_t)c * e->Tp0 * n, ninv_t, (size_t)T * n * sizeof(double), cudaMemcpyHostToDevice, st));
+    }
+    e->tn_loaded[c] = ninv_t ? 1 : 0;
     std::vector<double> wv(n);
     std::vector<double> wtv(pt ? (size_t)T * n : 0);
     bool anyf = false;
@@ -781,7 +842,10 @@ static int load_chain_impl(hp_engine* e, int c, const double* vis, const uint8_t
     if (pt) {
         CU_TRY(cudaMemcpyAsync(e->wT + (size_t)c * Tp * n, wtv.data(), (size_t)T * n * sizeof(double), cudaMemcpyHostToDevice, st));
         std::vector<int> same(Tp, 0);
-        for (int t = 1; t < T; ++t) same[t] = std::memcmp(flags + (size_t)t * n, flags + (size_t)(t - 1) * n, n) == 0 ? 1 : 0;
+        // k_pt_cholsolve re-uses the factor of t - 1 when M_t is the same: equal flags and, with per-time noise, equal weights
+        for (int t = 1; t < T; ++t)
+            same[t] = std::memcmp(flags + (size_t)t * n, flags + (size_t)(t - 1) * n, n) == 0 &&
+                      (!ninv_t || std::memcmp(ninv_t + (size_t)t * n, ninv_t + (size_t)(t - 1) * n, n * sizeof(double)) == 0) ? 1 : 0;
         CU_TRY(cudaMemcpyAsync(e->ptSame + (size_t)c * Tp, same.data(), (size_t)Tp * sizeof(int), cudaMemcpyHostToDevice, st));
         if (e->lowrank_rows()) {
             // channels flagged at time t beyond the all-times mask
@@ -804,8 +868,9 @@ static int load_chain_impl(hp_engine* e, int c, const double* vis, const uint8_t
             CU_TRY(cudaMemcpyAsync(e->ptFcnt + (size_t)c * T, fcnt.data(), (size_t)T * sizeof(int), cudaMemcpyHostToDevice, st));
             e->pt_kcap = 0;
             for (int v : e->pt_kmax) if (v > e->pt_kcap) e->pt_kcap = v;
-            // a time with more extra flags than the low-rank kernel takes: the whole engine uses k_pt_cholsolve
-            e->solve = e->pt_kcap <= hp::kPtLowMaxRank ? Solve::PtLowRank : Solve::PtDirect;
+            // a time with more extra flags than the low-rank kernel takes, or a chain with per-time noise: the whole engine uses
+            // k_pt_cholsolve
+            e->solve = (e->pt_kcap <= hp::kPtLowMaxRank && !e->any_tn()) ? Solve::PtLowRank : Solve::PtDirect;
             if (e->solve == Solve::PtDirect && e->cfg.general_basis0)
                 return fail(HP_ERR_SIZE, "per-time flags with a general S_initial: a time has more than 64 channels flagged beyond the "
                                          "all-times mask (only the low-rank form of the per-time solve takes a general first basis)");
@@ -817,6 +882,8 @@ static int load_chain_impl(hp_engine* e, int c, const double* vis, const uint8_t
     else k_mask_cols<<<nblocks((long long)T * n), 256, 0, st>>>(wd, e->w + (size_t)c * n, T, n);
     k_noise_vectors<<<nblocks(n), 256, 0, st>>>(e->w + (size_t)c * n, e->ninvd + (size_t)c * n, e->ni + (size_t)c * n,
                                                e->nu + (size_t)c * n, n);
+    if (pt && e->ninvT && !ninv_t)
+        k_bcast_rows<<<nblocks((long long)T * n), 256, 0, st>>>(e->ninvT + (size_t)c * e->Tp0 * n, e->ninvd + (size_t)c * n, T, n);
     if (ps_prior) CU_TRY(cudaMemcpyAsync(e->prior + (size_t)c * 2 * n, ps_prior, 2 * n * sizeof(double), cudaMemcpyHostToDevice, st));
     else CU_TRY(cudaMemsetAsync(e->prior + (size_t)c * 2 * n, 0, 2 * n * sizeof(double), st));
     if (ninv_dense) {
@@ -867,6 +934,26 @@ int hp_engine_load_chain(hp_engine* e, int c, const double* vis, const uint8_t* 
     return load_chain_impl(e, c, vis, flags, fgmodes, ninv_diag, nullptr, nullptr, basis0, lam0sq, ps_prior);
 }
 
+int hp_engine_load_chain_time_noise(hp_engine* e, int c, const double* vis, const uint8_t* flags, const double* fgmodes,
+                                    const double* ninv_t, const double* basis0, const double* lam0sq, const double* ps_prior) {
+    if (!e || !ninv_t) return fail(HP_ERR_ARG, "hp_engine_load_chain_time_noise: null argument");
+    if (!e->cfg.time_flags || e->cfg.dense_noise)
+        return fail(HP_ERR_ARG, "hp_engine_load_chain_time_noise: needs an engine created with cfg.time_flags = 1 and diagonal noise");
+    const int n = e->n, T = e->T;
+    std::vector<double> env(n, 0.0);   // per-channel maximum over the times (ninv_diag of load_chain_impl)
+    for (int t = 0; t < T; ++t)
+        for (int x = 0; x < n; ++x) {
+            const double v = ninv_t[(size_t)t * n + x];
+            if (!std::isfinite(v) || !(v >= 0.0))
+                return fail(HP_ERR_ARG, "hp_engine_load_chain_time_noise: ninv_t must be finite and >= 0");
+            if (v > env[x]) env[x] = v;
+        }
+    if (e->cfg.general_basis0)
+        return fail(HP_ERR_SIZE, "per-time noise with a general S_initial: per-time noise runs one factorisation per time, which "
+                                 "takes a delay-diagonal S_initial only");
+    return load_chain_impl(e, c, vis, flags, fgmodes, env.data(), nullptr, nullptr, basis0, lam0sq, ps_prior, ninv_t);
+}
+
 int hp_engine_load_chain_dense(hp_engine* e, int c, const double* vis, const uint8_t* flags, const double* fgmodes,
                                const double* ninv_diag, const double* ninv_dense, const double* nih_dense,
                                const double* basis0, const double* lam0sq, const double* ps_prior) {
@@ -907,6 +994,10 @@ int hp_engine_set_draws(hp_engine* e, int c, const double* omega_a, const double
                 y.M = T; y.N = n; y.K = n; y.alpha = 1.0; y.batch = 1;
                 hp::launch_zgemm(y, st);
                 r.A = e->Yd + 2 * (size_t)c * Tp * n;
+            } else if (e->cfg.time_flags && e->tn_loaded[c]) {
+                // per-time noise: (w_t N_t^-1)^1/2 omega_b, element by element
+                k_mask_sqrt_elem<<<nblocks((long long)T * n), 256, 0, st>>>(e->stage, e->wT + (size_t)c * Tp * n,
+                                                                            e->ninvT + (size_t)c * e->Tp0 * n, (long long)T * n);
             } else if (e->cfg.time_flags) {
                 // N_t^-1/2 omega_b = sqrt(N^-1) (w_t omega_b)
                 k_mask_elem<<<nblocks((long long)T * n), 256, 0, st>>>(e->stage, e->wT + (size_t)c * Tp * n, (long long)T * n);
@@ -1205,6 +1296,8 @@ static void enqueue_post(hp_engine* e, Basis& b, const IterOut& o, const Sub& sb
         pa.Ft = OFFS(e->Ft, 2 * (m ? m : 1) * n); pa.wd = OFFS(e->wd, 2 * Tp * n); pa.w = OFFS(e->w, n); pa.ninvd = OFFS(e->ninvd, n);
         pa.w_bs = e->n; pa.w_ts = 0;
         if (e->cfg.time_flags) { pa.w = OFFS(e->wT, Tp * n); pa.w_bs = (long long)e->Tp * e->n; pa.w_ts = e->n; }
+        pa.ninv_bs = e->n; pa.ninv_ts = 0;
+        if (e->any_tn()) { pa.ninvd = OFFS(e->ninvT, (size_t)e->Tp0 * n); pa.ninv_bs = (long long)e->Tp0 * e->n; pa.ninv_ts = e->n; }
         pa.fg_out = fg; pa.fg_bs = o.fg_bs; pa.chisq_out = chisq; pa.chisq_bs = o.chisq_bs;
         pa.lnp1 = OFFS(e->lnp1, Tp); pa.Rm = e->cfg.dense_noise ? OFFS(e->Rm, 2 * Tp * n) : nullptr;
         pa.Empart = e->any_flagged ? OFFS(e->Empart, (size_t)e->ntilesE * n) : nullptr;

@@ -185,7 +185,7 @@ __global__ void __launch_bounds__(32 * kTP, kTP == 8 ? 2 : 1) k_post_fft(PostFft
     const double* X = a.X + 2 * ((size_t)sys * a.Tp + t0) * a.Np;
     const double* lam = a.lam + (size_t)sys * a.Np;
     const double* w = a.w + (size_t)sys * a.w_bs + (size_t)t0 * a.w_ts;
-    const double* nd = a.ninvd + (size_t)sys * n;
+    const double* nd = a.ninvd + (size_t)sys * a.ninv_bs + (size_t)t0 * a.ninv_ts;
     double* Sf = a.Sf + 2 * ((size_t)sys * a.sf_bs + (size_t)t0 * n);
     const double2* twg = reinterpret_cast<const double2*>(a.tw);
     const double rsn = rsqrt((double)n);
@@ -321,17 +321,17 @@ __global__ void __launch_bounds__(32 * kTP, kTP == 8 ? 2 : 1) k_post_fft(PostFft
             // all global loads of this channel first: the optional global stores below (chi^2, masked residual) would
             // otherwise keep the compiler from moving the next time's load above them (one exposed latency per time)
             double2 dv[kTP];
-            double wv[kTP];
+            double wv[kTP], nv[kTP];
 #pragma unroll
             for (int t = 0; t < kTP; ++t) {
                 dv[t] = make_double2(0.0, 0.0);
                 if (t0 + t < a.T) dv[t] = *reinterpret_cast<const double2*>(wd + 2 * ((size_t)t * n + x));
                 wv[t] = (a.w_ts == 0 || t0 + t < a.T) ? w[(size_t)t * a.w_ts + x] : 0.0;
+                nv[t] = (a.ninv_ts == 0 || t0 + t < a.T) ? nd[(size_t)t * a.ninv_ts + x] : 0.0;
             }
-            const double ndx = nd[x];
 #pragma unroll
             for (int t = 0; t < kTP; ++t) {
-                const double wx = wv[t];
+                const double wx = wv[t], ndx = nv[t];
                 double2 s = sbuf[(size_t)t * n + x];
                 double2 mf = obuf[(size_t)t * n + x];
                 const double2 d = dv[t];

@@ -193,7 +193,6 @@ __global__ void __launch_bounds__(32 * kTP2, (E >= 16 ? 1 : kFft2Ctas)) k_post_f
     const double* X = a.X + 2 * ((size_t)sys * a.Tp + t0) * a.Np;
     const double* lam = a.lam + (size_t)sys * a.Np;
     const double* w = a.w + (size_t)sys * a.w_bs + (size_t)t0 * a.w_ts;
-    const double* nd = a.ninvd + (size_t)sys * n;
     const double* wd = a.wd + 2 * ((size_t)sys * a.Tp + t0) * n;
     double* Sf = a.Sf + 2 * ((size_t)sys * a.sf_bs + (size_t)t0 * n);
     const double2* twg = reinterpret_cast<const double2*>(a.tw);
@@ -266,6 +265,7 @@ __global__ void __launch_bounds__(32 * kTP2, (E >= 16 ? 1 : kFft2Ctas)) k_post_f
         const int g = lane >> 2, q = lane & 3;
         const bool tlive = t0 + g < a.T;
         const double* wrow = w + (size_t)g * a.w_ts;
+        const double* nd = a.ninvd + (size_t)sys * a.ninv_bs + (size_t)(t0 + g) * a.ninv_ts;   // this lane's time
         double lnp = 0.0;
         // One group of global loads in flight per warp: the B fragments of all k-steps (mk <= 32: eight; more modes: the
         // first eight, the rest on demand) and the data of the NEXT tile are requested before this tile's products.

@@ -232,6 +232,8 @@ struct PostFftArgs {
     const double* Ft;      // [nsys][m][n]
     const double* wd; const double* w; const double* ninvd;
     long long w_bs, w_ts;  // w[sys * w_bs + t * w_ts + x]: (n, 0) time-invariant flags, (Tp n, n) per-time flags
+    long long ninv_bs, ninv_ts;  // chi^2 / ln-posterior weight ninvd[sys * ninv_bs + t * ninv_ts + x]: (n, 0) one diagonal
+                                 //   per chain, (Tp0 n, n) per-time noise
     double* fg_out; double* chisq_out; long long fg_bs, chisq_bs;
     double* lnp1;          // [nsys][Tp]
     double* Rm;            // [nsys][Tp][n] complex or null: w * resid (dense noise: ln_post term via k_zgemm2)

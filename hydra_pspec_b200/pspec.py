@@ -223,6 +223,48 @@ def _noise_model(Ninv, flags, nfreqs, need_sqrt):
     return d, dense, nih
 
 
+def _time_noise_model(Ninv, flags, ntimes, nfreqs):
+    """Per-time inverse noise covariance ``Ninv`` of shape ``(Ntimes, Nfreqs, Nfreqs)`` (an extension: the reference's
+    build_matrices takes one matrix, pspec.py:361).  Returns ``(Ninv, flags, ninv_t)``:
+
+    - ``Ninv`` 2-D: unchanged, ``ninv_t = None``;
+    - all slices identical: ``Ninv[0]`` and ``ninv_t = None`` -- the chain is exactly the one of the 2-D matrix;
+    - all slices diagonal: ``Ninv = None``, the flags as ``(Ntimes, Nfreqs)`` (1-D flags are broadcast) and ``ninv_t``, the
+      ``(Ntimes, Nfreqs)`` diagonals: time t uses ``Ninv[t]`` in its GCR system and as its chi^2 / ln-posterior weight,
+      one factorisation per time on the device (csrc/hp_pertime.cu).
+
+    A non-diagonal slice raises ``NotImplementedError`` (a dense rank change per time); a diagonal that is not real, finite
+    and non-negative raises ``ValueError``.
+    """
+    Ninv = np.asarray(Ninv)
+    if Ninv.ndim != 3:
+        return Ninv, flags, None
+    if Ninv.shape != (ntimes, nfreqs, nfreqs):
+        raise ValueError("Ninv shape must be (Ntimes, Nfreqs, Nfreqs) or (Nfreqs, Nfreqs)")
+    if np.all(Ninv == Ninv[0]):
+        return Ninv[0], flags, None
+    d = np.diagonal(Ninv, axis1=1, axis2=2)
+    if np.count_nonzero(Ninv) != np.count_nonzero(d):
+        raise NotImplementedError("per-time Ninv: only diagonal slices are supported (a non-diagonal N_t^-1 is a dense rank "
+                                  "change per time)")
+    flags, ninv_t = _time_noise_diag(d, flags, ntimes, nfreqs)
+    return None, flags, ninv_t
+
+
+def _time_noise_diag(d, flags, ntimes, nfreqs):
+    """``(flags, ninv_t)`` of per-time noise given by its ``(Ntimes, Nfreqs)`` diagonals ``d``: checked to be real, finite and
+    non-negative (``ValueError`` otherwise), the flags broadcast to ``(Ntimes, Nfreqs)``."""
+    d = np.asarray(d)
+    if d.shape != (ntimes, nfreqs):
+        raise ValueError("per-time noise diagonals must have shape (Ntimes, Nfreqs)")
+    if np.any(np.imag(d) != 0) or not np.all(np.isfinite(d)) or np.any(np.real(d) < 0):
+        raise ValueError("per-time Ninv: the diagonals must be real, finite and non-negative")
+    flags = np.asarray(flags)
+    if flags.ndim == 1:
+        flags = np.broadcast_to(flags, (ntimes, nfreqs))
+    return np.ascontiguousarray(flags), np.ascontiguousarray(np.real(d), dtype=np.float64)
+
+
 # --------------------------------------------------------------------------------------------
 class GibbsEngine:
     """Batched Gibbs sampler: ``nchains`` baselines of identical shape resident on one GPU.
@@ -284,7 +326,10 @@ class GibbsEngine:
 
     # -- loading
     def load_chain(self, chain, vis, flags, fgmodes, ninv_diag, lam0sq, ps_prior=None, basis0=None, ninv_dense=None,
-                   nih_dense=None):
+                   nih_dense=None, ninv_t=None):
+        """Load one baseline.  ``ninv_t``: ``(Ntimes, Nfreqs)`` diagonal of the inverse noise covariance of every time (engines
+        with ``time_flags``; ``ninv_diag`` is then ignored): the chain runs one factorisation per time
+        (``hp_engine_load_chain_time_noise``)."""
         T, n, m = self.ntimes, self.nfreqs, self.nmodes
         vis = _lib.c128(vis)
         assert vis.shape == (T, n)
@@ -295,10 +340,18 @@ class GibbsEngine:
             assert fl.shape == (n,), "`flags` array must have shape (Nfreqs,)"
         F = _lib.c128(fgmodes)
         assert F.shape == (n, m), "fgmodes must have shape (Nfreqs, Nmodes)"
-        nd = _lib.f64(ninv_diag)
         l0 = _lib.f64(lam0sq)
         pr = None if ps_prior is None else _lib.f64(ps_prior)
         b0 = None if basis0 is None else _lib.c128(basis0)
+        if ninv_t is not None:
+            if not self.time_flags:
+                raise ValueError("ninv_t (per-time noise) needs an engine created with time_flags=True")
+            nt = _lib.f64(ninv_t)
+            assert nt.shape == (T, n), "ninv_t must have shape (Ntimes, Nfreqs)"
+            _lib.check(_lib.lib().hp_engine_load_chain_time_noise(self._h, int(chain), _lib.ptr(vis), _lib.ptr(fl), _lib.ptr(F),
+                                                                  _lib.ptr(nt), _lib.ptr(b0), _lib.ptr(l0), _lib.ptr(pr)))
+            return
+        nd = _lib.f64(ninv_diag)
         if ninv_dense is not None:
             nD = _lib.c128(ninv_dense)
             nH = None if nih_dense is None else _lib.c128(nih_dense)
@@ -508,10 +561,11 @@ _STAGING_BYTES = int(float(os.environ.get("HP_STAGING_GB", "2")) * 2 ** 30)   # 
 
 
 def _device_bytes_per_chain(ntimes, nfreqs, nmodes, Niter, rng, big_per_iter, general, dense, per_time, summary,
-                            batch=False):
+                            batch=False, time_noise=False):
     """Estimated device memory of one chain of an engine (how many chains share an engine in gibbs_sample_batch).
     ``big_per_iter``: host bytes of one chain's kept outputs per iteration (``_big_bytes_per_iter`` / nchains).
-    ``summary`` / ``batch``: the posterior moments / their batch means are accumulated."""
+    ``summary`` / ``batch``: the posterior moments / their batch means are accumulated.  ``time_noise``: some chain of the
+    engine has per-time noise (the weights of every time)."""
     Np = 32 * ((nfreqs + nmodes + 31) // 32)
     Tp = 16 * ((ntimes + 15) // 16)
     per_chain = 16 * Tp * Np * (4 if rng == "numpy" else 3) + 16 * Tp * nfreqs * 3 + 16 * nfreqs * Np * (2 if general else 1) \
@@ -526,6 +580,8 @@ def _device_bytes_per_chain(ntimes, nfreqs, nmodes, Niter, rng, big_per_iter, ge
         per_chain += 24 * ntimes * (nfreqs + nmodes)   # posterior moments: complex mean + real M2 per element
     if batch:
         per_chain += 24 * ntimes * (nfreqs + nmodes)   # batch means: complex snapshot + real M2_bm per element
+    if time_noise:
+        per_chain += 8 * Tp * nfreqs   # diag(N_t^-1) of every (padded) time
     return per_chain
 
 
@@ -673,13 +729,17 @@ def _check_per_time_supported(solver, basis0, ninv_dense):
 
 
 def _single_chain_engine(vis, flags, S, fgmodes, Ninv, ps_prior, max_iters, rng, solver, map_estimate, keep,
-                         seed, device, s_uniforms=None, ring_iters=0):
-    """Engine with one chain loaded and (numpy mode) its draws injected."""
+                         seed, device, s_uniforms=None, ring_iters=0, ninv_t=None):
+    """Engine with one chain loaded and (numpy mode) its draws injected.  ``ninv_t``: per-time noise diagonals
+    (:func:`_time_noise_model`; ``Ninv`` is then not read)."""
     vis = np.asarray(vis)
     ntimes, nfreqs = vis.shape
     nmodes = np.asarray(fgmodes).shape[1]
     per_time = np.asarray(flags).ndim == 2
-    ninv_diag, ninv_dense, nih_dense = _noise_model(Ninv, flags, nfreqs, need_sqrt=(rng == "numpy" and not map_estimate))
+    if ninv_t is not None:
+        ninv_diag, ninv_dense, nih_dense = None, None, None
+    else:
+        ninv_diag, ninv_dense, nih_dense = _noise_model(Ninv, flags, nfreqs, need_sqrt=(rng == "numpy" and not map_estimate))
     basis0, lam0sq = _analyse_signal_cov(S, device=device)
     if solver is None:
         solver = "reference-cg" if (rng == "numpy" and not per_time) else "exact"
@@ -693,7 +753,7 @@ def _single_chain_engine(vis, flags, S, fgmodes, Ninv, ps_prior, max_iters, rng,
                       force_dense_transforms=_FORCE_DENSE_TRANSFORMS and not per_time, dense_noise=ninv_dense is not None,
                       time_flags=per_time, ring_iters=ring_iters)
     eng.load_chain(0, vis, flags, fgmodes, ninv_diag, lam0sq, ps_prior=ps_prior, basis0=basis0, ninv_dense=ninv_dense,
-                   nih_dense=nih_dense)
+                   nih_dense=nih_dense, ninv_t=ninv_t)
     if rng == "numpy":
         if map_estimate:
             oma = omb = None  # pspec.py:210-212
@@ -756,10 +816,11 @@ def gibbs_step_fgmodes(vis, flags, signal_S, fgmodes, Ninv, ps_prior=None, f0=No
     nfreqs = vis.shape[1]
     flags = np.asarray(flags)
     assert flags.shape == (nfreqs,), "`flags` array must have shape (Nfreqs,)"
+    Ninv, flags, ninv_t = _time_noise_model(Ninv, flags, vis.shape[0], nfreqs)
     pr = _check_prior(ps_prior, nfreqs)
     u = np.array([np.random.uniform() for _ in range(nfreqs)])[None, :] if rng == "numpy" else None
     eng = _single_chain_engine(vis, flags, signal_S, fgmodes, Ninv, pr, 1, rng, solver, map_estimate,
-                               ("cr", "fg", "chisq"), None, device, s_uniforms=u)
+                               ("cr", "fg", "chisq"), None, device, s_uniforms=u, ninv_t=ninv_t)
     try:
         eng.run(1)
         out = (eng.signal_cr(0)[0], eng.signal_S(0), eng.signal_ps(0)[0], eng.fg_amps(0)[0], eng.chisq(0)[0],
@@ -777,6 +838,8 @@ def gibbs_sample_with_fg(vis, flags, S_initial, fgmodes, Ninv, ps_prior, Niter=1
     """Gibbs chain for one baseline (pspec.py:493-658); same arguments and return tuple:
     ``signal_cr, signal_S, signal_ps, fg_amps, chisq, ln_post, write_time``.
 
+    ``Ninv`` may be ``(Ntimes, Nfreqs, Nfreqs)``: identical slices run the 2-D path, diagonal slices a per-time noise model
+    (time t uses ``Ninv[t]``, :func:`_time_noise_model`; one factorisation per time, ``solver="exact"``).
     Extra keyword arguments: ``rng`` / ``solver`` (see the module docstring) and ``device``.
     ``nproc`` is accepted and ignored (all times are solved in one batched launch).
     ``summary=dict(burn_in=..., thin=...)``: the posterior moments of signal_cr and fg_amps are accumulated on the device
@@ -798,6 +861,7 @@ def gibbs_sample_with_fg(vis, flags, S_initial, fgmodes, Ninv, ps_prior, Niter=1
     Ninv = np.asarray(Ninv)
     if len(Ninv.shape) == 3:
         assert Ninv.shape[0] == ntimes, "Ninv shape must be (Ntimes, Nfreqs, Nfreqs) or (Nfreqs, Nfreqs)"
+    Ninv, flags, ninv_t = _time_noise_model(Ninv, flags, ntimes, nfreqs)
     pr = _check_prior(ps_prior, nfreqs)
     u = None
     if rng == "numpy":
@@ -807,7 +871,7 @@ def gibbs_sample_with_fg(vis, flags, S_initial, fgmodes, Ninv, ps_prior, Niter=1
             u = np.random.RandomState(seed).uniform(size=(Niter, nfreqs))  # pspec.py:577
     nmodes = fgmodes.shape[1]
     eng = _single_chain_engine(vis, flags, S_initial, fgmodes, Ninv, pr, Niter, rng, solver, map_estimate,
-                               ("cr", "fg", "chisq"), seed, device, s_uniforms=u, ring_iters=_RING_ITERS)
+                               ("cr", "fg", "chisq"), seed, device, s_uniforms=u, ring_iters=_RING_ITERS, ninv_t=ninv_t)
     write_time = [0.0]
     moments = None
     try:
@@ -870,7 +934,9 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
     (run-hydra-pspec.py:487-557): ``baselines`` is a list of dicts with the arguments of
     :func:`gibbs_sample_with_fg` (``vis, flags, S_initial, fgmodes, Ninv, ps_prior`` and optionally
     ``out_dir``); all chains live in one :class:`GibbsEngine` and every kernel launch covers all of
-    them.  Returns one ``gibbs_sample_with_fg``-style tuple per baseline (arrays that were not kept
+    them.  ``Ninv`` may be ``(Ntimes, Nfreqs, Nfreqs)`` with diagonal slices (per-time noise, :func:`_time_noise_model`); an
+    optional ``ninv_t`` of shape ``(Ntimes, Nfreqs)`` gives the same diagonals directly, in place of ``Ninv``, without the
+    Ntimes Nfreqs^2 host array.  Such baselines run one factorisation per time.  Returns one ``gibbs_sample_with_fg``-style tuple per baseline (arrays that were not kept
     are ``None``).  With ``rng="numpy"`` each chain gets the reference's draws for ``seed`` (every
     baseline the same streams, as in the reference, where each chain reseeds numpy).
 
@@ -902,14 +968,24 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
         assert flags.shape in ((nfreqs,), (ntimes, nfreqs)), "`flags` array must have shape (Nfreqs,) [or (Ntimes, Nfreqs)]"
         F = np.asarray(b["fgmodes"])
         assert F.shape == (nfreqs, nmodes), "fgmodes must have shape (Nfreqs, Nmodes)"
-        nd, nD, nH = _noise_model(b["Ninv"], flags, nfreqs, need_sqrt=(rng == "numpy" and not map_estimate))
-        prep.append(dict(vis=vis * flags, flags=flags, F=F, nd=nd, nD=nD, nH=nH, prior=_check_prior(b.get("ps_prior"), nfreqs)))
+        if b.get("ninv_t") is not None:
+            Ninv = None
+            flags, nt = _time_noise_diag(b["ninv_t"], flags, ntimes, nfreqs)
+        else:
+            Ninv, flags, nt = _time_noise_model(b["Ninv"], flags, ntimes, nfreqs)
+        if nt is None:
+            nd, nD, nH = _noise_model(Ninv, flags, nfreqs, need_sqrt=(rng == "numpy" and not map_estimate))
+        else:
+            nd, nD, nH = None, None, None
+        prep.append(dict(vis=vis * flags, flags=flags, F=F, nd=nd, nD=nD, nH=nH, nt=nt,
+                         prior=_check_prior(b.get("ps_prior"), nfreqs)))
     # one batched device eigendecomposition for all baselines with a non-delay-diagonal S_initial
     covs = [np.eye(nfreqs) if b.get("S_initial") is None else b["S_initial"] for b in baselines]
     for pr_, (basis0, lam0sq) in zip(prep, _analyse_signal_covs(covs, device=device)):
         pr_["basis0"], pr_["lam0sq"] = basis0, lam0sq
     general = any(p["basis0"] is not None for p in prep)
     dense = any(p["nD"] is not None for p in prep)
+    time_noise = any(p["nt"] is not None for p in prep)   # per-time noise: those baselines have (Ntimes, Nfreqs) flags
     per_time = any(p["flags"].ndim == 2 for p in prep)
     if per_time:
         if solver_default and rng == "numpy":
@@ -961,7 +1037,8 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
     # ---- how many chains share an engine: all of them unless the device arena would not fit (then groups run one after
     # the other; the Philox chain ids keep the samples independent of the grouping)
     per_chain = _device_bytes_per_chain(ntimes, nfreqs, nmodes, Niter, rng, per_iter // nb, general, dense, per_time,
-                                        summary is not None, batch=summary is not None and summary.get("batch", 0) > 0)
+                                        summary is not None, batch=summary is not None and summary.get("batch", 0) > 0,
+                                        time_noise=time_noise)
     dev_budget = float(os.environ.get("HP_DEVICE_BUDGET_GB", "150")) * 2 ** 30
     group = max(1, min(nb, int(dev_budget // per_chain)))
     write_times = [0.0] * nb
@@ -988,7 +1065,7 @@ def gibbs_sample_batch(baselines, Niter=100, seed=None, rng="philox", solver=Non
                     if rng == "numpy" and not map_estimate:
                         nH = np.diag(np.sqrt(p["nd"] * p["flags"].astype(float))).astype(np.complex128)
                 eng.load_chain(lc, p["vis"], p["flags"], p["F"], p["nd"], p["lam0sq"], ps_prior=p["prior"], basis0=b0,
-                               ninv_dense=nD, nih_dense=nH)
+                               ninv_dense=nD, nih_dense=nH, ninv_t=p["nt"])
                 if rng == "numpy":
                     eng.set_draws(lc, oma, omb, _s_draws_from_uniforms(u, p["prior"], ntimes))
             if summary is not None:

@@ -116,6 +116,22 @@ int hp_engine_load_chain_dense(hp_engine* e, int chain, const double* vis, const
                                const double* ninv_diag, const double* ninv_dense, const double* nih_dense,
                                const double* basis0, const double* lam0sq, const double* ps_prior);
 
+/* Same with a diagonal inverse noise covariance per time (an extension: the reference's build_matrices takes one N^-1,
+ * pspec.py:361).  Needs cfg.time_flags = 1 and diagonal noise (cfg.dense_noise = 0), otherwise HP_ERR_ARG.
+ *   flags      [Ntimes][Nfreqs] uint8, 1 = unflagged
+ *   ninv_t     [Ntimes][Nfreqs] diag(N_t^-1) of every time, finite and >= 0 (HP_ERR_ARG otherwise); time t uses
+ *              w_t N_t^-1 in the GCR system and N_t^-1 as its chi^2 / ln-posterior weight
+ * A chain loaded this way runs one factorisation per time (csrc/hp_pertime.cu) and puts the whole engine on that form
+ * (hp_engine_pt_form reports it); times whose flags and weights equal those of the time before re-use its factor.
+ * Reloading the chain with hp_engine_load_chain removes the per-time noise; the engine returns to the low-rank form when no
+ * chain has it and no time exceeds that form's rank.  A general basis0 (cfg.general_basis0) is refused with HP_ERR_SIZE.
+ * The per-time weights of all chains (8 Ntimes Nfreqs bytes per chain, times padded to 16) are allocated, outside the
+ * creation-time arena, when the first chain is loaded this way.
+ */
+int hp_engine_load_chain_time_noise(hp_engine* e, int chain, const double* vis, const uint8_t* flags, const double* fgmodes,
+                                    const double* ninv_t, const double* basis0, const double* lam0sq,
+                                    const double* ps_prior);
+
 /* Injected draws (HP_RNG_INJECTED).
  *   omega_a, omega_b [Ntimes][Nfreqs] complex128: the unit complex Gaussians of pspec.py:215-217
  *                    (NULL, NULL = map_estimate, pspec.py:210-212)
@@ -211,7 +227,8 @@ int hp_engine_set_profile(hp_engine* e, int on);
 /* Per-time flags (cfg.time_flags): which form of the per-time solve the engine runs for the chains loaded so far.
  *   *low_rank = 1: one shared factorisation per chain + a rank-k_t correction per time (csrc/hp_ptlow.cu); 0: one
  *   factorisation per (chain, time) (csrc/hp_pertime.cu: a time has more than 64 channels flagged beyond the chain's
- *   all-times mask, Nfreqs + Nmodes > 448, or cfg.force_dense_solve).  *max_rank = largest k_t of the loaded chains.
+ *   all-times mask, a chain carries per-time noise (hp_engine_load_chain_time_noise), Nfreqs + Nmodes > 448, or
+ *   cfg.force_dense_solve).  *max_rank = largest k_t of the loaded chains.
  * Replaces nothing in the reference (it has no per-time flags, pspec.py:428); either pointer may be NULL. */
 int hp_engine_pt_form(const hp_engine* e, int* low_rank, int* max_rank);
 /* Total kernel launches issued by hp_engine_run / hp_engine_gcr so far. */

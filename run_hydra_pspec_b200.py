@@ -78,6 +78,9 @@ def build_parser():
     p.add_argument("--time_flags", choices=("any", "per-time"), default="any",
                    help="any: a channel flagged at any time is flagged at all times (the reference, "
                         "run-hydra-pspec.py:520-526); per-time: keep the (Ntimes, Nfreqs) flags (in-painting)")
+    p.add_argument("--noise_weights", choices=("none", "nsamples"), default=argparse.SUPPRESS,
+                   help="none (default): one inverse noise covariance for all times; nsamples: diagonal noise per time and channel, "
+                        "N_t^-1 = nsamples[t] * diag(N^-1) (needs --nsamples and a diagonal N^-1, i.e. no --noise_cov)")
     p.add_argument("--samples", choices=("all", "summary", "both"), default="all",
                    help="all: every sample of signal_cr / fg_amps / chisq (gcr-eor.npy, fg-amps.npy, chisq.npy); summary: only "
                         "their posterior mean and variance, accumulated on the GPU (gcr-eor-mean.npy, gcr-eor-var.npy, "
@@ -223,8 +226,12 @@ def assemble_baselines(args, antpairs, freqs, get, out_dir):
         else:
             fgmodes = np.array([scipy.special.legendre(i)(np.linspace(-1.0, 1.0, freqs.size))
                                 for i in range(args.Nfgmodes)]).T
+        ninv_t = None
+        if getattr(args, "noise_weights", "none") == "nsamples":
+            # the noise of a cell averaged over nsamples samples has variance sigma^2 / nsamples (the simulated noise above)
+            ninv_t = np.asarray(nsamples, dtype=np.float64) * np.real(np.diagonal(Ninv))[None, :]
         all_data_weights.append({"antpair": tuple(int(a) for a in antpair), "d": d, "w": flags, "fgmodes": fgmodes,
-                                 "S_initial": sigcov0, "Ninv": Ninv, "out_dir": out_dir})
+                                 "S_initial": sigcov0, "Ninv": Ninv, "ninv_t": ninv_t, "out_dir": out_dir})
     return all_data_weights
 
 
@@ -236,6 +243,14 @@ def ps_prior_for(args, Nfreqs):
         ps_prior[0, inds] = args.ps_prior_hi
         ps_prior[1, inds] = args.ps_prior_lo
     return ps_prior
+
+
+def time_noise_ninv(ninv_t):
+    """(Ntimes, Nfreqs, Nfreqs) inverse noise covariance with diagonal slices diag(ninv_t[t])."""
+    T, n = ninv_t.shape
+    out = np.zeros((T, n, n), dtype=np.float64)
+    out[:, np.arange(n), np.arange(n)] = ninv_t
+    return out
 
 
 def time_invariant_flags(w):
@@ -254,6 +269,12 @@ def main(argv=None):
             parser.error("--batch needs --samples summary or both")
         if batch < 1:
             parser.error("--batch must be >= 1")
+    if getattr(args, "noise_weights", "none") == "nsamples":   # absent from the namespace unless given
+        if not args.nsamples:
+            parser.error("--noise_weights nsamples needs --nsamples")
+        if args.noise_cov:
+            parser.error("--noise_weights nsamples needs a diagonal inverse noise covariance: it cannot be combined with "
+                         "--noise_cov")
     summary = None if args.samples == "all" else dict(burn_in=args.burn_in, thin=args.thin)
     if batch:
         summary["batch"] = batch
@@ -321,14 +342,17 @@ def main(argv=None):
         w = ~np.asarray(data["w"], dtype=bool)
         flags = w if args.time_flags == "per-time" else time_invariant_flags(w)
         jobs.append(dict(vis=data["d"], flags=flags, S_initial=data["S_initial"], fgmodes=data["fgmodes"],
-                         Ninv=data["Ninv"], ps_prior=ps_prior_for(args, data["d"].shape[1]), out_dir=bl_dir,
-                         antpair=antpair))
+                         Ninv=data["Ninv"], ninv_t=data["ninv_t"], ps_prior=ps_prior_for(args, data["d"].shape[1]),
+                         out_dir=bl_dir, antpair=antpair))
 
     ant_pairs, write_times = [], []
     if args.rng == "numpy":
         for job in jobs:  # one chain after the other, the reference's streams
             if verbose:
                 print(f"Printing status messages for:\nRank:     {rank}\nBaseline: {job['antpair']}", end="\n\n")
+            if job["ninv_t"] is not None and args.samples != "summary":
+                # the drop-in takes per-time noise as a 3-D Ninv; built for one baseline at a time
+                job = dict(job, Ninv=time_noise_ninv(job["ninv_t"]), ninv_t=None)
             if args.samples == "summary":
                 # the same chain through the batched form, which can leave the samples on the device (keep=())
                 res = pspec.gibbs_sample_batch([job], Niter=args.Niter, seed=args.seed, rng="numpy", solver=args.solver,
