@@ -79,6 +79,10 @@ _SIGNATURES = {
     "hp_test_solve3": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                  C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "hp_test_solve3_schedule": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "hp_test_pt_lowrank": (C.c_int, [C.c_int] * 4 + [C.c_void_p] * 8 + [C.c_int, C.c_uint32, C.c_uint32, C.c_uint32,
+                                                                        C.c_void_p, C.c_void_p, C.c_void_p]),
+    "hp_test_pt_cholsolve": (C.c_int, [C.c_int] * 4 + [C.c_void_p] * 5 + [C.c_int, C.c_int, C.c_uint32, C.c_uint32,
+                                                                          C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "hp_fp64_peak_tflops": (C.c_double, [C.c_int, C.c_double]),
     "hp_release_cached_memory": (None, []),
     "hp_pinned_alloc": (C.c_void_p, [C.c_size_t]),

@@ -43,6 +43,14 @@ void hp_host_normals_fast(uint32_t k0, uint32_t k1, int n, double* out) {
     }
 }
 
+// One pair of normals from the Philox block of any counter: normal_pair (fast = 0) or normal_pair_fast (fast = 1).  Lets the
+// GPU tests reproduce a kernel's draws from its counter layout.
+void hp_host_normal_pair(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, int fast, double* out) {
+    hp::u32x4 c; c.x = c0; c.y = c1; c.z = c2; c.w = c3;
+    if (fast) hp::normal_pair_fast(hp::philox4x32_10(c, k0, k1), out[0], out[1]);
+    else hp::normal_pair(hp::philox4x32_10(c, k0, k1), out[0], out[1]);
+}
+
 void hp_host_gammas(double alpha, uint32_t k0, uint32_t k1, int n, double* out) {
     for (int i = 0; i < n; ++i) out[i] = hp::gamma_mt(alpha, (uint32_t)i, 0, 7, k0, k1);
 }

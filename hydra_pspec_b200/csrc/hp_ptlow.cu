@@ -102,11 +102,15 @@ __global__ void __launch_bounds__(256, kPtLowMinBlocks) k_pt_lowrank(PtLowArgs a
             }
         }
         __syncwarp();
-        // K = I - P_ff (lower triangle): the k (k + 1) / 2 entries spread over the lanes, all loads independent
+        // K = I - P_ff (lower triangle): the k (k + 1) / 2 entries spread over the lanes, all loads independent.  Only the
+        // lower triangle of P is computed (lower_out), so an entry whose channels come in descending order is read as the
+        // conjugate of its mirror: the channel list need not be sorted.
         const int ktri = tri(k);
         for (int e = lane; e < ktri; e += 32) {
             const int rc = tab[e], r = rc >> 8, c = rc & 255;
-            const double2 p = Pm[(size_t)fl[r] * n + fl[c]];
+            const int fr = fl[r], fc = fl[c];
+            double2 p = Pm[(size_t)(fr >= fc ? fr : fc) * n + (fr >= fc ? fc : fr)];
+            if (fr < fc) p.y = -p.y;
             Kp[e] = make_double2((c == r ? 1.0 : 0.0) - p.x, c == r ? 0.0 : -p.y);
         }
         // c = (R^H b)_f, two channels at a time

@@ -175,6 +175,137 @@ int hp_test_solve3_schedule(int nblk, unsigned char* n, unsigned char* strips, i
     return HP_OK;
 }
 
+// k_pt_lowrank (hp_ptlow.cu) alone, launched as solve_pt_lowrank launches it, for nsys systems of N = Np - padding unknowns
+// with n columns of A each.  In: lam [nsys][N], Rfix [nsys][T][N], wa [nsys][T][n] or NULL, X0 [nsys][T][N] (x0_t = M_0^-1 b_t),
+// Rcols [nsys][n][N] (row x = R[:, x]), P [nsys][n][n], fidx [nsys][T][64], fcnt [nsys][T], chain_ids [nsys] (read with
+// philox only).  Out: X [nsys][T][N], info [nsys].  Every device element the kernel must not read is NaN: the padding columns
+// N .. Np of every row, the rows T .. Tp0 of X and all rows Tp0 + x of Rfix.
+int hp_test_pt_lowrank(int n, int N, int T, int nsys, const double* lam, const double* Rfix, const double* wa, const double* X0,
+                       const double* Rcols, const double* P, const uint16_t* fidx, const int* fcnt, int philox, uint32_t key0,
+                       uint32_t key1, uint32_t iter, const int* chain_ids, double* X, int* info) {
+    if (n < 1 || N < n || T < 1 || nsys < 1) return HP_ERR_ARG;
+    const int nblk = (N + 31) / 32, Np = nblk * 32;
+    if (nblk > 14) return HP_ERR_SIZE;   // k_pt_lowrank<14> holds at most 14 rows per lane
+    int kcap = 0;
+    for (size_t i = 0; i < (size_t)nsys * T; ++i) {
+        if (fcnt[i] < 0) return HP_ERR_ARG;
+        if (fcnt[i] > hp::kPtLowMaxRank) return HP_ERR_SIZE;
+        for (int e = 0; e < fcnt[i]; ++e)
+            if (fidx[i * hp::kPtLowMaxRank + e] >= n) return HP_ERR_ARG;
+        if (fcnt[i] > kcap) kcap = fcnt[i];
+    }
+    const int Tp0 = 16 * ((T + 15) / 16), Tp = Tp0 + 16 * ((n + 15) / 16);
+    const size_t rows = (size_t)nsys * Tp;
+    double *dlam, *dR, *dW = nullptr, *dX, *dP;
+    uint16_t* dF;
+    int *dC, *dinfo, *dch;
+    if (cudaMalloc(&dlam, 8ull * nsys * Np) || cudaMalloc(&dR, 16 * rows * Np) || cudaMalloc(&dX, 16 * rows * Np) ||
+        cudaMalloc(&dP, 16ull * nsys * n * n) || cudaMalloc(&dF, 2ull * nsys * T * hp::kPtLowMaxRank) ||
+        cudaMalloc(&dC, 4ull * nsys * T) || cudaMalloc(&dinfo, 4ull * nsys) || cudaMalloc(&dch, 4ull * nsys) ||
+        (wa && cudaMalloc(&dW, 16 * rows * Np)))
+        return HP_ERR_CUDA;
+    cudaMemset(dlam, 0xff, 8ull * nsys * Np);   // 0xff..: NaN
+    cudaMemset(dR, 0xff, 16 * rows * Np);
+    cudaMemset(dX, 0xff, 16 * rows * Np);
+    cudaMemset(dinfo, 0, 4ull * nsys);
+    cudaMemcpy2D(dlam, 8ull * Np, lam, 8ull * N, 8ull * N, nsys, cudaMemcpyHostToDevice);
+    for (int s = 0; s < nsys; ++s) {
+        const size_t d0 = 2ull * s * Tp * Np;
+        cudaMemcpy2D(dR + d0, 16ull * Np, Rfix + 2ull * s * T * N, 16ull * N, 16ull * N, T, cudaMemcpyHostToDevice);
+        cudaMemcpy2D(dX + d0, 16ull * Np, X0 + 2ull * s * T * N, 16ull * N, 16ull * N, T, cudaMemcpyHostToDevice);
+        cudaMemcpy2D(dX + d0 + 2ull * Tp0 * Np, 16ull * Np, Rcols + 2ull * s * n * N, 16ull * N, 16ull * N, n, cudaMemcpyHostToDevice);
+    }
+    if (wa) {
+        cudaMemset(dW, 0xff, 16 * rows * Np);
+        for (int s = 0; s < nsys; ++s)
+            cudaMemcpy2D(dW + 2ull * s * Tp * Np, 16ull * Np, wa + 2ull * s * T * n, 16ull * n, 16ull * n, T, cudaMemcpyHostToDevice);
+    }
+    cudaMemcpy(dP, P, 16ull * nsys * n * n, cudaMemcpyHostToDevice);
+    cudaMemcpy(dF, fidx, 2ull * nsys * T * hp::kPtLowMaxRank, cudaMemcpyHostToDevice);
+    cudaMemcpy(dC, fcnt, 4ull * nsys * T, cudaMemcpyHostToDevice);
+    if (philox) cudaMemcpy(dch, chain_ids, 4ull * nsys, cudaMemcpyHostToDevice);
+    else cudaMemset(dch, 0xff, 4ull * nsys);
+    hp::PtLowArgs la{};
+    la.Rfix = dR; la.wa = dW; la.lam = dlam; la.X = dX; la.Pm = dP; la.fidx = dF; la.fcnt = dC; la.info = dinfo;
+    la.n = n; la.N = N; la.Np = Np; la.T = T; la.Tp = Tp; la.Tp0 = Tp0; la.nsys = nsys; la.nblk = nblk; la.kcap = kcap;
+    la.philox = philox ? 1 : 0;
+    la.dk = hp::DrawKey{key0, key1, iter, dch};
+    hp::launch_pt_lowrank(la, 0);
+    cudaError_t e = cudaDeviceSynchronize();
+    if (e == cudaSuccess) {
+        for (int s = 0; s < nsys; ++s)
+            cudaMemcpy2D(X + 2ull * s * T * N, 16ull * N, dX + 2ull * s * Tp * Np, 16ull * Np, 16ull * N, T, cudaMemcpyDeviceToHost);
+        cudaMemcpy(info, dinfo, 4ull * nsys, cudaMemcpyDeviceToHost);
+    }
+    cudaFree(dlam); cudaFree(dR); cudaFree(dW); cudaFree(dX); cudaFree(dP); cudaFree(dF); cudaFree(dC); cudaFree(dinfo); cudaFree(dch);
+    return e == cudaSuccess ? HP_OK : HP_ERR_CUDA;
+}
+
+// k_pt_cholsolve (hp_pertime.cu) alone for nsys systems of N = n + m unknowns and T times.  In: H [nsys][T][1 + m][N] (column 0:
+// chat_t in its first n entries; column 1 + j: [Q|F]^H (w_t N^-1) F[:, j]), lam [nsys][N], Rfix [nsys][T][N], wa [nsys][T][n]
+// or NULL, same_prev [nsys][T] or NULL, grid (0: pt_grid), chain_ids [nsys] (read with philox only).  Out: X [nsys][T][N],
+// info [nsys].  The kernel reads the padding rows N .. Np of lam, Rfix and wa (zero in the engine): they are zero here; the
+// padding rows of H and the entries n .. N of column 0 are NaN, and so is the scratch the factors live in, so that a
+// factor re-used without having been computed poisons the result.
+int hp_test_pt_cholsolve(int n, int m, int T, int nsys, const double* H, const double* lam, const double* Rfix, const double* wa,
+                         const int* same_prev, int grid, int philox, uint32_t key0, uint32_t key1, uint32_t iter,
+                         const int* chain_ids, double* X, int* info) {
+    if (n < 1 || m < 0 || T < 1 || nsys < 1 || grid < 0) return HP_ERR_ARG;
+    const int N = n + m, nblk = (N + 31) / 32, Np = nblk * 32, Tp = 16 * ((T + 15) / 16);
+    int max_smem = 0, dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (hp::pt_smem_bytes(nblk, n) > (size_t)max_smem) return HP_ERR_SIZE;
+    if (grid == 0) grid = hp::pt_grid(nsys, T);
+    const size_t rows = (size_t)nsys * Tp, hcols = (size_t)(1 + m), scr = (size_t)grid * hp::pt_scratch_doubles_per_cta(nblk);
+    double *dH, *dlam, *dR, *dW = nullptr, *dX, *dS;
+    int *dsame = nullptr, *dinfo, *dch;
+    if (cudaMalloc(&dH, 16 * rows * hcols * Np) || cudaMalloc(&dlam, 8ull * nsys * Np) || cudaMalloc(&dR, 16 * rows * Np) ||
+        cudaMalloc(&dX, 16 * rows * Np) || cudaMalloc(&dS, 8 * scr) || cudaMalloc(&dinfo, 4ull * nsys) ||
+        cudaMalloc(&dch, 4ull * nsys) || (wa && cudaMalloc(&dW, 16 * rows * Np)) || (same_prev && cudaMalloc(&dsame, 4 * rows)))
+        return HP_ERR_CUDA;
+    cudaMemset(dH, 0xff, 16 * rows * hcols * Np);   // 0xff..: NaN
+    cudaMemset(dX, 0xff, 16 * rows * Np);
+    cudaMemset(dS, 0xff, 8 * scr);
+    cudaMemset(dlam, 0, 8ull * nsys * Np);
+    cudaMemset(dR, 0, 16 * rows * Np);
+    cudaMemset(dinfo, 0, 4ull * nsys);
+    cudaMemcpy2D(dlam, 8ull * Np, lam, 8ull * N, 8ull * N, nsys, cudaMemcpyHostToDevice);
+    for (int s = 0; s < nsys; ++s) {
+        double* h0 = dH + 2ull * s * Tp * hcols * Np;
+        cudaMemcpy2D(h0, 16ull * Np, H + 2ull * s * T * hcols * N, 16ull * N, 16ull * N, T * hcols, cudaMemcpyHostToDevice);
+        for (int t = 0; t < T; ++t)   // column 0 carries chat_t in its first n entries only
+            if (N > n) cudaMemset(h0 + 2ull * t * hcols * Np + 2ull * n, 0xff, 16ull * (N - n));
+        cudaMemcpy2D(dR + 2ull * s * Tp * Np, 16ull * Np, Rfix + 2ull * s * T * N, 16ull * N, 16ull * N, T, cudaMemcpyHostToDevice);
+    }
+    if (wa) {
+        cudaMemset(dW, 0, 16 * rows * Np);
+        for (int s = 0; s < nsys; ++s)
+            cudaMemcpy2D(dW + 2ull * s * Tp * Np, 16ull * Np, wa + 2ull * s * T * n, 16ull * n, 16ull * n, T, cudaMemcpyHostToDevice);
+    }
+    if (same_prev) {
+        cudaMemset(dsame, 0, 4 * rows);
+        cudaMemcpy2D(dsame, 4ull * Tp, same_prev, 4ull * T, 4ull * T, nsys, cudaMemcpyHostToDevice);
+    }
+    if (philox) cudaMemcpy(dch, chain_ids, 4ull * nsys, cudaMemcpyHostToDevice);
+    else cudaMemset(dch, 0xff, 4ull * nsys);
+    hp::PtArgs pa{};
+    pa.H = dH; pa.lam = dlam; pa.Rfix = dR; pa.wa = dW; pa.X = dX; pa.scratch = dS; pa.same_prev = dsame; pa.info = dinfo;
+    pa.nblk = nblk; pa.n = n; pa.m = m; pa.N = N; pa.T = T; pa.Tp = Tp; pa.nsys = nsys;
+    pa.philox_wa = philox ? 1 : 0;
+    pa.dk = hp::DrawKey{key0, key1, iter, dch};
+    hp::launch_pt_cholsolve(pa, grid, 0);
+    cudaError_t e = cudaDeviceSynchronize();
+    if (e == cudaSuccess) {
+        for (int s = 0; s < nsys; ++s)
+            cudaMemcpy2D(X + 2ull * s * T * N, 16ull * N, dX + 2ull * s * Tp * Np, 16ull * Np, 16ull * N, T, cudaMemcpyDeviceToHost);
+        cudaMemcpy(info, dinfo, 4ull * nsys, cudaMemcpyDeviceToHost);
+    }
+    cudaFree(dH); cudaFree(dlam); cudaFree(dR); cudaFree(dW); cudaFree(dX); cudaFree(dS); cudaFree(dsame); cudaFree(dinfo);
+    cudaFree(dch);
+    return e == cudaSuccess ? HP_OK : HP_ERR_CUDA;
+}
+
 // ---- measurement helpers -----------------------------------------------------------------
 namespace {
 __global__ void __launch_bounds__(256) k_fp64_peak(double* out, int iters, double a, double b) {

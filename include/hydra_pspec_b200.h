@@ -262,6 +262,21 @@ int hp_test_solve3(int n, int m, int T, int nsys, const double* G, const double*
  * n[2][nwarps] strips per pass and warp, strips[2][nwarps][max_per_warp] their 16-row strip indices */
 int hp_test_solve3_schedule(int nblk, unsigned char* n, unsigned char* strips, int* nwarps, int* max_per_warp);
 
+/* k_pt_lowrank (csrc/hp_ptlow.cu) alone, launched as the engine launches it, for nsys systems of N unknowns (n columns of A):
+ * lam [nsys][N], Rfix [nsys][T][N], wa [nsys][T][n] or NULL, X0 [nsys][T][N] = M_0^-1 b_t, Rcols [nsys][n][N] = R^T (row x is
+ * R[:, x]), P [nsys][n][n] (lower triangle read), fidx [nsys][T][64], fcnt [nsys][T], chain_ids [nsys] (philox only);
+ * out X [nsys][T][N], info [nsys].  HP_ERR_SIZE for N > 448 or a count above 64. */
+int hp_test_pt_lowrank(int n, int N, int T, int nsys, const double* lam, const double* Rfix, const double* wa, const double* X0,
+                       const double* Rcols, const double* P, const uint16_t* fidx, const int* fcnt, int philox, uint32_t key0,
+                       uint32_t key1, uint32_t iter, const int* chain_ids, double* X, int* info);
+/* k_pt_cholsolve (csrc/hp_pertime.cu) alone for nsys systems of N = n + m unknowns: H [nsys][T][1 + m][N] (column 0 = chat_t,
+ * first n entries), lam [nsys][N], Rfix [nsys][T][N], wa [nsys][T][n] or NULL, same_prev [nsys][T] or NULL, grid (0: the
+ * engine's persistent grid), chain_ids [nsys] (philox only); out X [nsys][T][N], info [nsys].  HP_ERR_SIZE when the shared
+ * working set exceeds the device's opt-in limit. */
+int hp_test_pt_cholsolve(int n, int m, int T, int nsys, const double* H, const double* lam, const double* Rfix, const double* wa,
+                         const int* same_prev, int grid, int philox, uint32_t key0, uint32_t key1, uint32_t iter,
+                         const int* chain_ids, double* X, int* info);
+
 /* ---- measurement helpers ---------------------------------------------------------------------- */
 /* FP64 tensor-pipe (DMMA.8x8x4) peak of the device measured with an issue loop for ~`seconds`; TFLOP/s. */
 double hp_fp64_peak_tflops(int device, double seconds);

@@ -202,20 +202,40 @@ def test_per_time_repeated_masks_reuse_the_factor(hold, pt_form):
         assert rel(o, r) < (1e-8 if k == "chisq" else TOL), k
 
 
-@pytest.mark.parametrize("frac,expect_lowrank", [(0.2, True), (0.45, False)])
-def test_per_time_rank_limit_selects_the_form(frac, expect_lowrank):
+@pytest.mark.parametrize("nf,nm,frac,expect_lowrank", [
+    pytest.param(256, 16, 0.2, True, id="0.2-True"),
+    pytest.param(256, 16, 0.45, False, id="0.45-False"),
+    pytest.param(384, 32, 0.1, True, id="384-32-0.1-True"),       # N = 416: k_pt_lowrank<14>, one time at rank 64
+    pytest.param(384, 32, 0.45, False, id="384-32-0.45-False"),
+    pytest.param(512, 16, 0.1, False, id="512-16-0.1-False"),     # N = 528: no k_solve3, so direct although every k_t <= 64
+    pytest.param(1024, 64, 0.05, False, id="1024-64-0.05-False"),  # nblk = 34, k_post_fft2 at 1024 (4 times, 1 iteration)
+])
+def test_per_time_rank_limit_selects_the_form(nf, nm, frac, expect_lowrank):
     """Nfreq=256: 20 % per-time flags stay below the 64-channel limit of the low-rank form (ranks up to ~60); 45 % exceed it
-    and the engine falls back to one factorisation per time.  Both against the oracle."""
+    and the engine falls back to one factorisation per time.  At 384 + 32 the same two sides of the rank limit, at 512 + 16 and
+    1024 + 64 the direct form because N > 448.  The form is asserted on an engine loaded with the same chain; both forms
+    against the oracle."""
     from hydra_pspec_b200 import pspec
-    vis, flags, S0, F, Ninv, prior = make_case(6, 256, 16, frac, 61)
+    nt, niter = (4, 1) if nf >= 1024 else (6, 2)
+    vis, flags, S0, F, Ninv, prior = make_case(nt, nf, nm, frac, 61)
     if expect_lowrank:
         wbar = flags.any(axis=0)
         flags[1, np.flatnonzero(wbar)[:64]] = False       # one time at exactly the limit
         flags[1, np.flatnonzero(wbar)[64:]] = True
     kmax = int(np.max(np.sum(flags.any(axis=0)[None, :] & ~flags, axis=1)))
-    assert (kmax <= 64) == expect_lowrank
-    ref = ho.gibbs_sample_with_fg(vis, flags, S0, F, Ninv, prior, Niter=2, seed=9, solver="direct")
-    out = pspec.gibbs_sample_with_fg(vis, flags, S0, F, Ninv, prior, Niter=2, seed=9, verbose=False)
+    if nf + nm <= 448:
+        assert (kmax <= 64) == expect_lowrank
+    eng = pspec.GibbsEngine(1, nt, nf, nm, max_iters=1, rng="numpy", keep=(), time_flags=True)
+    try:
+        eng.load_chain(0, vis, flags, F, np.real(np.diag(Ninv)), np.full(nf, 1.0 / nf))
+        form, kcap = eng.pt_form()
+    finally:
+        eng.close()
+    assert form == ("low-rank" if expect_lowrank else "direct")
+    if expect_lowrank:
+        assert kcap == kmax == 64
+    ref = ho.gibbs_sample_with_fg(vis, flags, S0, F, Ninv, prior, Niter=niter, seed=9, solver="direct")
+    out = pspec.gibbs_sample_with_fg(vis, flags, S0, F, Ninv, prior, Niter=niter, seed=9, verbose=False)
     for o, r, k in zip(out[:6], ref, KEYS):
         assert rel(o, r) < (1e-8 if k == "chisq" else TOL), k
 

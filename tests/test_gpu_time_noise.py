@@ -71,6 +71,7 @@ def make_case(nt, nf, nm, seed, weights, per_time_flags):
     (96, 8, "every+zeros", True),
     (120, 0, "every+zero_time", False),
     (120, 8, "piecewise", True),
+    (512, 16, "piecewise", True),       # N = 528: k_pt_cholsolve at nblk = 17, k_post_fft2 at 512
 ])
 def test_time_noise_chain_matches_oracle(nf, nm, weights, per_time_flags):
     from hydra_pspec_b200 import pspec

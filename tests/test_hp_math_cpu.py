@@ -29,6 +29,7 @@ def hm():
     L.hp_host_normals.argtypes = [C.c_uint32, C.c_uint32, C.c_int, C.c_void_p]
     L.hp_host_normals_fast.argtypes = [C.c_uint32, C.c_uint32, C.c_int, C.c_void_p]
     L.hp_host_gammas.argtypes = [C.c_double, C.c_uint32, C.c_uint32, C.c_int, C.c_void_p]
+    L.hp_host_normal_pair.argtypes = [C.c_uint32] * 6 + [C.c_int, C.c_void_p]
     return L
 
 
@@ -66,6 +67,26 @@ def test_fast_normals_are_standard(hm):
     # tails are populated as expected: P(|x| > 4) = 6.33e-5
     frac = np.mean(np.abs(x) > 4)
     assert abs(frac - 6.334e-5) < 5 * np.sqrt(6.334e-5 / n)
+
+
+def test_normal_pair_of_any_counter(hm):
+    """hp_host_normal_pair (the draws of one general Philox counter, used by the GPU kernel tests) with counters (i, 0, 0, 0)
+    is the stream of hp_host_normals / hp_host_normals_fast, and every counter word and key word changes the draw."""
+    n = 2000
+    out = np.empty(2)
+    for fast, stream in ((0, hm.hp_host_normals), (1, hm.hp_host_normals_fast)):
+        x = np.empty(n)
+        stream(0xA5A5A5A5, 77, n, x.ctypes.data_as(C.c_void_p))
+        got = np.empty(n)
+        for i in range(n // 2):
+            hm.hp_host_normal_pair(i, 0, 0, 0, 0xA5A5A5A5, 77, fast, got[2 * i:].ctypes.data_as(C.c_void_p))
+        assert np.array_equal(got, x)
+        hm.hp_host_normal_pair(3, 0, 0, 0, 0xA5A5A5A5, 77, fast, out.ctypes.data_as(C.c_void_p))
+        base = out.copy()
+        for args in ((3, 1, 0, 0, 0xA5A5A5A5, 77), (3, 0, 1, 0, 0xA5A5A5A5, 77), (3, 0, 0, 1, 0xA5A5A5A5, 77),
+                     (0x80000003, 0, 0, 0, 0xA5A5A5A5, 77), (3, 0, 0, 0, 0xA5A5A5A4, 77), (3, 0, 0, 0, 0xA5A5A5A5, 76)):
+            hm.hp_host_normal_pair(*args, fast, out.ctypes.data_as(C.c_void_p))
+            assert not np.any(out == base), args
 
 
 @pytest.mark.parametrize("alpha", [1.0, 15.0, 202.0, 1023.0])
